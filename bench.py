@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W            # this repo (CUDA, C ABI)
     python bench.py --impl reference --steps K --warmup W    # the reference's CPU path (its own code from oracle/_ref,
                                                              # else the oracle port) on the host cores
+    python bench.py --steps K --warmup W --dump-outputs DIR  # also DIR/rects.npy: the rects of the last timed step
 
 A "step" is one pass of the whole hot path (pyramid resize -> integral images -> cascade ->
 raw rects) over one batch of synthetic 1080p frames per GPU.  Workload = BASELINE.json's
@@ -127,6 +128,18 @@ class ClockSampler:
                     reasons.add(nm)
         return {"sm_mhz": float(np.median(sm)) if sm else None, "sm_max_mhz": max(mx) if mx else None,
                 "samples": len(sm), "reasons": sorted(reasons)}
+
+
+def dump_rects(dirname: str, rects: np.ndarray):
+    """--dump-outputs: int32 [n, 6] rects (x, y, w, h, global frame, cascade) -> dirname/rects.npy in float64, rows
+    sorted by frame, cascade, y, x, w, h (the device appends them in no fixed order).  Above 1 << 20 rows (48 MiB) a
+    fixed-seed sample of the rows is kept, so the file stays under 64 MB."""
+    out = rects[np.lexsort(rects.T[[3, 2, 0, 1, 5, 4]])].astype(np.float64)
+    cap = 1 << 20
+    if len(out) > cap:
+        out = out[np.sort(np.random.default_rng(0).choice(len(out), cap, replace=False))]
+    os.makedirs(dirname, exist_ok=True)
+    np.save(os.path.join(dirname, "rects.npy"), out)
 
 
 def cpu_reference(frames: np.ndarray, threads: int):
@@ -296,6 +309,8 @@ def run_stream_bench(args):
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)   # max over ranks
     dev_ms, e2e_s = (float(x) for x in t.tolist())
+    if args.dump_outputs and rank == 0:
+        dump_rects(args.dump_outputs, gathered)
     if rank == 0:
         wpf = sum(det.windows_per_frame(i) for i in range(len(cas)))
         steps = -(-(last - first) // B)
@@ -344,7 +359,15 @@ def main():
     ap.add_argument("--min-size", default="0x0", help="minimum window WxH")
     ap.add_argument("--cascade", default=CASCADE, help="stock cascade name (default: the metric's frontalface_alt; "
                     "frontalface_default is BASELINE.json configs[1]); a comma list shares one pyramid (configs[2], [3])")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the raw rects of the last timed step (with --stream: of the timed host-to-rects pass over "
+                         "the stream) to DIR/rects.npy (float64 [n, 6]: x, y, w, h, global frame, cascade; rows sorted), "
+                         "so that two builds can be compared on the same seeded frames")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs covers the GPU path (--impl native) only")
     CASCADE = args.cascade
     XML = [os.path.join(ROOT, "data", "haarcascades", f"haarcascade_{c}.xml") for c in CASCADE.split(",")]
     W, H = (int(v) for v in args.size.lower().split("x"))
@@ -414,7 +437,7 @@ def main():
     t0 = time.perf_counter()
     e0.record()
     for _ in range(args.steps):
-        step_device()
+        res = step_device()
     e1.record()
     barrier()
     wall = time.perf_counter() - t0
@@ -481,6 +504,8 @@ def main():
     gathered = sharding.gather_rects(local, device="cuda")
     gather_ms = 1e3 * (time.perf_counter() - t_g0)
     total_rects = len(gathered)
+    if args.dump_outputs and rank == 0:
+        dump_rects(args.dump_outputs, gathered)
     if world > 1:
         t = torch.tensor([ms, e2e_s, e2e_blocking_s, e2e_grouped_s], device="cuda", dtype=torch.float64)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)   # timing: max over ranks

@@ -1,7 +1,8 @@
 #!/usr/bin/env python3
 """Build oracle/_ref/libtempcv_ref.so: the REFERENCE'S OWN Haar code, compiled where it lies.
 
-TEST INFRASTRUCTURE ONLY.  Reads /root/reference/CLFaceDetection/tempcv.{hpp,cpp} (read-only),
+TEST INFRASTRUCTURE ONLY.  Reads tempcv.{hpp,cpp} of the original CLFaceDetection sources, from the
+directory CLFD_REFERENCE_DIR names (read-only),
 copies the line ranges below verbatim into oracle/_ref/*.inc (scratch files in a git-ignored
 directory, deleted again as soon as the compiler has read them) and compiles them together with oracle/ref_shim/ (a test-only stand-in for the few
 OpenCV 2.4 names those ranges touch) and oracle/vj_oracle.c (whose cv2-pinned resize / integral
@@ -28,8 +29,8 @@ clod.cpp as a whole needs the author's un-vendored CLUtil and <OpenCL/opencl.h>)
     clod.cpp    580-787         runClassifier, runClassifierWithPrecomputedFeatures, runSubwindow, runCascade
     clod.cpp   1339-1500        clodDetectObjects
 
-On a machine without /root/reference (the GPU box) nothing is built: the prebuilt .so travels
-with the snapshot, and tests that need it skip if it is absent.
+Without CLFD_REFERENCE_DIR nothing is built: a library already in oracle/_ref is used, and tests
+that need it skip if there is none.
 """
 from __future__ import annotations
 
@@ -39,7 +40,7 @@ import subprocess
 import sys
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF = os.environ.get("CLFD_REFERENCE_DIR", "/root/reference/CLFaceDetection")
+REF = os.environ.get("CLFD_REFERENCE_DIR", "")   # the original CLFaceDetection sources; none by default
 OUT = os.path.join(HERE, "_ref")
 LIB = os.path.join(OUT, "libtempcv_ref.so")
 
@@ -54,7 +55,7 @@ RANGES = {
 SOURCES = ("tempcv.hpp", "tempcv.cpp", "clod.h", "clod.cpp")
 
 def reference_available() -> bool:
-    return all(os.path.exists(os.path.join(REF, f)) for f in SOURCES)
+    return bool(REF) and all(os.path.exists(os.path.join(REF, f)) for f in SOURCES)
 
 
 def _extract() -> None:

@@ -102,10 +102,11 @@ def test_gather_rects_world_size_2_gloo(tmp_path):
 
 def test_reference_main_cpp_compiles_unchanged(tmp_path):
     """SURVEY.md 8-b: the reference's own main.cpp must build against include/ + include/shim
-    byte for byte.  Only possible where /root/reference is mounted (not on the GPU box)."""
-    ref = "/root/reference/CLFaceDetection/main.cpp"
-    if not os.path.exists(ref):
-        pytest.skip("reference tree not present")
+    byte for byte.  Only possible where CLFD_REFERENCE_DIR names the original sources."""
+    from oracle import build_ref
+    ref = os.path.join(build_ref.REF, "main.cpp")
+    if not build_ref.REF or not os.path.exists(ref):
+        pytest.skip("no original main.cpp (CLFD_REFERENCE_DIR)")
     obj = tmp_path / "main.o"
     exe = os.path.join(ROOT, "tests", "_build", "ref_main")
     os.makedirs(os.path.dirname(exe), exist_ok=True)

@@ -35,7 +35,7 @@ def test_clod_cpu_equals_reference_code():
     """fresh frames, min / max window sizes, straight against the reference's compiled clodDetectObjects"""
     from oracle import ref
     if not ref.available():
-        pytest.skip("oracle/_ref not built (no /root/reference on this machine)")
+        pytest.skip("no original sources (CLFD_REFERENCE_DIR) and no library in oracle/_ref")
     rng = np.random.default_rng(5)
     for name in ("frontalface_alt", "eye"):
         oc = oracle.Cascade(cascade_path(name))

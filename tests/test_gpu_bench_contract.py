@@ -38,6 +38,37 @@ def test_native_arm_line():
     assert c["clod_cpu"]["value"] > 0 and c["clod_cpu"]["cores"] >= 1 and c["clod_cpu"]["windows_per_frame"] > 0
 
 
+def test_dump_outputs_holds_the_last_steps_rects(tmp_path):
+    """--dump-outputs: the rects of the last timed step, sorted, as float64; frame 0's are the oracle's"""
+    import numpy as np
+    from clfacedetection_b200.frames import octave_frame
+    from conftest import oracle_cascade
+    d = _run("--steps", "2", "--warmup", "3", "--batch", "4", "--no-cpu-baseline", "--no-extra", "--dump-outputs", str(tmp_path))
+    assert d["steps"] == 2
+    r = np.load(tmp_path / "rects.npy")
+    assert r.dtype == np.float64 and r.shape == (d["rects_per_step"], 6) and len(r) > 0
+    assert np.array_equal(r, r[np.lexsort(r.T[[3, 2, 0, 1, 5, 4]])])
+    assert set(r[:, 4].tolist()) <= {0, 1, 2, 3} and not r[:, 5].any()
+    key = lambda a: a[np.lexsort(a.T[[3, 2, 0, 1]])]
+    want = oracle_cascade("frontalface_alt").detect(octave_frame(1920, 1080, 0), 1.2, want_codes=False)[0]
+    assert np.array_equal(key(r[r[:, 4] == 0][:, :4].astype(np.int32)), key(want))
+
+
+def test_dump_outputs_of_the_stream_arm(tmp_path):
+    """--stream --dump-outputs: the gathered rects of the timed pass over the whole stream; frame 70's are the oracle's"""
+    import numpy as np
+    from clfacedetection_b200 import stream
+    from conftest import oracle_cascade
+    d = _run("--stream", "96", "--batch", "32", "--size", "480x360", "--cascade", "eye", "--dump-outputs", str(tmp_path))
+    r = np.load(tmp_path / "rects.npy")
+    assert r.dtype == np.float64 and r.shape == (d["rects_total"], 6) and len(r) > 0
+    assert np.array_equal(r, r[np.lexsort(r.T[[3, 2, 0, 1, 5, 4]])]) and r[:, 4].max() < 96
+    key = lambda a: a[np.lexsort(a.T[[3, 2, 0, 1]])]
+    frame = np.ascontiguousarray(stream.StreamSource(480, 360, pinned=False).frame(70))
+    want = oracle_cascade("eye").detect(frame, 1.2, want_codes=False)[0]
+    assert np.array_equal(key(r[r[:, 4] == 70][:, :4].astype(np.int32)), key(want))
+
+
 def test_reference_arm_line():
     d = _run("--impl", "reference", "--steps", "1", "--warmup", "1", "--ref-frames", "1")
     assert d["impl"] == "reference" and d["metric"] == "frames_per_sec_1080p" and d["value"] > 0

@@ -67,7 +67,7 @@ def test_clod_demo_scale_cascade_mode_matches_ref_sc(tmp_path):
 def test_reference_main_runs_unchanged():
     exe = os.path.join(ROOT, "tests", "_build", "ref_main")
     if not os.path.exists(exe):
-        pytest.skip("tests/_build/ref_main is built by the CPU suite where /root/reference is mounted")
+        pytest.skip("tests/_build/ref_main is built by the CPU suite where CLFD_REFERENCE_DIR names the original sources")
     out = subprocess.run([exe], capture_output=True, text=True, timeout=300, cwd=ROOT)
     assert out.returncode == 0, out.stderr
     for label in ("OpenCV:", "OpenCL (optimized):", "OpenCL (per-stage):"):

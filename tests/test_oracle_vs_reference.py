@@ -2,8 +2,8 @@
 compiled code -- tempcv.cpp:40-1516, 1702-2089 built by oracle/build_ref.py from where the sources
 lie (oracle/_ref/libtempcv_ref.so).  Everything here runs on the CPU.
 
-Skipped only where neither /root/reference nor a prebuilt oracle/_ref exists; the same comparison
-is then made against the vectors that library produced (tests/test_reference_golden.py).
+Skipped where CLFD_REFERENCE_DIR does not name the original sources and oracle/_ref holds no built
+library; tests/test_reference_golden.py then compares with the vectors that library produced.
 """
 import os
 import tempfile
@@ -17,7 +17,7 @@ from clfacedetection_b200.frames import octave_frame, uniform_frame
 from conftest import ALL_CASCADES, cascade_path, oracle_cascade
 from oracle import ref
 
-pytestmark = pytest.mark.skipif(not ref.available(), reason="no /root/reference and no prebuilt oracle/_ref")
+pytestmark = pytest.mark.skipif(not ref.available(), reason="no original sources (CLFD_REFERENCE_DIR) and no library in oracle/_ref")
 
 _ref_cache = {}
 

@@ -1,7 +1,7 @@
 """The CPU oracle and the product's host code against tests/golden/reference_tempcv.npz -- vectors
 recorded from the REFERENCE'S OWN compiled functions (tempcv.cpp:40-1516, 1702-2089) by
-tests/golden/make_ref_golden.py.  Needs neither /root/reference nor oracle/_ref, so it also runs on
-the GPU box; the CUDA path is compared with the same file in tests/test_gpu_reference_golden.py."""
+tests/golden/make_ref_golden.py.  Needs neither the original sources nor oracle/_ref, so it runs on every
+machine; the CUDA path is compared with the same file in tests/test_gpu_reference_golden.py."""
 import os
 
 import numpy as np
