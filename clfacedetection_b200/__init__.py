@@ -235,6 +235,14 @@ class Detector:
                                                 self._rect_cap, C.byref(n), C.c_void_p(stream) if stream else None))
         return DetectResult(self._rects[:n.value].copy(), self.stats())
 
+    def _geometry(self, frames):
+        """(n_frames, frame stride, row stride) of a uint8 [n, H, W] numpy array or torch tensor of this detector's shape"""
+        n, H, W = frames.shape
+        assert (H, W) == (self.height, self.width)
+        if isinstance(frames, np.ndarray):
+            return n, frames.strides[0], frames.strides[1]
+        return n, frames.stride(0), frames.stride(1)
+
     # ---- host input, end to end (the call a clod user makes) ----------------------------
     def detect(self, frames) -> DetectResult:
         """frames: uint8 [n,H,W] (numpy, or a pinned torch CPU tensor)"""
@@ -242,12 +250,7 @@ class Detector:
             if frames.ndim == 2:
                 frames = frames[None]
             frames = np.ascontiguousarray(frames, np.uint8)
-            n, H, W = frames.shape
-            fs, rs = frames.strides[0], frames.strides[1]
-        else:
-            n, H, W = frames.shape
-            fs, rs = frames.stride(0), frames.stride(1)
-        assert (H, W) == (self.height, self.width)
+        n, fs, rs = self._geometry(frames)
         cnt = C.c_int64()
         abi.check(abi.lib().clfd_detect(self._h, _ptr(frames), n, fs, rs,
                                         self._rects.ctypes.data_as(C.POINTER(abi.Rect)), self._rect_cap, C.byref(cnt)))
@@ -258,12 +261,7 @@ class Detector:
         """frames as for detect(); must stay alive (and should be pinned) until collected"""
         if isinstance(frames, np.ndarray):
             assert frames.ndim == 3 and frames.dtype == np.uint8 and frames.flags.c_contiguous
-            n, H, W = frames.shape
-            fs, rs = frames.strides[0], frames.strides[1]
-        else:
-            n, H, W = frames.shape
-            fs, rs = frames.stride(0), frames.stride(1)
-        assert (H, W) == (self.height, self.width)
+        n, fs, rs = self._geometry(frames)
         abi.check(abi.lib().clfd_detect_submit(self._h, _ptr(frames), n, fs, rs))
 
     def submit_views(self, first_frame, n_frames: int, frame_stride: int, row_stride: int) -> None:

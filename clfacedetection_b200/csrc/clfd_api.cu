@@ -107,8 +107,8 @@ struct PyramidPlan {
     int build(int W_, int H_, const std::vector<std::pair<int, int>> &sizes, int batch, bool tilt, cudaStream_t s);
     void fill_args(PyramidArgs &a, const uint8_t *frames, size_t frame_stride, int row_stride, int n_frames) const;
     // frames: first frame of the range; frame_base: index of that frame in the per-frame device buffers
-    int run(clfd_context *ctx, const uint8_t *frames, size_t frame_stride, int row_stride, int frame_base, int n_frames,
-            cudaStream_t s, cudaEvent_t *ev, int *n_launch);
+    int run(const uint8_t *frames, size_t frame_stride, int row_stride, int frame_base, int n_frames, cudaStream_t s,
+            cudaEvent_t *ev, int *n_launch);
 };
 
 int PyramidPlan::build(int W_, int H_, const std::vector<std::pair<int, int>> &sizes, int batch, bool tilt,
@@ -239,9 +239,9 @@ void PyramidPlan::fill_args(PyramidArgs &a, const uint8_t *frames, size_t frame_
     a.max_level_w = max_level_w;
 }
 
-// ev (optional): 5 events recorded before K1, K2, K3, K4 and after K4
-int PyramidPlan::run(clfd_context *ctx, const uint8_t *frames, size_t frame_stride, int row_stride, int frame_base,
-                     int n_frames, cudaStream_t s, cudaEvent_t *ev, int *n_launch) {
+// ev (optional): 5 events recorded before K1, K2, K3, K4 and after K4; *n_launch: the kernels enqueued
+int PyramidPlan::run(const uint8_t *frames, size_t frame_stride, int row_stride, int frame_base, int n_frames,
+                     cudaStream_t s, cudaEvent_t *ev, int *n_launch) {
     if (n_frames <= 0 || frame_base < 0 || frame_base + n_frames > max_batch)
         INVALID("frames %d..%d outside 0..%d", frame_base, frame_base + n_frames, max_batch);
     if (row_stride < W) INVALID("row stride %d smaller than the frame width %d", row_stride, W);
@@ -253,18 +253,17 @@ int PyramidPlan::run(clfd_context *ctx, const uint8_t *frames, size_t frame_stri
     a.sum += (size_t)frame_base * a.sum_frame_stride;
     a.sq = sq_at(a.sq, (size_t)frame_base * a.sum_frame_stride, sq32);
     if (a.tilted) { a.tilted += (size_t)frame_base * a.sum_frame_stride; a.tcar += (size_t)frame_base * a.tcar_frame_stride; }
-    int launches = 0, nint = 0;
+    int nint = 0, ntilt = 0;
     if (ev) CK(cudaEventRecord(ev[0], s));
-    CK(launch_resize_colsum(a, s)); launches++;
+    CK(launch_resize_colsum(a, s));
     if (ev) CK(cudaEventRecord(ev[1], s));
-    CK(launch_colscan(a, s)); launches++;
+    CK(launch_colscan(a, s));
     if (ev) CK(cudaEventRecord(ev[2], s));
-    CK(launch_integral_rows(a, s, &nint)); launches += nint;
+    CK(launch_integral_rows(a, s, &nint));
     if (ev) CK(cudaEventRecord(ev[3], s));
-    if (want_tilted) { CK(launch_tilted(a, s)); launches += tilted_launches(); }
+    if (want_tilted) CK(launch_tilted(a, s, &ntilt));
     if (ev) CK(cudaEventRecord(ev[4], s));
-    ctx->launches += launches;
-    if (n_launch) *n_launch = launches;
+    *n_launch = 2 + nint + ntilt;
     return 0;
 }
 
@@ -427,16 +426,21 @@ int clfd_context_synchronize(clfd_context *ctx) {
 // ------------------------------------------------------------------------------------
 // cascades
 // ------------------------------------------------------------------------------------
+// a validated HostCascade (hidden cascade built) -> packed device blobs (uploaded per detector, upload_cascade) + its id
+static int publish_cascade(std::unique_ptr<clfd_cascade> c, clfd_cascade **out) {
+    pack_cascade(c->host, c->packed);
+    c->id = g_next_cascade_id.fetch_add(1);
+    *out = c.release();
+    return 0;
+}
+
 int clfd_cascade_load_xml(const char *path, clfd_cascade **out) {
     if (!path || !out) INVALID("NULL argument");
     *out = nullptr;
     std::unique_ptr<clfd_cascade> c(new clfd_cascade());
     int rc = load_cascade_xml(path, c->host);
     if (rc) return rc;
-    pack_cascade(c->host, c->packed);
-    c->id = g_next_cascade_id.fetch_add(1);
-    *out = c.release();
-    return 0;
+    return publish_cascade(std::move(c), out);
 }
 
 int clfd_cascade_from_arrays(int win_w, int win_h, int n_stages, const int *st_ntrees, const float *st_thr,
@@ -480,10 +484,7 @@ int clfd_cascade_from_arrays(int win_w, int win_h, int n_stages, const int *st_n
     h.alpha.assign(alpha, alpha + N + T);
     int rc = build_hidden(h);
     if (rc) return rc;
-    pack_cascade(h, c->packed);
-    c->id = g_next_cascade_id.fetch_add(1);
-    *out = c.release();
-    return 0;
+    return publish_cascade(std::move(c), out);
 }
 
 void clfd_cascade_destroy(clfd_cascade *c) { cascade_release(c); }
@@ -592,9 +593,11 @@ int clfd_integral(clfd_context *ctx, const uint8_t *img, int w, int h, int strid
     if ((rc = in.set(img, w, h, stride, img_on_device, ctx->stream))) return rc;
     const bool keep_tilt = p->want_tilted;
     p->want_tilted = tilted != nullptr;
-    rc = p->run(ctx, in.dev, 0, in.stride, 0, 1, ctx->stream, nullptr, nullptr);
+    int launches = 0;
+    rc = p->run(in.dev, 0, in.stride, 0, 1, ctx->stream, nullptr, &launches);
     p->want_tilted = keep_tilt;
     if (rc) return rc;
+    ctx->launches += launches;
     const PyrLevel &L = p->levels[0];
     const cudaMemcpyKind kind = out_on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost;
     const size_t W1 = (size_t)w + 1;
@@ -723,6 +726,38 @@ static int build_flat_table(clfd_context *ctx, CascadePlan &cp) {
     return 0;
 }
 
+// A detector's copy of its cascade on the device: the generic kernels' global-memory blob and the tile kernel's
+// parameter blobs with this copy's device pointers patched in; with use_patch, also the patch kernel's blob.
+static int upload_cascade(CascadePlan &cp, bool use_patch, cudaStream_t s) {
+    const PackedCascade &pk = cp.cascade->packed;
+    int rc;
+    if ((rc = cp.d_stages.upload(pk.deep_stages, s)) || (rc = cp.d_nodes.upload(pk.deep_nodes, s)) ||
+        (rc = cp.d_tree_first.upload(pk.tree_first_node, s)) || (rc = cp.d_alpha.upload(pk.alpha, s)))
+        return rc;
+    for (int yi = 0; yi < 2; yi++) {
+        cp.dense[yi] = pk.dense[yi];
+        if (!pk.tail[yi].empty() && (rc = cp.d_tail[yi].upload(pk.tail[yi], s))) return rc;
+        cp.dense[yi].tail = cp.d_tail[yi].p;
+        if (!pk.stage_tab[yi].empty() && (rc = cp.d_stage_tab[yi].upload(pk.stage_tab[yi], s))) return rc;
+        cp.dense[yi].stage_g = cp.d_stage_tab[yi].p;
+        if (!use_patch) cp.dense[yi].cut_stages = cp.dense[yi].tail_stages;
+    }
+    cp.use_patch = use_patch;
+    if (use_patch) {
+        cp.patch = pk.patch;
+        if ((rc = cp.d_patch_tail.upload(pk.patch_tail, s))) return rc;
+        cp.patch.tail = cp.d_patch_tail.p;
+    }
+    return 0;
+}
+
+// the tile kernel's grid over one level: kTileW x tile_h windows per CTA, tiles numbered from tile_base -> tile count
+static int plan_tiles(CasLevel &CL, int tile_h, int tile_base) {
+    CL.tiles_x = (CL.nx + kTileW - 1) / kTileW; CL.tiles_y = (CL.ny + tile_h - 1) / tile_h;
+    CL.tile_base = tile_base;
+    return CL.tiles_x * CL.tiles_y;
+}
+
 int clfd_detector_create(clfd_context *ctx, const clfd_cascade *const *cascades, int n_cascades,
                          const clfd_detector_config *cfg, clfd_detector **out) {
     if (!ctx || !cascades || !cfg || !out) INVALID("NULL argument");
@@ -806,9 +841,8 @@ int clfd_detector_create(clfd_context *ctx, const clfd_cascade *const *cascades,
                     CasLevel CL;
                     memset(&CL, 0, sizeof CL);
                     CL.pyr_level = 0; CL.nx = L.nx; CL.ny = L.ny; CL.ystep = 2; CL.win_w = L.win_w; CL.win_h = L.win_h;
-                    CL.tiles_x = (L.nx + kTileW - 1) / kTileW; CL.tiles_y = (L.ny + t->P.tile_h - 1) / t->P.tile_h;
-                    CL.tile_base = tile_base; CL.win_base = L.win_base; CL.factor = L.factor;
-                    t->tile_base = tile_base; t->n_tiles = CL.tiles_x * CL.tiles_y;
+                    CL.win_base = L.win_base; CL.factor = L.factor;
+                    t->tile_base = tile_base; t->n_tiles = plan_tiles(CL, t->P.tile_h, tile_base);
                     tile_base += t->n_tiles;
                     tl.push_back(CL);
                     cp.sc_tiles.push_back(std::move(t));
@@ -850,9 +884,8 @@ int clfd_detector_create(clfd_context *ctx, const clfd_cascade *const *cascades,
             CL.pyr_level = pyr_index[k];
             CL.nx = nx; CL.ny = ny; CL.ystep = ystep; CL.win_w = win_w; CL.win_h = win_h;
             const int tile_h = cp.cascade->packed.dense[ystep - 1].tile_h > 0 ? cp.cascade->packed.dense[ystep - 1].tile_h : kTileH;
-            CL.tiles_x = (nx + kTileW - 1) / kTileW; CL.tiles_y = (ny + tile_h - 1) / tile_h;
-            CL.tile_base = cp.n_tiles; CL.win_base = cp.windows_per_frame; CL.factor = factor;
-            cp.n_tiles += CL.tiles_x * CL.tiles_y;
+            CL.win_base = cp.windows_per_frame; CL.factor = factor;
+            cp.n_tiles += plan_tiles(CL, tile_h, cp.n_tiles);
             if (ystep == 2) cp.n_tiles_y2 = cp.n_tiles;
             cp.windows_per_frame += (long long)nx * ny;
             cp.bytes_cascade += (int64_t)(sz_w + 1) * (sz_h + 1) * (4 + 8 + (hc.has_tilted ? 4 : 0));
@@ -884,25 +917,8 @@ int clfd_detector_create(clfd_context *ctx, const clfd_cascade *const *cascades,
     for (auto &cpp : det->cas) {
         CascadePlan &cp = *cpp;
         const PackedCascade &pk = cp.cascade->packed;
-        if ((rc = cp.d_levels.upload(cp.levels, s)) || (rc = cp.d_stages.upload(pk.deep_stages, s)) ||
-            (rc = cp.d_nodes.upload(pk.deep_nodes, s)) || (rc = cp.d_tree_first.upload(pk.tree_first_node, s)) ||
-            (rc = cp.d_alpha.upload(pk.alpha, s)))
-            return rc;
-        for (int yi = 0; yi < 2; yi++) {
-            cp.dense[yi] = pk.dense[yi];
-            if (!pk.tail[yi].empty() && (rc = cp.d_tail[yi].upload(pk.tail[yi], s))) return rc;
-            cp.dense[yi].tail = cp.d_tail[yi].p;
-            if (!pk.stage_tab[yi].empty() && (rc = cp.d_stage_tab[yi].upload(pk.stage_tab[yi], s))) return rc;
-            cp.dense[yi].stage_g = cp.d_stage_tab[yi].p;
-        }
-        cp.use_patch = !scale_cascade && pk.patch_cut > 0;
-        if (cp.use_patch) {
-            cp.patch = pk.patch;
-            if ((rc = cp.d_patch_tail.upload(pk.patch_tail, s)) || (rc = cp.d_qcount.alloc((size_t)kSlots * std::max(cfg->max_batch, 1)))) return rc;
-            cp.patch.tail = cp.d_patch_tail.p;
-        } else {
-            for (int yi = 0; yi < 2; yi++) cp.dense[yi].cut_stages = cp.dense[yi].tail_stages;
-        }
+        if ((rc = cp.d_levels.upload(cp.levels, s)) || (rc = upload_cascade(cp, !scale_cascade && pk.patch_cut > 0, s))) return rc;
+        if (cp.use_patch && (rc = cp.d_qcount.alloc((size_t)kSlots * std::max(cfg->max_batch, 1)))) return rc;
         if ((rc = cp.d_counters.alloc(kCnt * kSlots)) || (rc = cp.d_count_b.alloc(kSlots))) return rc;
         // mid kernel: the stages right after the tile prefix of a LINEAR cascade whose trees the tile
         // kernel cannot take, while they are too small for a warp per window (< 24 trees), at most 8
@@ -981,6 +997,31 @@ int clfd_detector_set_profiling(clfd_detector *det, int enable) {
     return 0;
 }
 
+// What every cascade kernel reads for frames [frame_base, frame_base + n_frames): the detector's integral images
+// (pre-offset to frame_base), the cascade's level table and its global-memory blob.
+static CascadeArgs cascade_args(const clfd_detector *det, const CascadePlan &cp, int ci, int frame_base, int n_frames) {
+    const PyramidPlan &pyr = det->pyr;
+    const HostCascade &hc = cp.cascade->host;
+    const size_t fo = (size_t)frame_base * pyr.sum_frame_stride;
+    CascadeArgs a;
+    memset(&a, 0, sizeof a);
+    a.sum = pyr.sum.p + fo; a.sq = sq_at(pyr.sq.p, fo, pyr.sq32); a.sq32 = pyr.sq32 ? 1 : 0;
+    a.tilted = pyr.want_tilted ? pyr.tilted.p + fo : nullptr;
+    a.sum_frame_stride = pyr.sum_frame_stride;
+    a.sum_di = det->sum_di ? 1 : 0;
+    a.levels = pyr.d_levels.p; a.cas_levels = cp.d_levels.p;
+    a.n_cas_levels = (int)cp.levels.size(); a.n_tiles = cp.n_tiles; a.n_frames = n_frames;
+    a.frame_base = frame_base;
+    a.cascade_index = ci; a.windows_per_frame = cp.windows_per_frame;
+    a.deep.stages = cp.d_stages.p; a.deep.tree_first_node = cp.d_tree_first.p;
+    a.deep.nodes = cp.d_nodes.p; a.deep.alpha = cp.d_alpha.p;
+    a.deep.n_stages = hc.n_stages(); a.deep.is_tree = hc.is_tree; a.deep.has_tilted = hc.has_tilted;
+    a.deep.win_w = hc.win_w; a.deep.win_h = hc.win_h;
+    a.deep.inv_area = cp.cascade->packed.dense[0].inv_area;
+    a.deep.mid_begin = cp.mid_begin; a.deep.mid_end = cp.mid_end;
+    return a;
+}
+
 // Enqueue every kernel for frames [frame_base, frame_base + n_frames) of the current batch.
 // `first` resets the batch's rect / overflow counters; the kernels see frame numbers relative
 // to the range (the per-frame buffers are passed pre-offset) and add frame_base to the frame
@@ -993,10 +1034,9 @@ static int enqueue_range(clfd_detector *det, const uint8_t *frames_dev, int fram
     int launches = 0;
     cudaEvent_t *ev = det->profiling ? det->ev : nullptr;
     if (!det->pyr.levels.empty() && (parts & kPartPyramid)) {
-        int rc = det->pyr.run(ctx, frames_dev, frame_stride, row_stride, frame_base, n_frames, s, ev, &launches);
+        int rc = det->pyr.run(frames_dev, frame_stride, row_stride, frame_base, n_frames, s, ev, &launches);
         if (rc) return rc;
     }
-    const int pyr_launches = launches;
     if (parts & kPartCounters)
         for (auto &cpp : det->cas) {
             if (first) CK(cudaMemsetAsync(cpp->d_counters.p + kCnt * slot, 0, kCnt * sizeof(unsigned long long), s));
@@ -1004,6 +1044,7 @@ static int enqueue_range(clfd_detector *det, const uint8_t *frames_dev, int fram
             CK(cudaMemsetAsync(cpp->d_count_b.p + slot, 0, sizeof(unsigned long long), s));
         }
     if (!(parts & (kPartCascades | kPartPatch))) {
+        ctx->launches += launches;
         *n_launches += launches;
         return 0;
     }
@@ -1012,17 +1053,7 @@ static int enqueue_range(clfd_detector *det, const uint8_t *frames_dev, int fram
         CascadePlan &cp = *cpp;
         if (cp.windows_per_frame > 0) {
             const PackedCascade &pk = cp.cascade->packed;
-            const size_t fo = (size_t)frame_base * det->pyr.sum_frame_stride;
-            CascadeArgs a;
-            memset(&a, 0, sizeof a);
-            a.sum = det->pyr.sum.p + fo; a.sq = sq_at(det->pyr.sq.p, fo, det->pyr.sq32); a.sq32 = det->pyr.sq32 ? 1 : 0;
-            a.tilted = det->pyr.want_tilted ? det->pyr.tilted.p + fo : nullptr;
-            a.sum_frame_stride = det->pyr.sum_frame_stride;
-            a.sum_di = det->sum_di ? 1 : 0;
-            a.levels = det->pyr.d_levels.p; a.cas_levels = cp.d_levels.p;
-            a.n_cas_levels = (int)cp.levels.size(); a.n_tiles = cp.n_tiles; a.n_frames = n_frames;
-            a.frame_base = frame_base;
-            a.cascade_index = ci; a.windows_per_frame = cp.windows_per_frame;
+            CascadeArgs a = cascade_args(det, cp, ci, frame_base, n_frames);
             a.codes = det->cfg.want_codes ? cp.d_codes.p + (size_t)frame_base * cp.windows_per_frame : nullptr;
             a.count_exact = det->cfg.want_codes ? 1 : 0;
             a.queue = det->queue.p; a.queue_cap = det->queue_cap;
@@ -1035,13 +1066,6 @@ static int enqueue_range(clfd_detector *det, const uint8_t *frames_dev, int fram
                 a.qcount = cp.d_qcount.p + (size_t)slot * det->cfg.max_batch + frame_base;
                 if (parts & kPartCascades) CK(cudaMemsetAsync(a.qcount, 0, sizeof(unsigned long long), s));
             }
-            a.deep.stages = cp.d_stages.p; a.deep.tree_first_node = cp.d_tree_first.p;
-            a.deep.nodes = cp.d_nodes.p; a.deep.alpha = cp.d_alpha.p;
-            a.deep.n_stages = cp.cascade->host.n_stages(); a.deep.is_tree = cp.cascade->host.is_tree;
-            a.deep.has_tilted = cp.cascade->host.has_tilted;
-            a.deep.win_w = cp.cascade->host.win_w; a.deep.win_h = cp.cascade->host.win_h;
-            a.deep.inv_area = pk.dense[0].inv_area;
-            a.deep.mid_begin = cp.mid_begin; a.deep.mid_end = cp.mid_end;
             a.deep_in = a.queue; a.deep_count = a.counters + 1;
             if (det->cfg.mode == CLFD_MODE_SCALE_CASCADE) {
                 ScArgs sa;
@@ -1147,9 +1171,7 @@ static int enqueue_range(clfd_detector *det, const uint8_t *frames_dev, int fram
                     int in = pk.dense[0].tail_stages > 0 ? 0 : -1;   // -1: the grid
                     for (size_t k = 0; k + 1 < cp.mid_cuts.size(); k++) {
                         const int out = in == 0 ? 1 : 0;
-                        if (k > 0 || in == 0) { /* the output queue may hold an older pass: start it empty */
-                            if (!(k == 0)) CK(cudaMemsetAsync(cs[out], 0, sizeof(unsigned long long), s));
-                        }
+                        if (k > 0) CK(cudaMemsetAsync(cs[out], 0, sizeof(unsigned long long), s));   // holds an older pass
                         a.mid_in = in < 0 ? nullptr : qs[in]; a.mid_in_count = in < 0 ? nullptr : cs[in];
                         a.mid_out = qs[out]; a.mid_out_count = cs[out];
                         a.deep.mid_begin = cp.mid_cuts[k]; a.deep.mid_end = cp.mid_cuts[k + 1];
@@ -1170,7 +1192,7 @@ static int enqueue_range(clfd_detector *det, const uint8_t *frames_dev, int fram
         ci++;
     }
     det->have_events = ev != nullptr;
-    ctx->launches += launches - pyr_launches;   // PyramidPlan::run counted its own
+    ctx->launches += launches;
     *n_launches += launches;
     return 0;
 }
@@ -1265,6 +1287,41 @@ int clfd_detector_enqueue(clfd_detector *det, const uint8_t *frames_dev, int n_f
     return 0;
 }
 
+// The device counters of one finished batch (kCnt per cascade at hc, copied back) -> det->stats and the rect count;
+// fails on a survivor-queue or rect-buffer overflow.
+static int take_counters(clfd_detector *det, const unsigned long long *hc, int n_frames, int64_t *n_rects) {
+    const int nc = (int)det->cas.size();
+    const unsigned long long total = hc[kCnt * (nc - 1)];   // all cascades append to one rect buffer
+    unsigned long long deep = 0, rect_over = 0, queue_over = 0;
+    for (int ci = 0; ci < nc; ci++) {
+        memcpy(det->cas[ci]->h_counters, hc + kCnt * ci, kCnt * sizeof(unsigned long long));
+        deep += hc[kCnt * ci + 1];
+        rect_over += hc[kCnt * ci + 2];
+        queue_over += hc[kCnt * ci + 3];
+    }
+    if (queue_over) { set_error("survivor queue overflow (%llu windows dropped)", queue_over); return CLFD_ERR_CAPACITY; }
+    det->stats.rects = (int64_t)total;
+    det->stats.deep_windows = (int64_t)deep;
+    det->stats.exact_stage_evals = det->stats.near_threshold_events = det->cfg.want_codes ? 0 : -1;   // -1: not counted
+    for (int ci = 0; ci < nc && det->cfg.want_codes; ci++) {
+        det->stats.exact_stage_evals += (int64_t)hc[kCnt * ci + 4];
+        det->stats.near_threshold_events += (int64_t)hc[kCnt * ci + 5];
+    }
+#ifdef CLFD_TILE_TIMING   // diagnostic build: the tile kernel's warp-slot accounting in place of the three counters
+    det->stats.exact_stage_evals = (int64_t)hc[4];
+    det->stats.near_threshold_events = (int64_t)hc[5];
+    det->stats.deep_windows = (int64_t)hc[6];
+#endif
+    det->stats.windows = 0;
+    for (auto &cpp : det->cas) det->stats.windows += cpp->windows_per_frame * n_frames;
+    *n_rects = (int64_t)total;
+    if (rect_over || total > det->rect_cap) {
+        set_error("device rect buffer overflow: %llu accepted windows, capacity %llu (raise max_rects)", total, det->rect_cap);
+        return CLFD_ERR_CAPACITY;
+    }
+    return 0;
+}
+
 int clfd_detector_fetch(clfd_detector *det, clfd_rect *rects, int64_t cap, int64_t *n_rects, void *cuda_stream) {
     if (!det || !n_rects) INVALID("NULL argument");
     clfd_context *ctx = det->ctx;
@@ -1275,34 +1332,9 @@ int clfd_detector_fetch(clfd_detector *det, clfd_rect *rects, int64_t cap, int64
         CK(cudaMemcpyAsync(det->h_counters + kCnt * ci, det->cas[ci]->d_counters.p, kCnt * sizeof(unsigned long long),
                            cudaMemcpyDeviceToHost, s));
     CK(cudaStreamSynchronize(s));
-    unsigned long long total = det->h_counters[kCnt * (nc - 1)];
-    unsigned long long deep = 0, rect_over = 0, queue_over = 0;
-    for (int ci = 0; ci < nc; ci++) {
-        memcpy(det->cas[ci]->h_counters, det->h_counters + kCnt * ci, kCnt * sizeof(unsigned long long));
-        deep += det->h_counters[kCnt * ci + 1];
-        rect_over += det->h_counters[kCnt * ci + 2];
-        queue_over += det->h_counters[kCnt * ci + 3];
-    }
-    if (queue_over) { set_error("survivor queue overflow (%llu windows dropped)", queue_over); return CLFD_ERR_CAPACITY; }
-    det->stats.rects = (int64_t)total;
-    det->stats.deep_windows = (int64_t)deep;
-    det->stats.exact_stage_evals = det->stats.near_threshold_events = det->cfg.want_codes ? 0 : -1;   // -1: not counted
-    for (int ci = 0; ci < nc && det->cfg.want_codes; ci++) {
-        det->stats.exact_stage_evals += (int64_t)det->h_counters[kCnt * ci + 4];
-        det->stats.near_threshold_events += (int64_t)det->h_counters[kCnt * ci + 5];
-    }
-#ifdef CLFD_TILE_TIMING   // diagnostic build: the tile kernel's warp-slot accounting in place of the three counters
-    det->stats.exact_stage_evals = (int64_t)det->h_counters[4];
-    det->stats.near_threshold_events = (int64_t)det->h_counters[5];
-    det->stats.deep_windows = (int64_t)det->h_counters[6];
-#endif
-    det->stats.windows = 0;
-    for (auto &cpp : det->cas) det->stats.windows += cpp->windows_per_frame * det->last_frames;
-    *n_rects = (int64_t)total;
-    if (rect_over || total > det->rect_cap) {
-        set_error("device rect buffer overflow: %llu accepted windows, capacity %llu (raise max_rects)", total, det->rect_cap);
-        return CLFD_ERR_CAPACITY;
-    }
+    int rc = take_counters(det, det->h_counters, det->last_frames, n_rects);
+    if (rc) return rc;
+    const unsigned long long total = (unsigned long long)*n_rects;
     if (det->have_events) {
         // [0] resize+colsum [1] colscan [2] integral rows [3] tilted [4] tile kernel [5] deep kernel
         cudaEventElapsedTime(&det->kernel_ms[0], det->ev[0], det->ev[1]);
@@ -1345,7 +1377,7 @@ int clfd_detect_submit(clfd_detector *det, const uint8_t *frames_host, int n_fra
         if (!det->h_rects1) CK(cudaMallocHost((void **)&det->h_rects1, (size_t)kEagerRects * sizeof(DevRect)));
     }
     int n_chunks = 1;
-    if (det->cas.size() == 1 && n_frames >= 8) n_chunks = n_frames >= 32 ? 4 : 2;
+    if (n_frames >= 8) n_chunks = n_frames >= 32 ? 4 : 2;
     // with a batch already in flight the whole copy overlaps THAT batch's compute: no need to
     // pay the extra kernel boundaries of a cut
     if (det->n_submitted > det->n_collected) n_chunks = 1;
@@ -1415,36 +1447,9 @@ int clfd_detect_collect(clfd_detector *det, clfd_rect *rects, int64_t cap, int64
     const int slot = (int)(det->n_collected % kSlots);
     det->n_collected++;
     CK(cudaEventSynchronize(det->done[slot]));
-    const int nc = (int)det->cas.size();
-    const unsigned long long *hc = det->h_counters + (size_t)slot * kCnt * 16;
-    const unsigned long long total = hc[kCnt * (nc - 1)];
-    unsigned long long deep = 0, rect_over = 0, queue_over = 0;
-    for (int ci = 0; ci < nc; ci++) {
-        memcpy(det->cas[ci]->h_counters, hc + kCnt * ci, kCnt * sizeof(unsigned long long));
-        deep += hc[kCnt * ci + 1];
-        rect_over += hc[kCnt * ci + 2];
-        queue_over += hc[kCnt * ci + 3];
-    }
-    if (queue_over) { set_error("survivor queue overflow (%llu windows dropped)", queue_over); return CLFD_ERR_CAPACITY; }
-    det->stats.rects = (int64_t)total;
-    det->stats.deep_windows = (int64_t)deep;
-    det->stats.exact_stage_evals = det->stats.near_threshold_events = det->cfg.want_codes ? 0 : -1;   // -1: not counted
-    for (int ci = 0; ci < nc && det->cfg.want_codes; ci++) {
-        det->stats.exact_stage_evals += (int64_t)hc[kCnt * ci + 4];
-        det->stats.near_threshold_events += (int64_t)hc[kCnt * ci + 5];
-    }
-#ifdef CLFD_TILE_TIMING
-    det->stats.exact_stage_evals = (int64_t)hc[4];
-    det->stats.near_threshold_events = (int64_t)hc[5];
-    det->stats.deep_windows = (int64_t)hc[6];
-#endif
-    det->stats.windows = 0;
-    for (auto &cpp : det->cas) det->stats.windows += cpp->windows_per_frame * det->slot_frames[slot];
-    *n_rects = (int64_t)total;
-    if (rect_over || total > det->rect_cap) {
-        set_error("device rect buffer overflow: %llu accepted windows, capacity %llu (raise max_rects)", total, det->rect_cap);
-        return CLFD_ERR_CAPACITY;
-    }
+    int rc = take_counters(det, det->h_counters + (size_t)slot * kCnt * 16, det->slot_frames[slot], n_rects);
+    if (rc) return rc;
+    const unsigned long long total = (unsigned long long)*n_rects;
     if (total == 0 || !rects) return 0;
     if ((int64_t)total > cap) { set_error("rect buffer too small: need %llu, have %lld", total, (long long)cap); return CLFD_ERR_CAPACITY; }
     static_assert(sizeof(DevRect) == sizeof(clfd_rect), "rect layout");
@@ -1518,21 +1523,8 @@ int clfd_detector_reject_levels(clfd_detector *det, int cascade, clfd_rect *rect
     int rc;
     const unsigned long long roc_cap = 1ull << 20;
     if (!det->roc.p && ((rc = det->roc.alloc(roc_cap)) || (rc = det->roc_count.alloc(1)))) return rc;
-    CascadeArgs a;
-    memset(&a, 0, sizeof a);
-    a.sum = det->pyr.sum.p; a.sq = det->pyr.sq.p; a.sq32 = det->pyr.sq32 ? 1 : 0;
-    a.tilted = det->pyr.want_tilted ? det->pyr.tilted.p : nullptr;
-    a.sum_frame_stride = det->pyr.sum_frame_stride;
-    a.levels = det->pyr.d_levels.p; a.cas_levels = cp.d_levels.p;
-    a.n_cas_levels = (int)cp.levels.size(); a.n_frames = det->last_frames;
-    a.cascade_index = cascade; a.windows_per_frame = cp.windows_per_frame;
+    CascadeArgs a = cascade_args(det, cp, cascade, 0, det->last_frames);
     a.codes = cp.d_codes.p;
-    a.deep.stages = cp.d_stages.p; a.deep.tree_first_node = cp.d_tree_first.p;
-    a.deep.nodes = cp.d_nodes.p; a.deep.alpha = cp.d_alpha.p;
-    a.deep.n_stages = cp.cascade->host.n_stages(); a.deep.is_tree = cp.cascade->host.is_tree;
-    a.deep.has_tilted = cp.cascade->host.has_tilted;
-    a.deep.win_w = cp.cascade->host.win_w; a.deep.win_h = cp.cascade->host.win_h;
-    a.deep.inv_area = cp.cascade->packed.dense[0].inv_area;
     CK(cudaMemsetAsync(det->roc_count.p, 0, sizeof(unsigned long long), ctx->stream));
     CK(launch_roc_collect(a, det->roc.p, roc_cap, det->roc_count.p, ctx->stream));
     ctx->launches++;

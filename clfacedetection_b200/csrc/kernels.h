@@ -60,9 +60,9 @@ struct SmemLimitCache {
 
 cudaError_t launch_resize_colsum(const PyramidArgs &a, cudaStream_t stream);
 cudaError_t launch_colscan(const PyramidArgs &a, cudaStream_t stream);
+// these two enqueue several kernels: *n_launches is how many
 cudaError_t launch_integral_rows(const PyramidArgs &a, cudaStream_t stream, int *n_launches);
-cudaError_t launch_tilted(const PyramidArgs &a, cudaStream_t stream);
-int tilted_launches();       // kernels launch_tilted enqueues
+cudaError_t launch_tilted(const PyramidArgs &a, cudaStream_t stream, int *n_launches);
 int tilt_tile_interior();    // output columns per warp tile of k_tilt_tiles
 
 cudaError_t launch_bgr_to_gray(const uint8_t *bgr, int w, int h, int stride, int channels,
@@ -100,16 +100,14 @@ cudaError_t launch_enqueue_all(const CascadeArgs &a, cudaStream_t stream);
 // thread-per-window evaluation of stages [deep.mid_begin, deep.mid_end) (generic trees), survivors -> queue_b
 cudaError_t launch_cascade_mid(const CascadeArgs &a, int n_sms, cudaStream_t stream);
 // warp-per-window evaluation of the queue
+cudaError_t launch_cascade_deep(const CascadeArgs &a, int n_sms, cudaStream_t stream);
 // reject-level output: scans the exit codes of n_frames frames, appends the candidates of
 // tempcv.cpp:1084-1094 (count at counter[0]) with the exact stage sum of their last stage
 cudaError_t launch_roc_collect(const CascadeArgs &a, RocItem *out, unsigned long long cap, unsigned long long *counter, cudaStream_t stream);
-cudaError_t launch_cascade_deep(const CascadeArgs &a, int n_sms, cudaStream_t stream);
 
 // the survivors the tile kernel handed over at DenseParams::cut_stages, a warp per window
 // P: the cascade's patch blob (PackedCascade::patch: records in patch layout)
 cudaError_t launch_cascade_patch(const DenseParams &P, const CascadeArgs &a, int n_sms, cudaStream_t stream);
-
-size_t dense_smem_bytes(const DenseParams &P);
 
 // ---- scale-cascade mode (kernels_sc.cu) -----------------------------------------------
 struct ScArgs {

@@ -725,8 +725,10 @@ __global__ void __launch_bounds__(256) k_tilt_tcarry(const PyramidArgs a) {
     if (X <= L.w) car[kTcTC * ps + (size_t)(L.nrb - 1) * L.sum_pitch + X] = acc;
 }
 
-cudaError_t launch_tilted(const PyramidArgs &a, cudaStream_t stream) {
+cudaError_t launch_tilted(const PyramidArgs &a, cudaStream_t stream, int *n_launches) {
+    *n_launches = 0;
     if (a.n_tilt_tile_items == 0 || a.n_frames == 0 || !a.tilted) return cudaSuccess;
+    *n_launches = 4;
     const dim3 tiles((a.n_tilt_tile_items + kTiltWarps - 1) / kTiltWarps, a.n_frames);
     const size_t smem = (size_t)kTiltWarps * kTiltSmemLocal;
     static SmemLimitCache lim_local, lim_final;
@@ -738,7 +740,6 @@ cudaError_t launch_tilted(const PyramidArgs &a, cudaStream_t stream) {
     k_tilt_tiles<true><<<tiles, 32 * kTiltWarps, smem, stream>>>(a);
     return cudaGetLastError();
 }
-int tilted_launches() { return 4; }
 int tilt_tile_interior() { return kTiltInterior; }
 
 // ------------------------------------------------------------------------------------

@@ -183,7 +183,6 @@ __host__ __device__ inline DenseSmemPlan dense_smem_plan(const DenseParams &P) {
 constexpr bool kTilesCount = true;
 #else
 constexpr bool kTilesCount = false;
-size_t dense_smem_bytes(const DenseParams &P) { return dense_smem_plan(P).total; }
 #endif
 
 struct DenseCtx {
