@@ -35,6 +35,8 @@ static inline int cv_round(double v) { return (int)lrint(v); }
 static inline int cv_floor(double v) { int i = (int)v; return i - (i > v); }
 static inline size_t round_up(size_t v, size_t m) { return (v + m - 1) / m * m; }
 
+constexpr int kMaxPyramidWindow = 255;   // largest cascade window (either side) of the image-pyramid mode
+
 // ------------------------------------------------------------------------------------
 // objects
 // ------------------------------------------------------------------------------------
@@ -782,6 +784,12 @@ int clfd_detector_create(clfd_context *ctx, const clfd_cascade *const *cascades,
     bool any_tilted = false;
     for (int ci = 0; ci < n_cascades; ci++) {
         if (!cascades[ci]) INVALID("cascade %d is NULL", ci);
+        // the image-pyramid kernels keep a window's corner offsets in bytes (DeepNode) and its squared integral modulo
+        // 2^32, exact while (w - 2)(h - 2) * 255^2 < 2^32; the scale-cascade mode has neither limit
+        const HostCascade &hc = cascades[ci]->host;
+        if (!scale_cascade && (hc.win_w > kMaxPyramidWindow || hc.win_h > kMaxPyramidWindow))
+            INVALID("cascade %d: window %dx%d is larger than %d pixels, the limit of the image-pyramid mode (the "
+                    "scale-cascade mode takes it)", ci, hc.win_w, hc.win_h, kMaxPyramidWindow);
         det->cas.emplace_back(new CascadePlan());
         det->cas.back()->cascade = cascades[ci];
         const_cast<clfd_cascade *>(cascades[ci])->refs.fetch_add(1);   // released by ~CascadePlan

@@ -262,8 +262,10 @@ void pack_sc_level(const HostCascade &c, double scale, int pitch, ScLevel &L, Sc
 // of stage i-1 with no `next` alternative).  Every eligible stump gets a TailStump record
 // (global memory, warp-autonomous phase); the stumps of the first n_fixed stages are also
 // parameter resident (DenseStump, fixed-geometry phase).
+// allow_tiles = false: no stage for the tile kernel (tail_stages = exec_stages = 0), the generic kernels take the cascade.
 static void pack_dense_one(const HostCascade &c, int ystep, DenseParams &P, std::vector<TailStump> &tail,
-                           std::vector<DenseStage> &stage_tab, int &dense_stumps, int patch_stride = 0) {
+                           std::vector<DenseStage> &stage_tab, int &dense_stumps, int patch_stride = 0,
+                           bool allow_tiles = true) {
     const int S = c.n_stages(), T = c.n_trees();
     memset(&P, 0, sizeof P);
     P.total_stages = S;
@@ -291,7 +293,7 @@ static void pack_dense_one(const HostCascade &c, int ystep, DenseParams &P, std:
     }
     const size_t tile_bytes = (size_t)dense_tile_rows(c.win_h, ystep, P.tile_h) * P.tile_stride * 4;
     const size_t tilt_base = (tile_bytes + 127) & ~(size_t)127;
-    const bool dense_ok = tile_bytes <= 65536 && (!P.tilted_tile || 2 * tilt_base <= 160 * 1024) && c.win_w <= 255 && c.win_h <= 255;
+    const bool dense_ok = allow_tiles && tile_bytes <= 65536 && (!P.tilted_tile || 2 * tilt_base <= 160 * 1024) && c.win_w <= 255 && c.win_h <= 255;
     // multi-node trees (<= kMaxTreeNodes nodes, children after their parent) are evaluated node by node
     // with a per-window "node I am at" state; every tree is padded to npt = the cascade's largest tree
     int npt = 1;
@@ -528,6 +530,15 @@ void pack_cascade(const HostCascade &c, PackedCascade &out) {
     }
 
     for (int yi = 0; yi < 2; yi++) pack_dense_one(c, yi + 1, out.dense[yi], out.tail[yi], out.stage_tab[yi], out.dense_stumps);
+    // Both blobs hand the tile kernel the same stages.  The host code decides from dense[0] alone whether a cascade has a
+    // tile prefix, whether the tile kernel finishes it (no mid / deep kernels then, chunk overlap, the flat-window table:
+    // enqueue_range, overlap_applies, build_flat_table in clfd_api.cu), but launches the ystep-2 levels' tiles with
+    // dense[1].  The ystep-2 tile spans twice the rows and columns of windows, so it stops fitting shared memory at a
+    // smaller window (45 x 45 for a plain stump cascade, 44 x 44 fits): when either tile does not fit, neither row step
+    // uses the tile kernel and the generic kernels take the whole cascade on every level.
+    if (out.dense[0].tail_stages != out.dense[1].tail_stages || out.dense[0].exec_stages != out.dense[1].exec_stages)
+        for (int yi = 0; yi < 2; yi++)
+            pack_dense_one(c, yi + 1, out.dense[yi], out.tail[yi], out.stage_tab[yi], out.dense_stumps, 0, false);
     // Patch kernel (A/B hook, OFF by default: CLFD_PATCH_CUT=n switches it on).  A window that survives the first stages
     // is rare and goes deep: finished inside the tile kernel it keeps one warp busy for tens of microseconds while the
     // CTA's other warps have nothing left (15 % of the tile kernel's warp slots, tools/tile_timing.py).  With a cut the
