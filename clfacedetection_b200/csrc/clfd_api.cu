@@ -1560,12 +1560,14 @@ int clfd_detector_read_level(clfd_detector *det, int cascade, int level, int fra
                              uint64_t *sqsum, int32_t *tilted) {
     if (!det || cascade < 0 || cascade >= (int)det->cas.size()) INVALID("bad argument");
     CascadePlan &cp = *det->cas[cascade];
-    if (level < 0 || level >= (int)cp.levels.size()) INVALID("level %d outside 0..%zu", level, cp.levels.size());
+    // pub_levels: the scale-cascade planner fills no CasLevel list; every one of its scales reads pyramid level 0
+    if (level < 0 || level >= (int)cp.pub_levels.size()) INVALID("level %d outside 0..%zu", level, cp.pub_levels.size());
     if (frame < 0 || frame >= det->last_frames) INVALID("frame %d outside the last batch", frame);
     if (tilted && !det->pyr.want_tilted) INVALID("detector has no tilted integral (no cascade with tilted features)");
     CK(cudaSetDevice(det->ctx->device));
     CK(cudaDeviceSynchronize());
-    const PyrLevel &L = det->pyr.levels[cp.levels[level].pyr_level];
+    const bool scale_cascade = det->cfg.mode == CLFD_MODE_SCALE_CASCADE;
+    const PyrLevel &L = det->pyr.levels[scale_cascade ? 0 : cp.levels[level].pyr_level];
     const size_t W1 = (size_t)L.w + 1;
     const size_t so = (size_t)frame * det->pyr.sum_frame_stride + L.sum_off;
     if (pyr) CK(cudaMemcpy2D(pyr, L.w, det->pyr.pyr.p + (size_t)frame * det->pyr.pyr_frame_stride + L.pyr_off, L.pyr_pitch, L.w, L.h, cudaMemcpyDeviceToHost));

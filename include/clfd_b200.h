@@ -245,7 +245,11 @@ CLFD_API int clfd_detector_get_codes(clfd_detector *det, int cascade, int16_t *c
  * A pyramid-mode detector keeps its squared integral modulo 2^32 (all it ever needs are windows'
  * sums of squares, which are below 2^32): sqsum then returns those low words, widened.  It also stores the
  * int32 integral of the levels whose windows are 2 pixels apart column-de-interleaved (the tile kernel's
- * shared-memory order); `sum` is handed back in the natural order regardless. */
+ * shared-memory order); `sum` is handed back in the natural order regardless.
+ * A scale-cascade detector has one image, the frame itself: every level 0 .. num_levels-1 reads it
+ * (pyr = the frame, the natural-order sum, the full 64-bit sqsum and, with tilted features, tilted).
+ * sum and tilted are int32 like the reference's CV_32S integrals: on a frame whose pixels add up to
+ * 2^31 or more they wrap modulo 2^32; the kernels only ever use differences of them (window sums). */
 CLFD_API int clfd_detector_read_level(clfd_detector *det, int cascade, int level, int frame,
                                       uint8_t *pyr, int32_t *sum, uint64_t *sqsum,
                                       int32_t *tilted);

@@ -10,15 +10,25 @@ pytestmark = pytest.mark.gpu
 
 
 def _check_integral(ctx, img, tilted):
+    """against the oracle and against numpy: int64 sums wrapped to int32 (the CV_32S integrals wrap once a frame's
+    pixels add up to 2^31; the oracle's int32 adds alone are not relied on for that) and exact uint64 squares"""
     s, q, t = ctx.integral(img, tilted=tilted)
     os_, oq, ot = oracle.integral(img, tilted=tilted)
     assert np.array_equal(s, os_)
     assert np.array_equal(q, oq.astype(np.uint64))
     if tilted:
         assert np.array_equal(t, ot)
+    ref = np.zeros(s.shape, np.int64)
+    ref[1:, 1:] = img.astype(np.int64).cumsum(0).cumsum(1)
+    assert np.array_equal(s, (ref & 0xFFFFFFFF).astype(np.uint32).view(np.int32))
+    del ref
+    sq = np.zeros(q.shape, np.uint64)
+    sq[1:, 1:] = (img.astype(np.uint64) ** 2).cumsum(0).cumsum(1)
+    assert np.array_equal(q, sq)
 
 
-@pytest.mark.parametrize("shape", [(1, 1), (5, 7), (31, 33), (257, 64), (640, 480), (1333, 750), (1920, 1080)])
+@pytest.mark.parametrize("shape", [(1, 1), (5, 7), (31, 33), (257, 64), (640, 480), (1333, 750), (1920, 1080),
+                                   (4095, 33), (4096, 31), (8191, 40), (7680, 4320)])
 @pytest.mark.parametrize("tilted", [False, True])
 def test_integral_uniform_noise(gpu_ctx, shape, tilted):
     w, h = shape
@@ -26,11 +36,15 @@ def test_integral_uniform_noise(gpu_ctx, shape, tilted):
 
 
 def test_integral_4k_all_255_needs_64_bit(gpu_ctx):
-    img = np.full((2160, 3840), 255, np.uint8)
-    s, q, _ = gpu_ctx.integral(img)
-    assert int(q[-1, -1]) == 255 * 255 * 3840 * 2160 > 2 ** 32
-    assert int(s[-1, -1]) == 255 * 3840 * 2160
-    _check_integral(gpu_ctx, img, False)
+    """UHD and DCI 4K white frames: the squares pass 2^32; at 4096 x 2160 the int32 sum passes 2^31 and wraps"""
+    for w, tilted in ((3840, False), (4096, True)):
+        img = np.full((2160, w), 255, np.uint8)
+        s, q, _ = gpu_ctx.integral(img)
+        assert int(q[-1, -1]) == 255 * 255 * w * 2160 > 2 ** 32
+        total = 255 * w * 2160
+        assert int(s[-1, -1]) == (total if total < 2 ** 31 else total - 2 ** 32)
+        assert (total >= 2 ** 31) == (w == 4096)
+        _check_integral(gpu_ctx, img, tilted)
 
 
 def test_integral_all_zero_and_strided(gpu_ctx):
