@@ -225,9 +225,14 @@ class Detector:
         return {n: int(getattr(s, n)) for n, _ in abi.RunStats._fields_}
 
     # ---- device-resident input ---------------------------------------------------------
-    def enqueue(self, frames_dev, n_frames: int, frame_stride: int, row_stride: int, stream: int = 0):
-        abi.check(abi.lib().clfd_detector_enqueue(self._h, _ptr(frames_dev), n_frames, frame_stride, row_stride,
-                                                  C.c_void_p(stream) if stream else None))
+    def enqueue(self, frames_dev, n_frames: int, frame_stride: int, row_stride: int, stream: int = 0, channels: int = 1):
+        """channels 3 / 4: interleaved BGR / BGRA frames, converted to gray on `stream` first"""
+        s = C.c_void_p(stream) if stream else None
+        if channels == 1:
+            abi.check(abi.lib().clfd_detector_enqueue(self._h, _ptr(frames_dev), n_frames, frame_stride, row_stride, s))
+        else:
+            abi.check(abi.lib().clfd_detector_enqueue_color(self._h, _ptr(frames_dev), n_frames, channels, frame_stride,
+                                                            row_stride, s))
 
     def fetch(self, stream: int = 0) -> DetectResult:
         n = C.c_int64()
@@ -236,33 +241,46 @@ class Detector:
         return DetectResult(self._rects[:n.value].copy(), self.stats())
 
     def _geometry(self, frames):
-        """(n_frames, frame stride, row stride) of a uint8 [n, H, W] numpy array or torch tensor of this detector's shape"""
-        n, H, W = frames.shape
+        """(n_frames, frame stride, row stride, channels) of a uint8 [n, H, W] or [n, H, W, C] (C = 3 BGR, 4 BGRA) numpy
+        array or torch tensor of this detector's shape"""
+        n, H, W = frames.shape[:3]
         assert (H, W) == (self.height, self.width)
-        if isinstance(frames, np.ndarray):
-            return n, frames.strides[0], frames.strides[1]
-        return n, frames.stride(0), frames.stride(1)
+        strides = frames.strides if isinstance(frames, np.ndarray) else frames.stride()
+        if frames.ndim == 3:
+            return n, strides[0], strides[1], 1
+        c = frames.shape[3]
+        if frames.ndim != 4 or c not in (3, 4):
+            raise ValueError(f"frames of shape {tuple(frames.shape)}: expected [n, H, W] or [n, H, W, 3 | 4]")
+        if strides[3] != 1 or strides[2] != c:
+            raise ValueError(f"colour frames need interleaved pixels (strides {tuple(strides)})")
+        return n, strides[0], strides[1], c
 
     # ---- host input, end to end (the call a clod user makes) ----------------------------
     def detect(self, frames) -> DetectResult:
-        """frames: uint8 [n,H,W] (numpy, or a pinned torch CPU tensor)"""
+        """frames: uint8 [n,H,W], or [n,H,W,3 | 4] BGR / BGRA (numpy, or a pinned torch CPU tensor)"""
         if isinstance(frames, np.ndarray):
             if frames.ndim == 2:
                 frames = frames[None]
             frames = np.ascontiguousarray(frames, np.uint8)
-        n, fs, rs = self._geometry(frames)
+        n, fs, rs, c = self._geometry(frames)
         cnt = C.c_int64()
-        abi.check(abi.lib().clfd_detect(self._h, _ptr(frames), n, fs, rs,
-                                        self._rects.ctypes.data_as(C.POINTER(abi.Rect)), self._rect_cap, C.byref(cnt)))
+        out = self._rects.ctypes.data_as(C.POINTER(abi.Rect))
+        if c == 1:
+            abi.check(abi.lib().clfd_detect(self._h, _ptr(frames), n, fs, rs, out, self._rect_cap, C.byref(cnt)))
+        else:
+            abi.check(abi.lib().clfd_detect_color(self._h, _ptr(frames), n, c, fs, rs, out, self._rect_cap, C.byref(cnt)))
         return DetectResult(self._rects[:cnt.value].copy(), self.stats())
 
     # ---- host input, streaming: submit batch i+1 while batch i computes -----------------
     def submit(self, frames) -> None:
         """frames as for detect(); must stay alive (and should be pinned) until collected"""
         if isinstance(frames, np.ndarray):
-            assert frames.ndim == 3 and frames.dtype == np.uint8 and frames.flags.c_contiguous
-        n, fs, rs = self._geometry(frames)
-        abi.check(abi.lib().clfd_detect_submit(self._h, _ptr(frames), n, fs, rs))
+            assert frames.ndim in (3, 4) and frames.dtype == np.uint8 and frames.flags.c_contiguous
+        n, fs, rs, c = self._geometry(frames)
+        if c == 1:
+            abi.check(abi.lib().clfd_detect_submit(self._h, _ptr(frames), n, fs, rs))
+        else:
+            abi.check(abi.lib().clfd_detect_submit_color(self._h, _ptr(frames), n, c, fs, rs))
 
     def submit_views(self, first_frame, n_frames: int, frame_stride: int, row_stride: int) -> None:
         """submit n_frames frames that start frame_stride bytes apart at `first_frame` (a pinned tensor view or an

@@ -110,6 +110,10 @@ def lib() -> C.CDLL:
     L.clfd_detect_image.argtypes = [vp, u8p, C.c_int, C.c_int, C.POINTER(Rect), C.c_int64, C.POINTER(C.c_int64)]
     L.clfd_detect_submit.argtypes = [vp, u8p, C.c_int, C.c_size_t, C.c_int]
     L.clfd_detect_collect.argtypes = [vp, C.POINTER(Rect), C.c_int64, C.POINTER(C.c_int64)]
+    L.clfd_detector_enqueue_color.argtypes = [vp, u8p, C.c_int, C.c_int, C.c_size_t, C.c_int, vp]
+    L.clfd_detect_submit_color.argtypes = [vp, u8p, C.c_int, C.c_int, C.c_size_t, C.c_int]
+    L.clfd_detect_color.argtypes = [vp, u8p, C.c_int, C.c_int, C.c_size_t, C.c_int, C.POINTER(Rect), C.c_int64,
+                                    C.POINTER(C.c_int64)]
     L.clfd_detector_get_codes.argtypes = [vp, C.c_int, C.POINTER(C.c_int16), C.c_int64]
     L.clfd_detector_read_level.argtypes = [vp, C.c_int, C.c_int, C.c_int, vp, vp, vp, vp]
     L.clfd_detector_get_stats.argtypes = [vp, C.POINTER(RunStats)]

@@ -326,8 +326,8 @@ struct clfd_detector {
     DevBuf<QueueItem> queue, queue_b;
     DevBuf<DevRect> rects;
     DevBuf<uint8_t> dev_frames[kSlots];   // staging for host input (clfd_detect / clfd_detect_submit)
+    DevBuf<uint8_t> dev_color[kSlots];    // interleaved colour staging of clfd_detect_submit_color, allocated at first use
     DevBuf<DevRect> rects2;               // rect buffer of slot 1 (slot 0 uses `rects`)
-    DevBuf<uint8_t> dev_bgr;              // interleaved colour input of clfd_detect_image
     DevBuf<RocItem> roc;                  // candidates of clfd_detector_reject_levels
     DevBuf<unsigned long long> roc_count;
     DevRect *h_rects = nullptr;           // pinned, kSlots x rect_cap... slot 1 holds kEagerRects only
@@ -343,6 +343,7 @@ struct clfd_detector {
     cudaEvent_t ev[16] = {nullptr};
     float kernel_ms[8] = {0};
     bool have_events = false;
+    bool color_events = false;   // ev[8] / ev[9] bracket the colour conversion of the last batch (kernel_ms[6])
     bool sum_di = false;   // the ystep-2 levels of pyr.sum are column-de-interleaved (PyrLevel::di)
     // clfd_detect pipelines the H2D copy of a batch with its own compute, chunk by chunk
     cudaStream_t copy_stream = nullptr;
@@ -567,6 +568,16 @@ static int scratch_plan(clfd_context *ctx, int W, int H, int lw, int lh, bool ti
     return 0;
 }
 
+// k_color_to_gray of n_frames interleaved frames into gray frames of W x H with a 16-byte row pitch, frames pitch * H apart
+static ColorArgs color_args(const uint8_t *src, int n_frames, size_t frame_stride, int row_stride, int channels, int W, int H,
+                            uint8_t *dst) {
+    ColorArgs a;
+    a.src = src; a.frame_stride = frame_stride; a.row_stride = row_stride; a.channels = channels;
+    a.W = W; a.H = H; a.n_frames = n_frames;
+    a.dst = dst; a.dst_pitch = (int)round_up(W, 16); a.dst_frame_stride = (size_t)a.dst_pitch * H;
+    return a;
+}
+
 // copies a host or device 8-bit image into a fresh device buffer when it lives on the host
 struct InputImage {
     const uint8_t *dev = nullptr;
@@ -640,17 +651,14 @@ int clfd_bgr_to_gray(clfd_context *ctx, const uint8_t *bgr, int w, int h, int st
     InputImage in;
     int rc = in.set(bgr, w * channels, h, stride, src_on_device, ctx->stream);
     if (rc) return rc;
-    uint8_t *out = gray;
-    int ostride = gstride;
+    // the kernel writes 16-byte rows (zero padding behind the last pixel): a buffer of that pitch, then the caller's rows
+    const int ostride = (int)round_up(w, 16);
     DevBuf<uint8_t> tmp;
-    if (!dst_on_device) {
-        ostride = (int)round_up(w, 16);
-        if ((rc = tmp.alloc((size_t)ostride * h))) return rc;
-        out = tmp.p;
-    }
-    CK(launch_bgr_to_gray(in.dev, w, h, in.stride, channels, out, ostride, ctx->stream));
+    if ((rc = tmp.alloc((size_t)ostride * h))) return rc;
+    CK(launch_color_to_gray(color_args(in.dev, 1, 0, in.stride, channels, w, h, tmp.p), ctx->stream));
     ctx->launches++;
-    if (!dst_on_device) CK(cudaMemcpy2DAsync(gray, gstride, out, ostride, w, h, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpy2DAsync(gray, gstride, tmp.p, ostride, w, h, dst_on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost,
+                         ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
     return 0;
 }
@@ -676,7 +684,7 @@ int clfd_integral_image(clfd_context *ctx, const uint8_t *img, int w, int h, int
     DevBuf<uint8_t> g;
     const int dstride = (int)round_up(w, 16);
     if ((rc = g.alloc((size_t)dstride * h + 16))) return rc;
-    CK(launch_bgr_to_gray(in.dev, w, h, in.stride, channels, g.p, dstride, ctx->stream));
+    CK(launch_color_to_gray(color_args(in.dev, 1, 0, in.stride, channels, w, h, g.p), ctx->stream));
     ctx->launches++;
     if (gray) CK(cudaMemcpy2DAsync(gray, gstride, g.p, dstride, w, h, cudaMemcpyDeviceToHost, ctx->stream));
     return clfd_integral(ctx, g.p, w, h, dstride, 1, sum, sqsum, tilted, 0);   // (synchronises the stream before it returns)
@@ -1292,6 +1300,47 @@ int clfd_detector_enqueue(clfd_detector *det, const uint8_t *frames_dev, int n_f
                  : enqueue_range(det, frames_dev, 0, n_frames, frame_stride, row_stride, s, true, &launches);
     if (rc) return rc;
     det->stats.kernel_launches = launches;
+    det->color_events = false;
+    return 0;
+}
+
+// What the colour entry points accept besides channels == 1 (which they hand to the gray calls).
+static int check_color_batch(const clfd_detector *det, int n_frames, int channels, int row_stride) {
+    if (channels != 3 && channels != 4) INVALID("channels %d: must be 1 (gray), 3 (BGR) or 4 (BGRA)", channels);
+    if (n_frames <= 0 || n_frames > det->cfg.max_batch) INVALID("n_frames %d outside 1..%d", n_frames, det->cfg.max_batch);
+    if ((long long)row_stride < (long long)det->cfg.width * channels)
+        INVALID("row stride %d smaller than %d pixels of %d channels", row_stride, det->cfg.width, channels);
+    return 0;
+}
+
+// Colour -> gray of a batch into the detector's gray frame layout (16-byte row pitch) on stream s.  With profiling on,
+// ev[8] / ev[9] bracket the conversion (clfd_detector_get_kernel_ms [6]).
+static int enqueue_color_to_gray(clfd_detector *det, const uint8_t *src, int n_frames, int channels, size_t frame_stride,
+                                 int row_stride, uint8_t *dst, cudaStream_t s) {
+    if (det->profiling) CK(cudaEventRecord(det->ev[8], s));
+    CK(launch_color_to_gray(color_args(src, n_frames, frame_stride, row_stride, channels, det->cfg.width, det->cfg.height, dst), s));
+    if (det->profiling) CK(cudaEventRecord(det->ev[9], s));
+    det->ctx->launches++;
+    return 0;
+}
+
+int clfd_detector_enqueue_color(clfd_detector *det, const uint8_t *frames_dev, int n_frames, int channels,
+                                size_t frame_stride, int row_stride, void *cuda_stream) {
+    if (!det || !frames_dev) INVALID("NULL argument");
+    if (channels == 1) return clfd_detector_enqueue(det, frames_dev, n_frames, frame_stride, row_stride, cuda_stream);
+    int rc = check_color_batch(det, n_frames, channels, row_stride);
+    if (rc) return rc;
+    if (det->n_submitted != det->n_collected)
+        INVALID("clfd_detector_enqueue_color while submitted batches are in flight (they may still read its frame buffer)");
+    clfd_context *ctx = det->ctx;
+    CK(cudaSetDevice(ctx->device));
+    cudaStream_t s = cuda_stream ? (cudaStream_t)cuda_stream : ctx->stream;
+    const size_t dstride = round_up(det->cfg.width, 16), dframe = dstride * det->cfg.height;
+    if (!det->dev_frames[0].p && (rc = det->dev_frames[0].alloc(dframe * det->cfg.max_batch + 64))) return rc;
+    if ((rc = enqueue_color_to_gray(det, frames_dev, n_frames, channels, frame_stride, row_stride, det->dev_frames[0].p, s))) return rc;
+    if ((rc = clfd_detector_enqueue(det, det->dev_frames[0].p, n_frames, dframe, (int)dstride, cuda_stream))) return rc;
+    det->stats.kernel_launches += 1;
+    det->color_events = det->profiling;
     return 0;
 }
 
@@ -1330,6 +1379,20 @@ static int take_counters(clfd_detector *det, const unsigned long long *hc, int n
     return 0;
 }
 
+// event times of the last batch -> det->kernel_ms (clfd_detector_get_kernel_ms)
+static void read_kernel_ms(clfd_detector *det) {
+    // [0] resize+colsum [1] colscan [2] integral rows [3] tilted [4] tile kernel [5] deep kernel [6] colour conversion
+    cudaEventElapsedTime(&det->kernel_ms[0], det->ev[0], det->ev[1]);
+    cudaEventElapsedTime(&det->kernel_ms[1], det->ev[1], det->ev[2]);
+    cudaEventElapsedTime(&det->kernel_ms[2], det->ev[2], det->ev[3]);
+    cudaEventElapsedTime(&det->kernel_ms[3], det->ev[3], det->ev[4]);
+    cudaEventElapsedTime(&det->kernel_ms[4], det->ev[5], det->ev[6]);
+    cudaEventElapsedTime(&det->kernel_ms[5], det->ev[6], det->ev[7]);
+    det->kernel_ms[6] = 0;
+    if (det->color_events) cudaEventElapsedTime(&det->kernel_ms[6], det->ev[8], det->ev[9]);
+    (void)cudaGetLastError();   // an event a batch did not record fails its query: not an error of the next launch
+}
+
 int clfd_detector_fetch(clfd_detector *det, clfd_rect *rects, int64_t cap, int64_t *n_rects, void *cuda_stream) {
     if (!det || !n_rects) INVALID("NULL argument");
     clfd_context *ctx = det->ctx;
@@ -1343,15 +1406,7 @@ int clfd_detector_fetch(clfd_detector *det, clfd_rect *rects, int64_t cap, int64
     int rc = take_counters(det, det->h_counters, det->last_frames, n_rects);
     if (rc) return rc;
     const unsigned long long total = (unsigned long long)*n_rects;
-    if (det->have_events) {
-        // [0] resize+colsum [1] colscan [2] integral rows [3] tilted [4] tile kernel [5] deep kernel
-        cudaEventElapsedTime(&det->kernel_ms[0], det->ev[0], det->ev[1]);
-        cudaEventElapsedTime(&det->kernel_ms[1], det->ev[1], det->ev[2]);
-        cudaEventElapsedTime(&det->kernel_ms[2], det->ev[2], det->ev[3]);
-        cudaEventElapsedTime(&det->kernel_ms[3], det->ev[3], det->ev[4]);
-        cudaEventElapsedTime(&det->kernel_ms[4], det->ev[5], det->ev[6]);
-        cudaEventElapsedTime(&det->kernel_ms[5], det->ev[6], det->ev[7]);
-    }
+    if (det->have_events) read_kernel_ms(det);
     if (total == 0 || !rects) return 0;
     if ((int64_t)total > cap) { set_error("rect buffer too small: need %llu, have %lld", total, (long long)cap); return CLFD_ERR_CAPACITY; }
     CK(cudaMemcpyAsync(det->h_rects, det->rects.p, total * sizeof(DevRect), cudaMemcpyDeviceToHost, s));
@@ -1368,7 +1423,10 @@ int clfd_detector_fetch(clfd_detector *det, clfd_rect *rects, int64_t cap, int64
 //     next inside a range, so they run as one range;
 //   * counters and the first kEagerRects rects are copied back behind the kernels and an event
 //     marks the slot done, so the NEXT batch's host-to-device copy overlaps this batch's compute.
-int clfd_detect_submit(clfd_detector *det, const uint8_t *frames_host, int n_frames, size_t frame_stride, int row_stride) {
+//   * colour batches (channels 3 / 4) go to a per-slot colour staging buffer instead, and the conversion of each range
+//     runs on the copy stream behind its copy, into the slot's gray frames: from there on the batch is a gray batch.
+static int submit_batch(clfd_detector *det, const uint8_t *frames_host, int n_frames, int channels, size_t frame_stride,
+                        int row_stride) {
     if (!det || !frames_host) INVALID("NULL argument");
     clfd_context *ctx = det->ctx;
     CK(cudaSetDevice(ctx->device));
@@ -1380,6 +1438,12 @@ int clfd_detect_submit(clfd_detector *det, const uint8_t *frames_host, int n_fra
     const size_t dstride = round_up(W, 16), dframe = dstride * H;
     int rc;
     if (!det->dev_frames[slot].p && (rc = det->dev_frames[slot].alloc(dframe * det->cfg.max_batch + 64))) return rc;
+    // colour staging: rows of W * channels bytes at a 16-byte pitch.  The slot's last batch has been collected, so the
+    // buffer may grow here
+    const size_t cstride = round_up((size_t)W * channels, 16), cframe = cstride * H;
+    if (channels != 1 && det->dev_color[slot].n < cframe * det->cfg.max_batch &&
+        (rc = det->dev_color[slot].alloc(cframe * det->cfg.max_batch)))
+        return rc;
     if (slot == 1) {
         if (!det->rects2.p && (rc = det->rects2.alloc(det->rect_cap))) return rc;
         if (!det->h_rects1) CK(cudaMallocHost((void **)&det->h_rects1, (size_t)kEagerRects * sizeof(DevRect)));
@@ -1393,6 +1457,7 @@ int clfd_detect_submit(clfd_detector *det, const uint8_t *frames_host, int n_fra
     if (det->cas.size() != 1) n_chunks = 1;
     const bool overlap = overlap_applies(det, n_frames);
     if (overlap) n_chunks = overlap_chunks(n_frames);   // the compute chunks are the copy chunks
+    if (channels != 1 && det->profiling) n_chunks = 1;  // one pair of events brackets the whole conversion
     if (!det->copy_stream) CK(cudaStreamCreateWithFlags(&det->copy_stream, cudaStreamNonBlocking));
     for (int k = 0; k < n_chunks; k++)
         if (!det->copied[k]) CK(cudaEventCreateWithFlags(&det->copied[k], cudaEventDisableTiming));
@@ -1404,21 +1469,34 @@ int clfd_detect_submit(clfd_detector *det, const uint8_t *frames_host, int n_fra
     det->last_frames = n_frames;
     det->slot_frames[slot] = n_frames;
     int launches = 0;
+    cudaStream_t cs = det->copy_stream;
+    // nf frames of `wbytes` bytes per row from the host to d (pitch dpitch, frames dfr apart); nothing behind the last
+    // row's last pixel is read
+    auto h2d = [&](uint8_t *d, size_t dpitch, size_t dfr, const uint8_t *src, size_t wbytes, int nf) -> int {
+        if ((size_t)row_stride == dpitch && frame_stride == dfr) {
+            CK(cudaMemcpyAsync(d, src, dfr * nf - (dpitch - wbytes), cudaMemcpyHostToDevice, cs));
+        } else if (frame_stride == (size_t)row_stride * H) {
+            CK(cudaMemcpy2DAsync(d, dpitch, src, row_stride, wbytes, (size_t)H * nf, cudaMemcpyHostToDevice, cs));
+        } else {
+            for (int f = 0; f < nf; f++)
+                CK(cudaMemcpy2DAsync(d + f * dfr, dpitch, src + f * frame_stride, row_stride, wbytes, H,
+                                     cudaMemcpyHostToDevice, cs));
+        }
+        return 0;
+    };
     for (int k = 0; k < n_chunks; k++) {
         const int f0 = (int)((long long)n_frames * k / n_chunks), f1 = (int)((long long)n_frames * (k + 1) / n_chunks);
         const int nf = f1 - f0;
         if (nf <= 0) continue;
         uint8_t *dst = det->dev_frames[slot].p + (size_t)f0 * dframe;
         const uint8_t *src = frames_host + (size_t)f0 * frame_stride;
-        cudaStream_t cs = det->copy_stream;
-        if ((size_t)row_stride == dstride && frame_stride == dframe) {
-            CK(cudaMemcpyAsync(dst, src, dframe * nf, cudaMemcpyHostToDevice, cs));
-        } else if (frame_stride == (size_t)row_stride * H) {
-            CK(cudaMemcpy2DAsync(dst, dstride, src, row_stride, W, (size_t)H * nf, cudaMemcpyHostToDevice, cs));
+        if (channels == 1) {
+            if ((rc = h2d(dst, dstride, dframe, src, W, nf))) return rc;
         } else {
-            for (int f = 0; f < nf; f++)
-                CK(cudaMemcpy2DAsync(dst + f * dframe, dstride, src + f * frame_stride, row_stride, W, H,
-                                     cudaMemcpyHostToDevice, cs));
+            uint8_t *stage = det->dev_color[slot].p + (size_t)f0 * cframe;
+            if ((rc = h2d(stage, cstride, cframe, src, (size_t)W * channels, nf))) return rc;
+            if ((rc = enqueue_color_to_gray(det, stage, nf, channels, cframe, (int)cstride, dst, cs))) return rc;
+            launches++;
         }
         CK(cudaEventRecord(det->copied[k], cs));
         if (overlap) continue;
@@ -1442,8 +1520,23 @@ int clfd_detect_submit(clfd_detector *det, const uint8_t *frames_host, int n_fra
     CK(cudaMemcpyAsync(slot ? det->h_rects1 : det->h_rects, slot ? det->rects2.p : det->rects.p, eager * sizeof(DevRect),
                        cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaEventRecord(det->done[slot], ctx->stream));
+    det->color_events = channels != 1 && det->profiling;
     det->n_submitted++;
     return 0;
+}
+
+int clfd_detect_submit(clfd_detector *det, const uint8_t *frames_host, int n_frames, size_t frame_stride, int row_stride) {
+    return submit_batch(det, frames_host, n_frames, 1, frame_stride, row_stride);
+}
+
+int clfd_detect_submit_color(clfd_detector *det, const uint8_t *frames_host, int n_frames, int channels, size_t frame_stride,
+                             int row_stride) {
+    if (!det || !frames_host) INVALID("NULL argument");
+    if (channels != 1) {
+        int rc = check_color_batch(det, n_frames, channels, row_stride);
+        if (rc) return rc;
+    }
+    return submit_batch(det, frames_host, n_frames, channels, frame_stride, row_stride);
 }
 
 // Wait for the oldest submitted batch and hand out its rects.
@@ -1455,6 +1548,7 @@ int clfd_detect_collect(clfd_detector *det, clfd_rect *rects, int64_t cap, int64
     const int slot = (int)(det->n_collected % kSlots);
     det->n_collected++;
     CK(cudaEventSynchronize(det->done[slot]));
+    if (det->have_events && det->n_collected == det->n_submitted) read_kernel_ms(det);   // the events are this batch's
     int rc = take_counters(det, det->h_counters + (size_t)slot * kCnt * 16, det->slot_frames[slot], n_rects);
     if (rc) return rc;
     const unsigned long long total = (unsigned long long)*n_rects;
@@ -1479,27 +1573,21 @@ int clfd_detect(clfd_detector *det, const uint8_t *frames_host, int n_frames, si
     return clfd_detect_collect(det, rects, cap, n_rects);
 }
 
-// One interleaved 8-bit image (1, 3 = BGR or 4 = BGRA channels) from the host: the colour
-// conversion runs on the device and feeds the detector directly (no gray round trip).
+// A batch of interleaved BGR / BGRA frames from the host, synchronous: the colour form of clfd_detect.
+int clfd_detect_color(clfd_detector *det, const uint8_t *frames_host, int n_frames, int channels, size_t frame_stride,
+                      int row_stride, clfd_rect *rects, int64_t cap, int64_t *n_rects) {
+    if (!det) INVALID("NULL argument");
+    if (det->n_submitted != det->n_collected) INVALID("clfd_detect_color while submitted batches are in flight");
+    int rc = clfd_detect_submit_color(det, frames_host, n_frames, channels, frame_stride, row_stride);
+    if (rc) return rc;
+    return clfd_detect_collect(det, rects, cap, n_rects);
+}
+
+// One interleaved 8-bit image (1, 3 = BGR or 4 = BGRA channels) from the host: a batch of one frame.
 int clfd_detect_image(clfd_detector *det, const uint8_t *img_host, int channels, int stride, clfd_rect *rects, int64_t cap,
                       int64_t *n_rects) {
     if (!det || !img_host) INVALID("NULL argument");
-    const int W = det->cfg.width, H = det->cfg.height;
-    if (channels == 1) return clfd_detect(det, img_host, 1, (size_t)stride * H, stride, rects, cap, n_rects);
-    if (channels != 3 && channels != 4) INVALID("channels must be 1, 3 or 4");
-    if (stride < W * channels) INVALID("row stride %d smaller than %d pixels of %d channels", stride, W, channels);
-    if (det->n_submitted != det->n_collected) INVALID("clfd_detect_image while submitted batches are in flight");
-    clfd_context *ctx = det->ctx;
-    CK(cudaSetDevice(ctx->device));
-    const size_t dstride = round_up(W, 16), dframe = dstride * H;
-    int rc;
-    if (!det->dev_frames[0].p && (rc = det->dev_frames[0].alloc(dframe * det->cfg.max_batch + 64))) return rc;
-    if (det->dev_bgr.n < (size_t)stride * H && (rc = det->dev_bgr.alloc((size_t)stride * H))) return rc;
-    CK(cudaMemcpyAsync(det->dev_bgr.p, img_host, (size_t)stride * H, cudaMemcpyHostToDevice, ctx->stream));
-    CK(launch_bgr_to_gray(det->dev_bgr.p, W, H, stride, channels, det->dev_frames[0].p, (int)dstride, ctx->stream));
-    ctx->launches++;
-    if ((rc = clfd_detector_enqueue(det, det->dev_frames[0].p, 1, dframe, (int)dstride, nullptr))) return rc;
-    return clfd_detector_fetch(det, rects, cap, n_rects, nullptr);
+    return clfd_detect_color(det, img_host, 1, channels, (size_t)stride * det->cfg.height, stride, rects, cap, n_rects);
 }
 
 int clfd_detector_get_codes(clfd_detector *det, int cascade, int16_t *codes, int64_t cap) {

@@ -65,8 +65,17 @@ cudaError_t launch_integral_rows(const PyramidArgs &a, cudaStream_t stream, int 
 cudaError_t launch_tilted(const PyramidArgs &a, cudaStream_t stream, int *n_launches);
 int tilt_tile_interior();    // output columns per warp tile of k_tilt_tiles
 
-cudaError_t launch_bgr_to_gray(const uint8_t *bgr, int w, int h, int stride, int channels,
-                               uint8_t *gray, int gstride, cudaStream_t stream);
+// BGR / BGRA -> gray of n_frames interleaved frames (kernels_clif.cu, k_color_to_gray)
+struct ColorArgs {
+    const uint8_t *src;         // device, n_frames x (H rows of row_stride bytes), frame_stride apart (any alignment)
+    size_t frame_stride;        // bytes; may be smaller than H * row_stride, or 0
+    int row_stride, channels;   // channels 3 (BGR) or 4 (BGRA, alpha ignored); row_stride >= W * channels
+    int W, H, n_frames;
+    uint8_t *dst;               // device, 16-byte aligned; written up to round_up(W, 16) per row (zero padding)
+    size_t dst_frame_stride;    // bytes, a multiple of 16
+    int dst_pitch;              // bytes, a multiple of 16 and >= round_up(W, 16)
+};
+cudaError_t launch_color_to_gray(const ColorArgs &a, cudaStream_t stream);
 
 // ---- cascade (clod) -----------------------------------------------------------------
 struct CascadeArgs {

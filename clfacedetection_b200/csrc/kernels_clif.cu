@@ -3,7 +3,7 @@
 //   * cvResize(img, level, CV_INTER_LINEAR) per pyramid level       (tempcv.cpp:1301)
 //   * integralImageSumRows / integralImageSumCols                    (clif.cl:79-120)
 //     and cvIntegral(sum, sqsum, tilted)                             (tempcv.cpp:1302)
-//   * bgrToGrayscale                                                 (clif.cl:4-18)
+//   * bgrToGrayscale                                                 (clif.cl:4-18), batched
 //
 // Design (HBM-bound byte work; no tensor cores):
 //   K1 resize_colsum : all levels x frames x 32-row blocks in one launch.  Each thread makes
@@ -743,20 +743,71 @@ cudaError_t launch_tilted(const PyramidArgs &a, cudaStream_t stream, int *n_laun
 int tilt_tile_interior() { return kTiltInterior; }
 
 // ------------------------------------------------------------------------------------
-// BGR(A) -> gray, OpenCV fixed point: (B*1868 + G*9617 + R*4899 + 8192) >> 14
+// BGR(A) -> gray, OpenCV fixed point: (B*1868 + G*9617 + R*4899 + 8192) >> 14, a batch of interleaved frames per launch
 // ------------------------------------------------------------------------------------
-__global__ void k_bgr_to_gray(const uint8_t *__restrict__ bgr, int w, int h, int stride, int channels,
-                              uint8_t *__restrict__ gray, int gstride) {
-    const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y;
-    if (x >= w || y >= h) return;
-    const uint8_t *p = bgr + (size_t)y * stride + (size_t)x * channels;
-    gray[(size_t)y * gstride + x] = (uint8_t)((p[0] * 1868 + p[1] * 9617 + p[2] * 4899 + 8192) >> 14);
+// A thread makes 16 gray pixels of one row and writes them with one 16-byte store (the gray pitch is a multiple of 16).
+// Its source bytes are the 16 pixels' 16 * C bytes: read as C words of 16 bytes when the row starts 16-byte aligned, as
+// 4 * C words of 4 bytes when it starts 4-byte aligned (a BGR group of 4 pixels is three words), and byte by byte
+// otherwise (odd strides or base pointer) and for a row's last, partial group.  No byte behind a row's W * C bytes is
+// read: the caller's buffer may end there (a frame stride below H * row_stride, or 0).
+__device__ __forceinline__ uint32_t gray_of(uint32_t b, uint32_t g, uint32_t r) {
+    return (b * 1868u + g * 9617u + r * 4899u + 8192u) >> 14;
 }
 
-cudaError_t launch_bgr_to_gray(const uint8_t *bgr, int w, int h, int stride, int channels,
-                               uint8_t *gray, int gstride, cudaStream_t stream) {
-    if (w <= 0 || h <= 0) return cudaSuccess;
-    k_bgr_to_gray<<<dim3((w + 255) / 256, h), 256, 0, stream>>>(bgr, w, h, stride, channels, gray, gstride);
+template <int C>
+__device__ __forceinline__ uint4 gray16_words(const uint8_t *__restrict__ p, bool a16) {
+    constexpr int NW = 4 * C;   // 32-bit words of the group
+    uint32_t w[NW];
+    if (a16) {
+#pragma unroll
+        for (int k = 0; k < C; k++) {
+            const uint4 v = __ldg(reinterpret_cast<const uint4 *>(p) + k);
+            w[4 * k] = v.x; w[4 * k + 1] = v.y; w[4 * k + 2] = v.z; w[4 * k + 3] = v.w;
+        }
+    } else {
+#pragma unroll
+        for (int k = 0; k < NW; k++) w[k] = __ldg(reinterpret_cast<const uint32_t *>(p) + k);
+    }
+    uint32_t out[4] = {0u, 0u, 0u, 0u};
+#pragma unroll
+    for (int i = 0; i < 16; i++) {
+        const int j = i * C;   // byte offset of pixel i
+        const uint32_t b = (w[j >> 2] >> (8 * (j & 3))) & 255u;
+        const uint32_t g = (w[(j + 1) >> 2] >> (8 * ((j + 1) & 3))) & 255u;
+        const uint32_t r = (w[(j + 2) >> 2] >> (8 * ((j + 2) & 3))) & 255u;
+        out[i >> 2] |= gray_of(b, g, r) << (8 * (i & 3));
+    }
+    return make_uint4(out[0], out[1], out[2], out[3]);
+}
+
+// grid: (ceil(H * groups per row / 256), n_frames); one item = (row, group of 16 pixels)
+template <int C>
+__global__ void __launch_bounds__(256) k_color_to_gray(const ColorArgs a) {
+    const int groups = (a.W + 15) >> 4;
+    const int item = blockIdx.x * blockDim.x + threadIdx.x;
+    if (item >= a.H * groups) return;
+    const int y = item / groups, x0 = (item - y * groups) * 16;
+    const uint8_t *__restrict__ row = a.src + (size_t)blockIdx.y * a.frame_stride + (size_t)y * a.row_stride;
+    const uint8_t *__restrict__ p = row + (size_t)x0 * C;
+    uint4 v;
+    if (x0 + 16 <= a.W && (reinterpret_cast<uintptr_t>(row) & 3) == 0) {
+        v = gray16_words<C>(p, (reinterpret_cast<uintptr_t>(row) & 15) == 0);
+    } else {
+        uint32_t out[4] = {0u, 0u, 0u, 0u};   // pixels behind the row's end: zero padding of the gray row
+        const int n = min(16, a.W - x0);
+        for (int i = 0; i < n; i++)
+            out[i >> 2] |= gray_of(__ldg(p + i * C), __ldg(p + i * C + 1), __ldg(p + i * C + 2)) << (8 * (i & 3));
+        v = make_uint4(out[0], out[1], out[2], out[3]);
+    }
+    *reinterpret_cast<uint4 *>(a.dst + (size_t)blockIdx.y * a.dst_frame_stride + (size_t)y * a.dst_pitch + x0) = v;
+}
+
+cudaError_t launch_color_to_gray(const ColorArgs &a, cudaStream_t stream) {
+    if (a.W <= 0 || a.H <= 0 || a.n_frames <= 0) return cudaSuccess;
+    const long long items = (long long)a.H * ((a.W + 15) >> 4);
+    const dim3 grid((unsigned)((items + 255) / 256), a.n_frames);
+    if (a.channels == 4) k_color_to_gray<4><<<grid, 256, 0, stream>>>(a);
+    else k_color_to_gray<3><<<grid, 256, 0, stream>>>(a);
     return cudaGetLastError();
 }
 
