@@ -301,11 +301,6 @@ struct CascadePlan {
     DevBuf<DenseStage> d_stage_tab[2];   // stage trees: stage table in execution order
     DevBuf<int16_t> d_flat_code;         // exit codes of flat windows by pixel value (DenseParams::flat_code), see build_flat_table
     DenseParams dense[2];          // the cascade's parameter blobs with this detector's tail pointers
-    // patch kernel (PackedCascade::patch_cut): the tile kernel stops at cut_stages, k_cascade_patch finishes its survivors
-    bool use_patch = false;
-    DenseParams patch;
-    DevBuf<TailStump> d_patch_tail;
-    DevBuf<unsigned long long> d_qcount;   // queue counters, one per (slot, first frame of a range): ranges run concurrently
     DevBuf<int16_t> d_codes;
     DevBuf<unsigned long long> d_counters;
     DevBuf<unsigned long long> d_count_b;   // second-queue counter, one per slot
@@ -350,9 +345,8 @@ struct clfd_detector {
     cudaEvent_t copied[kMaxChunks] = {nullptr};
     // chunk overlap (enqueue_overlapped): the HBM-bound pyramid kernels of chunk k+1 run beside the L1-bound tile
     // kernel of chunk k
-    cudaStream_t pyr_stream = nullptr, tile_stream[2] = {nullptr, nullptr}, patch_stream = nullptr;
+    cudaStream_t pyr_stream = nullptr, tile_stream[2] = {nullptr, nullptr};
     cudaEvent_t ev_fork = nullptr, ev_pyr[kMaxChunks] = {nullptr}, ev_tile[2] = {nullptr, nullptr};
-    cudaEvent_t ev_tiled[kMaxChunks] = {nullptr}, ev_patch = nullptr;   // a chunk's tile kernel is done / the last patch kernel is
     ~clfd_detector() {
         if (h_rects) cudaFreeHost(h_rects);
         if (h_rects1) cudaFreeHost(h_rects1);
@@ -364,9 +358,6 @@ struct clfd_detector {
         if (ev_fork) cudaEventDestroy(ev_fork);
         for (auto &e : ev_pyr) if (e) cudaEventDestroy(e);
         for (auto &e : ev_tile) if (e) cudaEventDestroy(e);
-        for (auto &e : ev_tiled) if (e) cudaEventDestroy(e);
-        if (ev_patch) cudaEventDestroy(ev_patch);
-        if (patch_stream) cudaStreamDestroy(patch_stream);
         if (pyr_stream) cudaStreamDestroy(pyr_stream);
         for (auto &t : tile_stream) if (t) cudaStreamDestroy(t);
     }
@@ -737,8 +728,8 @@ static int build_flat_table(clfd_context *ctx, CascadePlan &cp) {
 }
 
 // A detector's copy of its cascade on the device: the generic kernels' global-memory blob and the tile kernel's
-// parameter blobs with this copy's device pointers patched in; with use_patch, also the patch kernel's blob.
-static int upload_cascade(CascadePlan &cp, bool use_patch, cudaStream_t s) {
+// parameter blobs with this copy's device pointers patched in.
+static int upload_cascade(CascadePlan &cp, cudaStream_t s) {
     const PackedCascade &pk = cp.cascade->packed;
     int rc;
     if ((rc = cp.d_stages.upload(pk.deep_stages, s)) || (rc = cp.d_nodes.upload(pk.deep_nodes, s)) ||
@@ -750,13 +741,6 @@ static int upload_cascade(CascadePlan &cp, bool use_patch, cudaStream_t s) {
         cp.dense[yi].tail = cp.d_tail[yi].p;
         if (!pk.stage_tab[yi].empty() && (rc = cp.d_stage_tab[yi].upload(pk.stage_tab[yi], s))) return rc;
         cp.dense[yi].stage_g = cp.d_stage_tab[yi].p;
-        if (!use_patch) cp.dense[yi].cut_stages = cp.dense[yi].tail_stages;
-    }
-    cp.use_patch = use_patch;
-    if (use_patch) {
-        cp.patch = pk.patch;
-        if ((rc = cp.d_patch_tail.upload(pk.patch_tail, s))) return rc;
-        cp.patch.tail = cp.d_patch_tail.p;
     }
     return 0;
 }
@@ -933,8 +917,7 @@ int clfd_detector_create(clfd_context *ctx, const clfd_cascade *const *cascades,
     for (auto &cpp : det->cas) {
         CascadePlan &cp = *cpp;
         const PackedCascade &pk = cp.cascade->packed;
-        if ((rc = cp.d_levels.upload(cp.levels, s)) || (rc = upload_cascade(cp, !scale_cascade && pk.patch_cut > 0, s))) return rc;
-        if (cp.use_patch && (rc = cp.d_qcount.alloc((size_t)kSlots * std::max(cfg->max_batch, 1)))) return rc;
+        if ((rc = cp.d_levels.upload(cp.levels, s)) || (rc = upload_cascade(cp, s))) return rc;
         if ((rc = cp.d_counters.alloc(kCnt * kSlots)) || (rc = cp.d_count_b.alloc(kSlots))) return rc;
         // mid kernel: the stages right after the tile prefix of a LINEAR cascade whose trees the tile
         // kernel cannot take, while they are too small for a warp per window (< 24 trees), at most 8
@@ -1043,7 +1026,7 @@ static CascadeArgs cascade_args(const clfd_detector *det, const CascadePlan &cp,
 // to the range (the per-frame buffers are passed pre-offset) and add frame_base to the frame
 // index of the rects they emit.
 // parts: which halves of the range's work go onto stream s (enqueue_overlapped puts them on different streams)
-enum { kPartPyramid = 1, kPartCascades = 2, kPartCounters = 4, kPartPatch = 8, kPartAll = 15 };   // kPartPatch: the patch kernel behind the tile kernel
+enum { kPartPyramid = 1, kPartCascades = 2, kPartCounters = 4, kPartAll = 7 };
 static int enqueue_range(clfd_detector *det, const uint8_t *frames_dev, int frame_base, int n_frames, size_t frame_stride,
                          int row_stride, cudaStream_t s, bool first, int *n_launches, int slot = 0, int parts = kPartAll) {
     clfd_context *ctx = det->ctx;
@@ -1056,10 +1039,10 @@ static int enqueue_range(clfd_detector *det, const uint8_t *frames_dev, int fram
     if (parts & kPartCounters)
         for (auto &cpp : det->cas) {
             if (first) CK(cudaMemsetAsync(cpp->d_counters.p + kCnt * slot, 0, kCnt * sizeof(unsigned long long), s));
-            else if (!cpp->use_patch) CK(cudaMemsetAsync(cpp->d_counters.p + kCnt * slot + 1, 0, sizeof(unsigned long long), s));   // the queue is per range
+            else CK(cudaMemsetAsync(cpp->d_counters.p + kCnt * slot + 1, 0, sizeof(unsigned long long), s));   // the queue is per range
             CK(cudaMemsetAsync(cpp->d_count_b.p + slot, 0, sizeof(unsigned long long), s));
         }
-    if (!(parts & (kPartCascades | kPartPatch))) {
+    if (!(parts & kPartCascades)) {
         ctx->launches += launches;
         *n_launches += launches;
         return 0;
@@ -1075,13 +1058,6 @@ static int enqueue_range(clfd_detector *det, const uint8_t *frames_dev, int fram
             a.queue = det->queue.p; a.queue_cap = det->queue_cap;
             a.rects = slot ? det->rects2.p : det->rects.p; a.rect_cap = det->rect_cap;
             a.counters = cp.d_counters.p + kCnt * slot;
-            a.qcount = a.counters + 1;
-            if (cp.use_patch) {   // the range's own queue region and counter: ranges of a batch run on different streams
-                a.queue = det->queue.p + (size_t)frame_base * cp.windows_per_frame;
-                a.queue_cap = (unsigned long long)n_frames * cp.windows_per_frame;
-                a.qcount = cp.d_qcount.p + (size_t)slot * det->cfg.max_batch + frame_base;
-                if (parts & kPartCascades) CK(cudaMemsetAsync(a.qcount, 0, sizeof(unsigned long long), s));
-            }
             a.deep_in = a.queue; a.deep_count = a.counters + 1;
             if (det->cfg.mode == CLFD_MODE_SCALE_CASCADE) {
                 ScArgs sa;
@@ -1159,9 +1135,7 @@ static int enqueue_range(clfd_detector *det, const uint8_t *frames_dev, int fram
                 continue;
             }
             if (ev && ci == 0) CK(cudaEventRecord(ev[5], s));
-            if (!(parts & kPartCascades)) {
-                // (enqueue_overlapped: this call only puts the range's patch kernel on its own stream)
-            } else if (pk.dense[0].tail_stages > 0) {
+            if (pk.dense[0].tail_stages > 0) {
                 // ystep-2 levels (de-interleaved tile layout) and ystep-1 levels (natural layout)
                 if (cp.n_tiles_y2 > 0) { CK(launch_cascade_tiles(cp.dense[1], a, 0, cp.n_tiles_y2, s)); launches++; }
                 if (cp.n_tiles > cp.n_tiles_y2) {
@@ -1177,9 +1151,7 @@ static int enqueue_range(clfd_detector *det, const uint8_t *frames_dev, int fram
             if (ev && ci == 0) CK(cudaEventRecord(ev[6], s));
             // cascades the tile kernel finishes itself (tail_stages == total_stages) never fill the queue
             const bool tiles_finish = pk.dense[0].tail_stages > 0 && pk.dense[0].exec_stages == pk.dense[0].total_stages;
-            if (cp.use_patch) {   // the tile kernel stopped at cut_stages: a warp per survivor finishes the cascade
-                if (parts & kPartPatch) { CK(launch_cascade_patch(cp.patch, a, ctx->n_sms, s)); launches++; }
-            } else if (!tiles_finish) {
+            if (!tiles_finish) {
                 if (cp.mid_end > cp.mid_begin) {
                     // ping-pong between the tile queue (counters[1]) and queue_b (count_b)
                     QueueItem *qs[2] = {det->queue.p, det->queue_b.p};
@@ -1241,10 +1213,6 @@ static int overlap_setup(clfd_detector *det) {
     CK(cudaEventCreateWithFlags(&det->ev_fork, cudaEventDisableTiming));
     for (auto &e : det->ev_pyr) CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
     for (auto &e : det->ev_tile) CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-    // the patch kernels (small CTAs, a warp per deep window) get the slots a draining tile CTA frees before the next tile CTA
-    CK(cudaStreamCreateWithPriority(&det->patch_stream, cudaStreamNonBlocking, hi));
-    for (auto &e : det->ev_tiled) CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-    CK(cudaEventCreateWithFlags(&det->ev_patch, cudaEventDisableTiming));
     return 0;
 }
 static int enqueue_overlapped(clfd_detector *det, const uint8_t *frames_dev, int n_frames, size_t frame_stride, int row_stride,
@@ -1268,20 +1236,10 @@ static int enqueue_overlapped(clfd_detector *det, const uint8_t *frames_dev, int
         CK(cudaStreamWaitEvent(t, det->ev_pyr[k], 0));
         rc = enqueue_range(det, src, f0, f1 - f0, frame_stride, row_stride, t, false, n_launches, slot, kPartCascades);
         if (rc) return rc;
-        if (det->cas[0]->use_patch) {   // this chunk's patch kernel does not hold up the tile kernel of the chunk after the next
-            CK(cudaEventRecord(det->ev_tiled[k], t));
-            CK(cudaStreamWaitEvent(det->patch_stream, det->ev_tiled[k], 0));
-            rc = enqueue_range(det, src, f0, f1 - f0, frame_stride, row_stride, det->patch_stream, false, n_launches, slot, kPartPatch);
-            if (rc) return rc;
-        }
     }
     for (int i = 0; i < 2; i++) {
         CK(cudaEventRecord(det->ev_tile[i], det->tile_stream[i]));
         CK(cudaStreamWaitEvent(s, det->ev_tile[i], 0));
-    }
-    if (det->cas[0]->use_patch) {
-        CK(cudaEventRecord(det->ev_patch, det->patch_stream));
-        CK(cudaStreamWaitEvent(s, det->ev_patch, 0));
     }
     return 0;
 }

@@ -115,8 +115,6 @@ struct DenseParams {
     int n_fixed;        // leading stages run in fixed geometry (no compaction), <= n_stages
     int tail_stages;    // leading stages the tile kernel evaluates (upright stumps, linear): == total_stages
                         // when it finishes the cascade itself, otherwise survivors go to the deep kernel
-    int cut_stages;     // stages the tile kernel evaluates before it hands its survivors to the patch kernel (k_cascade_patch:
-                        // a warp per survivor, the window's own integral patch in shared memory); == tail_stages without one
     int g1_min;         // phase 2: more than this many windows in a warp -> thread per window (G = 1), max 16
     int tilted_tile;    // the cascade has tilted features: a second smem tile holds the tilted integral, right
                         // behind the first (tilted nodes' offsets already point into it)
@@ -126,8 +124,6 @@ struct DenseParams {
     int tile_h;         // window rows per tile: kTileH; kTileHSmall where two tiles (tilted) would leave one CTA per SM;
                         // 24 for plain stump cascades on ystep-2 levels
     int eq_x, eq_y, eq_w, eq_h;   // the variance rectangle inside the window (tempcv.cpp:614-616): (1, 1, w-2, h-2) at scale 1
-    int pool_min;       // stages after the fixed ones run POOLED (rows drawn from the whole tile's survivors, re-sorted by
-                        // bank class before every stage) while the tile has more than this many windows; 0: never
     int track_abs;      // some leaf value is a sentinel (|alpha| > 64: haarcascade_mcs_*): the static sum_eps of such a stage
                         // would send every window through the FP64 path; stage verdicts bound the FP32 sum by the
                         // magnitudes actually added instead (kernels_clod.cu, stage_verdict<TRACK>)

@@ -9,11 +9,6 @@ struct PackedCascade {
     int dense_stumps = 0;              // stumps in the stages the tile kernel evaluates
     std::vector<TailStump> tail[2];    // stumps of the tile-evaluated stages in tile-offset form, [ystep-1]
     std::vector<DenseStage> stage_tab[2];   // stage trees the tile kernel walks: all stages in execution order
-    // patch kernel (plain upright stump cascades the tile kernel could finish itself): the tile kernel stops at
-    // patch_cut stages (dense[].cut_stages) and k_cascade_patch finishes the survivors, a warp per window
-    int patch_cut = 0;                 // 0: no patch kernel
-    DenseParams patch;                 // stage table + geometry of the patch layout (natural order, row stride tile_stride)
-    std::vector<TailStump> patch_tail; // every stump record with its offsets in patch layout
     std::vector<DeepStage> deep_stages;  // global-memory blob of the deep kernel
     std::vector<DeepNode> deep_nodes;
     std::vector<int> tree_first_node;

@@ -264,15 +264,13 @@ void pack_sc_level(const HostCascade &c, double scale, int pitch, ScLevel &L, Sc
 // parameter resident (DenseStump, fixed-geometry phase).
 // allow_tiles = false: no stage for the tile kernel (tail_stages = exec_stages = 0), the generic kernels take the cascade.
 static void pack_dense_one(const HostCascade &c, int ystep, DenseParams &P, std::vector<TailStump> &tail,
-                           std::vector<DenseStage> &stage_tab, int &dense_stumps, int patch_stride = 0,
-                           bool allow_tiles = true) {
+                           std::vector<DenseStage> &stage_tab, int &dense_stumps, bool allow_tiles = true) {
     const int S = c.n_stages(), T = c.n_trees();
     memset(&P, 0, sizeof P);
     P.total_stages = S;
     P.win_w = c.win_w; P.win_h = c.win_h;
     P.tile_stride = dense_tile_stride(c.win_w, ystep);
     P.tile_half = dense_tile_half(c.win_w, ystep);
-    if (patch_stride > 0) { P.tile_stride = patch_stride; P.tile_half = 0; }   // patch layout: natural order, the window alone
     P.is_tree = c.is_tree ? 1 : 0;
     P.ystep = ystep;
     P.filter_eps = 9.5367431640625e-07f;  // 2^-20
@@ -350,7 +348,6 @@ static void pack_dense_one(const HostCascade &c, int ystep, DenseParams &P, std:
     for (int e = 0; e < E; e++) pos[order[e]] = e;
     P.tail_stages = elig;
     P.exec_stages = E;
-    P.cut_stages = elig;   // (pack_cascade lowers it when the cascade gets a patch kernel)
     P.g1_min = 12;   // measured: 8, 12, 16 within 0.6 % of each other, 12 best
     if (const char *e = getenv("CLFD_G1_MIN")) P.g1_min = std::max(1, std::min(16, atoi(e)));
     int n_elig_stumps = 0;
@@ -475,12 +472,6 @@ static void pack_dense_one(const HostCascade &c, int ystep, DenseParams &P, std:
         }
         tail.swap(blocked);
     }
-    // pooled stages (kernels_clod.cu): rows drawn from the whole tile's survivors while it holds more than pool_min
-    // windows.  OFF by default: on B200 they cut the shared-memory wavefronts by 17 % and the instructions by 5 %
-    // (ncu, profiles/r2_pooled_*.csv) but the block barrier per stage costs as much again (21.6 -> 22.0 ms per 64
-    // frames at pool_min = 64); kept as a tested A/B hook (CLFD_POOL_MIN=n, best with CLFD_N_FIXED=2)
-    P.pool_min = 0;
-    if (const char *e = getenv("CLFD_POOL_MIN")) P.pool_min = std::max(0, atoi(e));
     // sentinel leaf values (haarcascade_mcs_upperbody has one of 2.2e6 in stage 2): sum_eps, built from the largest
     // leaf of every stump, would exceed any real distance to the stage threshold and send every window of the stage
     // through the FP64 path; such cascades use the kernel instantiation that bounds the FP32 sum by what was added
@@ -538,32 +529,7 @@ void pack_cascade(const HostCascade &c, PackedCascade &out) {
     // uses the tile kernel and the generic kernels take the whole cascade on every level.
     if (out.dense[0].tail_stages != out.dense[1].tail_stages || out.dense[0].exec_stages != out.dense[1].exec_stages)
         for (int yi = 0; yi < 2; yi++)
-            pack_dense_one(c, yi + 1, out.dense[yi], out.tail[yi], out.stage_tab[yi], out.dense_stumps, 0, false);
-    // Patch kernel (A/B hook, OFF by default: CLFD_PATCH_CUT=n switches it on).  A window that survives the first stages
-    // is rare and goes deep: finished inside the tile kernel it keeps one warp busy for tens of microseconds while the
-    // CTA's other warps have nothing left (15 % of the tile kernel's warp slots, tools/tile_timing.py).  With a cut the
-    // tile kernel of a plain upright stump cascade stops after `cut` stages and its survivors go through the queue to
-    // k_cascade_patch, a warp per window.  Measured on B200 (frontalface_alt, 1080p, batch 64): the tile kernel drops from
-    // 21.1 to 18.3 ms at cut 8 (19.7 at 10, 20.4 at 12), but the patch kernel needs 5.3 ms for the 2.5 M windows -- 10 us
-    // per window and warp, a chain of dependent record fetches, reductions and verdicts that 32 resident warps per SM
-    // cannot hide -- so every cut is slower than none (2556 / 2760 / 2826 against 2853 frames/s).
-    out.patch_cut = 0;
-    const DenseParams &D = out.dense[0];
-    const bool finishes = D.tail_stages == S && D.exec_stages == S && out.dense[1].tail_stages == S;
-    if (finishes && !c.has_tilted && !c.is_tree && c.is_stump_based && D.npt == 1 && !D.track_abs && !out.dense[1].track_abs && S >= 8) {
-        int cut = 0;
-        if (const char *e = getenv("CLFD_PATCH_CUT")) cut = atoi(e);
-        if (cut > 0 && cut < S) {
-            cut = std::max(cut, std::max(D.n_fixed, out.dense[1].n_fixed));
-            std::vector<DenseStage> no_tab;
-            int n_stumps = 0;
-            pack_dense_one(c, 1, out.patch, out.patch_tail, no_tab, n_stumps, (c.win_w + 1) | 1);
-            if (out.patch.tail_stages == S && cut < S) {
-                out.patch_cut = cut;
-                for (int yi = 0; yi < 2; yi++) out.dense[yi].cut_stages = cut;
-            }
-        }
-    }
+            pack_dense_one(c, yi + 1, out.dense[yi], out.tail[yi], out.stage_tab[yi], out.dense_stumps, false);
 }
 
 // Tile-kernel blob of ONE scale of the scale-cascade mode, for the scales whose window step is

@@ -91,8 +91,7 @@ struct CascadeArgs {
     int count_exact;                // tile kernel: the instantiation that counts FP64 fallbacks / near-threshold sums (counters[4], [5])
     long long windows_per_frame;
     int16_t *codes;                 // device, [n_frames][windows_per_frame] or NULL
-    QueueItem *queue; unsigned long long queue_cap;   // written by the tile kernel / k_enqueue_all, counted in *qcount
-    unsigned long long *qcount;     // items in `queue`: counters + 1, or (patch kernel) the range's own counter
+    QueueItem *queue; unsigned long long queue_cap;   // written by the tile kernel / k_enqueue_all, counted in counters[1]
     // mid kernel pass: input queue (NULL = every grid window) -> output queue
     const QueueItem *mid_in; const unsigned long long *mid_in_count;
     QueueItem *mid_out; unsigned long long *mid_out_count;
@@ -113,10 +112,6 @@ cudaError_t launch_cascade_deep(const CascadeArgs &a, int n_sms, cudaStream_t st
 // reject-level output: scans the exit codes of n_frames frames, appends the candidates of
 // tempcv.cpp:1084-1094 (count at counter[0]) with the exact stage sum of their last stage
 cudaError_t launch_roc_collect(const CascadeArgs &a, RocItem *out, unsigned long long cap, unsigned long long *counter, cudaStream_t stream);
-
-// the survivors the tile kernel handed over at DenseParams::cut_stages, a warp per window
-// P: the cascade's patch blob (PackedCascade::patch: records in patch layout)
-cudaError_t launch_cascade_patch(const DenseParams &P, const CascadeArgs &a, int n_sms, cudaStream_t stream);
 
 // ---- scale-cascade mode (kernels_sc.cu) -----------------------------------------------
 struct ScArgs {

@@ -357,36 +357,16 @@ def test_generic_kernels_behind_the_tile_kernel(gpu_ctx, monkeypatch, hook, name
 
 @pytest.mark.parametrize("env", [{"CLFD_FORCE_EXACT": "1"}, {"CLFD_N_FIXED": "0"}, {"CLFD_N_FIXED": "5"}, {"CLFD_G1_MIN": "1"},
                                  {"CLFD_G1_MIN": "16"}, {"CLFD_TILE_H2": "32", "CLFD_NO_SMALL_TILES": "1"},
-                                 {"CLFD_POOL_MIN": "64", "CLFD_N_FIXED": "2"}, {"CLFD_POOL_MIN": "1", "CLFD_N_FIXED": "0"},
-                                 {"CLFD_NO_DI": "1"}])
+                                 {"CLFD_N_FIXED": "2"}, {"CLFD_NO_DI": "1"}])
 def test_tile_kernel_variants_under_every_split(gpu_ctx, monkeypatch, env):
-    """stage tree / multi-node / tilted variants of the tile kernel: all-FP64 evaluation, no fixed
-    stages (the stage-tree walk starts from a dealt list when the linear prefix is all fixed:
-    N_FIXED=5), thread-per-window only, pooled stages (rows drawn from the whole tile, block barrier per stage),
-    the ystep-2 levels' integral in natural order (LDG + STS tile staging instead of the TMA copies from a
-    column-de-interleaved integral, which every other test runs with)."""
+    """stage tree / multi-node / tilted variants of the tile kernel: all-FP64 evaluation, no, two or five
+    fixed stages (the stage-tree walk starts from a dealt list when the linear prefix is all fixed:
+    N_FIXED=5), thread-per-window only, the ystep-2 levels' integral in natural order (LDG + STS tile
+    staging instead of the TMA copies from a column-de-interleaved integral, which every other test runs with)."""
     for k, v in env.items():
         monkeypatch.setenv(k, v)
     _compare(gpu_ctx, ["frontalface_alt_tree", "frontalface_alt2", "eye_tree_eyeglasses", "fullbody", "frontalface_alt"],
              np.stack([octave_frame(400, 300, 8)]), 1.2)
-
-
-@pytest.mark.parametrize("cut", [0, 3, 5, 13, 21])
-def test_patch_kernel_any_cut(gpu_ctx, monkeypatch, cut):
-    """Plain stump cascades, A/B hook CLFD_PATCH_CUT (default 0 = the tile kernel does it all): the tile kernel stops
-    after `cut` stages and k_cascade_patch -- a warp per survivor, the window's own integral patch in shared memory,
-    the next window's patch arriving through cp.async meanwhile -- finishes them.  Exit codes, rects and the
-    FP64-fallback counters (diagnostic instantiations) and the production kernels' rects must not depend on the cut."""
-    monkeypatch.setenv("CLFD_PATCH_CUT", str(cut))
-    frames = np.stack([octave_frame(480, 360, 30 + i) for i in range(2)])
-    assert clfd.Cascade(cascade_path("frontalface_alt")).info.dense_stages == 22
-    _compare(gpu_ctx, ["frontalface_alt", "frontalface_default", "profileface"], frames, 1.2)
-    for nm in ("frontalface_alt", "frontalface_default"):
-        det = clfd.Detector(gpu_ctx, clfd.Cascade(cascade_path(nm)), 480, 360, max_batch=2, scale_factor=1.2)
-        res = det.detect(frames)
-        for f in range(2):
-            assert np.array_equal(res.frame_rects(f), _sorted(oracle_cascade(nm).detect(frames[f], 1.2, want_codes=False)[0])), (nm, f)
-        det.close()
 
 
 @pytest.mark.parametrize("name", ["frontalface_alt", "eye", "frontalface_alt2", "frontalface_alt_tree", "fullbody", "mcs_nose"])
