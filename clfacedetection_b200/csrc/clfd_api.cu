@@ -276,7 +276,7 @@ constexpr int kCnt = 8;
 struct CascadePlan {
     const clfd_cascade *cascade = nullptr;   // retained
     ~CascadePlan() { cascade_release(cascade); }
-    std::vector<CasLevel> levels;
+    std::vector<CasLevel> levels;   // the tile kernel's levels (scale-cascade mode: its scales of window step 2)
     std::vector<clfd_level> pub_levels;
     int n_tiles = 0;
     int n_tiles_y2 = 0;   // tiles of the ystep-2 levels (they come first)
@@ -292,10 +292,9 @@ struct CascadePlan {
     DevBuf<ScLevel> d_sc_levels;
     DevBuf<ScNode> d_sc_nodes;
     int sc_rows = 0;
-    // scales with window step 2 run through the tile kernel (pack_sc_dense): one blob + launch per scale
+    // scales with window step 2 run through the tile kernel (pack_sc_dense): one blob + launch per scale, grid levels[i]
     struct ScTile { DenseParams P; DevBuf<TailStump> tail; DevBuf<DenseStage> stage_tab; int tile_base = 0, n_tiles = 0; };
     std::vector<std::unique_ptr<ScTile>> sc_tiles;
-    DevBuf<CasLevel> d_sc_tile_levels;
     long long sc_tile_windows = 0;   // grid positions [0, sc_tile_windows) of a frame belong to those scales
     DevBuf<TailStump> d_tail[2];   // warp-per-window tail records of the tile kernel, [ystep-1]
     DevBuf<DenseStage> d_stage_tab[2];   // stage trees: stage table in execution order
@@ -305,31 +304,42 @@ struct CascadePlan {
     DevBuf<unsigned long long> d_counters;
     DevBuf<unsigned long long> d_count_b;   // second-queue counter, one per slot
     int mid_begin = 0, mid_end = 0;         // stages of the thread-per-window mid kernel (equal: none)
-    std::vector<int> mid_cuts;              // pass boundaries: mid_begin = cuts[0] < ... < cuts.back() = mid_end
-    unsigned long long h_counters[kCnt] = {0};
+    std::vector<int> pass_cuts;   // stage bounds of the survivor passes: mid kernel (mid_begin..mid_end) or k_sc_eval
+    int sc_deep_from = 0;                   // first stage of the k_sc_deep pass (n_stages: none)
 };
 
 constexpr int kMaxChunks = 8;
 constexpr int kSlots = 2;            // batches in flight through clfd_detect_submit / _collect
 constexpr int kEagerRects = 1 << 16; // rects copied back with the counters; more cost one extra copy
 
+// One batch in flight through clfd_detect_submit / _collect.  Slot 0's rects are allocated with the detector, the pinned
+// ones for rect_cap (clfd_detector_fetch copies through them); slot 1's at its first submit, the pinned ones for kEagerRects.
+struct BatchSlot {
+    DevBuf<uint8_t> frames;    // gray staging for host input (clfd_detect / clfd_detect_submit)
+    DevBuf<uint8_t> color;     // interleaved colour staging of clfd_detect_submit_color, allocated at first use
+    DevBuf<DevRect> rects;
+    DevRect *h_rects = nullptr;                 // pinned
+    unsigned long long *h_counters = nullptr;   // pinned, kCnt per cascade, 16 cascades
+    cudaEvent_t done = nullptr;
+    int n_frames = 0;
+    ~BatchSlot() {
+        if (h_rects) cudaFreeHost(h_rects);
+        if (h_counters) cudaFreeHost(h_counters);
+        if (done) cudaEventDestroy(done);
+    }
+};
+
 struct clfd_detector {
     clfd_context *ctx = nullptr;
     clfd_detector_config cfg;
     PyramidPlan pyr;
     std::vector<std::unique_ptr<CascadePlan>> cas;
+    // the kernels of one cascade for one range of frames (enqueue_range): enqueue_sc_cascade or enqueue_pyramid_cascade
+    int (*enqueue_cascade)(clfd_detector *, const CascadePlan &, CascadeArgs &, int, cudaStream_t, cudaEvent_t *, int *) = nullptr;
     DevBuf<QueueItem> queue, queue_b;
-    DevBuf<DevRect> rects;
-    DevBuf<uint8_t> dev_frames[kSlots];   // staging for host input (clfd_detect / clfd_detect_submit)
-    DevBuf<uint8_t> dev_color[kSlots];    // interleaved colour staging of clfd_detect_submit_color, allocated at first use
-    DevBuf<DevRect> rects2;               // rect buffer of slot 1 (slot 0 uses `rects`)
+    BatchSlot slot[kSlots];
     DevBuf<RocItem> roc;                  // candidates of clfd_detector_reject_levels
     DevBuf<unsigned long long> roc_count;
-    DevRect *h_rects = nullptr;           // pinned, kSlots x rect_cap... slot 1 holds kEagerRects only
-    DevRect *h_rects1 = nullptr;
-    unsigned long long *h_counters = nullptr;  // pinned, kSlots x (kCnt per cascade, 16 cascades)
-    cudaEvent_t done[kSlots] = {nullptr, nullptr};
-    int slot_frames[kSlots] = {0, 0};
     long long n_submitted = 0, n_collected = 0;
     unsigned long long rect_cap = 0, queue_cap = 0;
     int last_frames = 0;
@@ -348,10 +358,6 @@ struct clfd_detector {
     cudaStream_t pyr_stream = nullptr, tile_stream[2] = {nullptr, nullptr};
     cudaEvent_t ev_fork = nullptr, ev_pyr[kMaxChunks] = {nullptr}, ev_tile[2] = {nullptr, nullptr};
     ~clfd_detector() {
-        if (h_rects) cudaFreeHost(h_rects);
-        if (h_rects1) cudaFreeHost(h_rects1);
-        if (h_counters) cudaFreeHost(h_counters);
-        for (auto &e : done) if (e) cudaEventDestroy(e);
         for (auto &e : ev) if (e) cudaEventDestroy(e);
         for (auto &e : copied) if (e) cudaEventDestroy(e);
         if (copy_stream) cudaStreamDestroy(copy_stream);
@@ -362,6 +368,29 @@ struct clfd_detector {
         for (auto &t : tile_stream) if (t) cudaStreamDestroy(t);
     }
 };
+
+// A survivor queue and its item counter; items == nullptr stands for every window of the grid.
+struct SurvivorQueue { QueueItem *items = nullptr; unsigned long long *count = nullptr; };
+
+// launch(stage_begin, stage_end, in, out) for each pass of cp.pass_cuts, ping-ponging between det->queue (counter
+// counters[1], the first pass's input if from_queue, else the grid) and det->queue_b (counter d_count_b[slot]).  A counter
+// is cleared before a pass writes its queue unless this range has not written that queue yet.  *next: the last output.
+template <class Launch>
+static int run_pass_chain(const clfd_detector *det, const CascadePlan &cp, int slot, bool from_queue, cudaStream_t s,
+                          int *launches, SurvivorQueue *next, Launch launch) {
+    const SurvivorQueue q[2] = {{det->queue.p, cp.d_counters.p + kCnt * slot + 1}, {det->queue_b.p, cp.d_count_b.p + slot}};
+    bool written[2] = {from_queue, false};
+    SurvivorQueue in = from_queue ? q[0] : SurvivorQueue();
+    for (size_t k = 0, out = from_queue; k + 1 < cp.pass_cuts.size(); k++, out ^= 1) {
+        if (written[out]) CK(cudaMemsetAsync(q[out].count, 0, sizeof(unsigned long long), s));   // holds an older pass
+        if (int rc = launch(cp.pass_cuts[k], cp.pass_cuts[k + 1], in, q[out])) return rc;
+        (*launches)++;
+        written[out] = true;
+        in = q[out];
+    }
+    *next = in;
+    return 0;
+}
 
 // ------------------------------------------------------------------------------------
 // misc
@@ -752,133 +781,145 @@ static int plan_tiles(CasLevel &CL, int tile_h, int tile_base) {
     return CL.tiles_x * CL.tiles_y;
 }
 
-int clfd_detector_create(clfd_context *ctx, const clfd_cascade *const *cascades, int n_cascades,
-                         const clfd_detector_config *cfg, clfd_detector **out) {
-    if (!ctx || !cascades || !cfg || !out) INVALID("NULL argument");
-    *out = nullptr;
-    if (n_cascades <= 0 || n_cascades > 16) INVALID("n_cascades %d outside 1..16", n_cascades);
-    if (cfg->width <= 0 || cfg->height <= 0 || cfg->max_batch <= 0 || cfg->max_batch > 65535)
-        INVALID("bad frame geometry / batch");
-    if (!(cfg->scale_factor > 1)) INVALID("scale factor must be > 1");   // tempcv.cpp:1224-1225
-    if (cfg->width > 65535 || cfg->height > 65535) INVALID("frame too large");
-    CK(cudaSetDevice(ctx->device));
-    std::unique_ptr<clfd_detector> det(new clfd_detector());
-    det->ctx = ctx; det->cfg = *cfg;
-    memset(&det->stats, 0, sizeof det->stats);
-    const int W = cfg->width, H = cfg->height;
-    int max_w = cfg->max_w, max_h = cfg->max_h;
-    if (max_h == 0 || max_w == 0) { max_h = H; max_w = W; }   // tempcv.cpp:1230-1234
-
-    if (cfg->mode != CLFD_MODE_SCALE_IMAGE && cfg->mode != CLFD_MODE_SCALE_CASCADE) INVALID("unknown mode %d", cfg->mode);
-    const bool scale_cascade = cfg->mode == CLFD_MODE_SCALE_CASCADE;
-    std::vector<std::pair<int, int>> sizes;          // union pyramid
-    std::vector<char> sizes_y2;                      // ... and whether a level's windows are 2 pixels apart (factor <= 2)
-    bool any_tilted = false;
-    for (int ci = 0; ci < n_cascades; ci++) {
-        if (!cascades[ci]) INVALID("cascade %d is NULL", ci);
-        // the image-pyramid kernels keep a window's corner offsets in bytes (DeepNode) and its squared integral modulo
-        // 2^32, exact while (w - 2)(h - 2) * 255^2 < 2^32; the scale-cascade mode has neither limit
-        const HostCascade &hc = cascades[ci]->host;
-        if (!scale_cascade && (hc.win_w > kMaxPyramidWindow || hc.win_h > kMaxPyramidWindow))
-            INVALID("cascade %d: window %dx%d is larger than %d pixels, the limit of the image-pyramid mode (the "
-                    "scale-cascade mode takes it)", ci, hc.win_w, hc.win_h, kMaxPyramidWindow);
-        det->cas.emplace_back(new CascadePlan());
-        det->cas.back()->cascade = cascades[ci];
-        const_cast<clfd_cascade *>(cascades[ci])->refs.fetch_add(1);   // released by ~CascadePlan
-        any_tilted |= cascades[ci]->host.has_tilted;
-    }
-    if (scale_cascade) {
-        // one "pyramid level": the frame itself (a same-size INTER_LINEAR resize is the identity)
-        sizes.push_back({W, H});
-        const int pitch = (int)round_up(W + 1, 8);
-        for (int ci = 0; ci < n_cascades; ci++) {
-            CascadePlan &cp = *det->cas[ci];
-            const HostCascade &hc = cascades[ci]->host;
-            int n_factors = 0;   // tempcv.cpp:1344-1350
-            double factor = 1;
-            for (; factor * hc.win_w < W - 10 && factor * hc.win_h < H - 10; factor *= cfg->scale_factor) n_factors++;
-            factor = 1;
-            for (; n_factors-- > 0; factor *= cfg->scale_factor) {   // tempcv.cpp:1361-1380
-                const double ystep = std::max(2., factor);
-                const int win_w = cv_round(hc.win_w * factor), win_h = cv_round(hc.win_h * factor);
-                const int endX = cv_round((W - win_w) / ystep), endY = cv_round((H - win_h) / ystep);
-                if (win_w < cfg->min_w || win_h < cfg->min_h) continue;
-                if (endX <= 0 || endY <= 0) continue;
-                if (cp.sc_levels.size() >= 255) INVALID("more than 255 scales");
-                ScLevel L;
-                memset(&L, 0, sizeof L);
-                L.factor = factor; L.ystep = ystep; L.win_w = win_w; L.win_h = win_h; L.nx = endX; L.ny = endY;
-                L.node_base = (int)(cp.sc_levels.size() * hc.n_nodes());
-                L.row_base = cp.sc_rows; L.win_base = cp.windows_per_frame;
-                cp.sc_rows += endY;
-                cp.windows_per_frame += (long long)endX * endY;
-                cp.sc_levels.push_back(L);
-                clfd_level pl;
-                pl.factor = factor; pl.img_w = W; pl.img_h = H; pl.win_w = win_w; pl.win_h = win_h;
-                pl.ystep = 0; pl.nx = endX; pl.ny = endY; pl.win_base = L.win_base;
-                cp.pub_levels.push_back(pl);
-            }
-            std::vector<ScNode> nodes(cp.sc_levels.size() * (size_t)hc.n_nodes());
-            for (size_t li = 0; li < cp.sc_levels.size(); li++)
-                pack_sc_level(hc, cp.sc_levels[li].factor, pitch, cp.sc_levels[li], nodes.data() + li * hc.n_nodes());
-            int rc2;
-            if ((rc2 = cp.d_sc_levels.upload(cp.sc_levels, ctx->stream)) || (rc2 = cp.d_sc_nodes.upload(nodes, ctx->stream))) return rc2;
-            CK(cudaStreamSynchronize(ctx->stream));   // `nodes` goes out of scope
-            // the leading scales whose window step is exactly 2 (factor <= 2): tile kernel
-            if (!getenv("CLFD_SC_NO_TILES")) {
-                std::vector<CasLevel> tl;
-                int tile_base = 0;
-                for (size_t li = 0; li < cp.sc_levels.size(); li++) {
-                    const ScLevel &L = cp.sc_levels[li];
-                    if (L.ystep != 2.0 || L.win_base != cp.sc_tile_windows) break;
-                    std::unique_ptr<CascadePlan::ScTile> t(new CascadePlan::ScTile);
-                    std::vector<TailStump> tail;
-                    std::vector<DenseStage> stab;
-                    if (!pack_sc_dense(hc, L.factor, t->P, tail, stab)) break;
-                    if ((rc2 = t->tail.upload(tail, ctx->stream)) || (!stab.empty() && (rc2 = t->stage_tab.upload(stab, ctx->stream)))) return rc2;
-                    CK(cudaStreamSynchronize(ctx->stream));
-                    t->P.tail = t->tail.p; t->P.stage_g = t->stage_tab.p;
-                    CasLevel CL;
-                    memset(&CL, 0, sizeof CL);
-                    CL.pyr_level = 0; CL.nx = L.nx; CL.ny = L.ny; CL.ystep = 2; CL.win_w = L.win_w; CL.win_h = L.win_h;
-                    CL.win_base = L.win_base; CL.factor = L.factor;
-                    t->tile_base = tile_base; t->n_tiles = plan_tiles(CL, t->P.tile_h, tile_base);
-                    tile_base += t->n_tiles;
-                    tl.push_back(CL);
-                    cp.sc_tiles.push_back(std::move(t));
-                    cp.sc_tile_windows = L.win_base + (long long)L.nx * L.ny;
-                }
-                if (!tl.empty()) {
-                    if ((rc2 = cp.d_sc_tile_levels.upload(tl, ctx->stream))) return rc2;
-                    CK(cudaStreamSynchronize(ctx->stream));
-                }
-            }
-            cp.bytes_cascade += (int64_t)(W + 1) * (H + 1) * (4 + 8 + (hc.has_tilted ? 4 : 0)) + nodes.size() * sizeof(ScNode);
-        }
-    } else {
-    // level loop, all cascades in lock step over the shared factor sequence
-    std::map<int, int> pyr_index;                    // factor index -> pyramid level
-    std::vector<bool> done(n_cascades, false);
+// Scale-cascade mode, one cascade: its scales over the frame itself (tempcv.cpp:1344-1380) with their k_sc_eval node
+// tables, the tile-kernel route of the leading scales of window step 2, and the schedule of the survivor passes.
+static int plan_sc_cascade(CascadePlan &cp, const clfd_detector_config &cfg, cudaStream_t s) {
+    const HostCascade &hc = cp.cascade->host;
+    const int W = cfg.width, H = cfg.height, pitch = (int)round_up(W + 1, 8);
+    int n_factors = 0;   // tempcv.cpp:1344-1350
     double factor = 1;
-    for (int k = 0;; k++, factor *= cfg->scale_factor) {
+    for (; factor * hc.win_w < W - 10 && factor * hc.win_h < H - 10; factor *= cfg.scale_factor) n_factors++;
+    factor = 1;
+    for (; n_factors-- > 0; factor *= cfg.scale_factor) {   // tempcv.cpp:1361-1380
+        const double ystep = std::max(2., factor);
+        const int win_w = cv_round(hc.win_w * factor), win_h = cv_round(hc.win_h * factor);
+        const int endX = cv_round((W - win_w) / ystep), endY = cv_round((H - win_h) / ystep);
+        if (win_w < cfg.min_w || win_h < cfg.min_h) continue;
+        if (endX <= 0 || endY <= 0) continue;
+        if (cp.sc_levels.size() >= 255) INVALID("more than 255 scales");
+        ScLevel L;
+        memset(&L, 0, sizeof L);
+        L.factor = factor; L.ystep = ystep; L.win_w = win_w; L.win_h = win_h; L.nx = endX; L.ny = endY;
+        L.node_base = (int)(cp.sc_levels.size() * hc.n_nodes());
+        L.row_base = cp.sc_rows; L.win_base = cp.windows_per_frame;
+        cp.sc_rows += endY;
+        cp.windows_per_frame += (long long)endX * endY;
+        cp.sc_levels.push_back(L);
+        clfd_level pl;
+        pl.factor = factor; pl.img_w = W; pl.img_h = H; pl.win_w = win_w; pl.win_h = win_h;
+        pl.ystep = 0; pl.nx = endX; pl.ny = endY; pl.win_base = L.win_base;
+        cp.pub_levels.push_back(pl);
+    }
+    std::vector<ScNode> nodes(cp.sc_levels.size() * (size_t)hc.n_nodes());
+    for (size_t li = 0; li < cp.sc_levels.size(); li++)
+        pack_sc_level(hc, cp.sc_levels[li].factor, pitch, cp.sc_levels[li], nodes.data() + li * hc.n_nodes());
+    int rc;
+    if ((rc = cp.d_sc_levels.upload(cp.sc_levels, s)) || (rc = cp.d_sc_nodes.upload(nodes, s))) return rc;
+    CK(cudaStreamSynchronize(s));   // `nodes` goes out of scope
+    // the leading scales whose window step is exactly 2 (factor <= 2): tile kernel
+    int tile_base = 0;
+    for (size_t li = 0; li < cp.sc_levels.size(); li++) {
+        const ScLevel &L = cp.sc_levels[li];
+        if (L.ystep != 2.0 || L.win_base != cp.sc_tile_windows) break;
+        std::unique_ptr<CascadePlan::ScTile> t(new CascadePlan::ScTile);
+        std::vector<TailStump> tail;
+        std::vector<DenseStage> stab;
+        if (!pack_sc_dense(hc, L.factor, t->P, tail, stab)) break;
+        if ((rc = t->tail.upload(tail, s)) || (!stab.empty() && (rc = t->stage_tab.upload(stab, s)))) return rc;
+        CK(cudaStreamSynchronize(s));
+        t->P.tail = t->tail.p; t->P.stage_g = t->stage_tab.p;
+        CasLevel CL;
+        memset(&CL, 0, sizeof CL);
+        CL.pyr_level = 0; CL.nx = L.nx; CL.ny = L.ny; CL.ystep = 2; CL.win_w = L.win_w; CL.win_h = L.win_h;
+        CL.win_base = L.win_base; CL.factor = L.factor;
+        t->tile_base = tile_base; t->n_tiles = plan_tiles(CL, t->P.tile_h, tile_base);
+        tile_base += t->n_tiles;
+        cp.levels.push_back(CL);
+        cp.sc_tiles.push_back(std::move(t));
+        cp.sc_tile_windows = L.win_base + (long long)L.nx * L.ny;
+    }
+    cp.bytes_cascade += (int64_t)(W + 1) * (H + 1) * (4 + 8 + (hc.has_tilted ? 4 : 0)) + nodes.size() * sizeof(ScNode);
+    // k_sc_eval passes over growing stage ranges (cumulative trees >= 10, 40, 90, 160, ... per pass), survivors
+    // re-compacted through the two queues in between; a stage tree runs as one pass.  From the first stage after stage 0
+    // that has >= 50 trees on, the survivors are finished one warp per position (k_sc_deep).
+    static const int limit[7] = {10, 40, 90, 160, 300, 500, 800};
+    cp.pass_cuts.assign(1, 0);
+    cp.sc_deep_from = hc.n_stages();
+    for (int st = 0, acc = 0; st < hc.n_stages() && !hc.is_tree; st++) {
+        if (st > 0 && hc.st_ntrees[st] >= 50) { cp.sc_deep_from = st; break; }
+        acc += hc.st_ntrees[st];
+        if (cp.pass_cuts.size() <= 7 && acc >= limit[cp.pass_cuts.size() - 1] && st + 1 < hc.n_stages()) { cp.pass_cuts.push_back(st + 1); acc = 0; }
+    }
+    if (cp.pass_cuts.back() != cp.sc_deep_from) cp.pass_cuts.push_back(cp.sc_deep_from);
+    return 0;
+}
+
+// Scale-cascade mode, one cascade: the tile kernel over the step-2 scales (exit codes only), the k_sc_eval passes,
+// k_sc_deep and k_sc_rows.  ev (cascade 0, profiling): ev[5] before the first kernel, ev[6] and ev[7] after the last.
+static int enqueue_sc_cascade(clfd_detector *det, const CascadePlan &cp, CascadeArgs &a, int slot, cudaStream_t s,
+                              cudaEvent_t *ev, int *launches) {
+    const int n_sms = det->ctx->n_sms, n_stages = cp.cascade->host.n_stages();
+    ScArgs sa;
+    memset(&sa, 0, sizeof sa);
+    const PyrLevel &L0 = det->pyr.levels[0];
+    sa.sum = a.sum + L0.sum_off; sa.sq = a.sq + L0.sum_off; sa.tilted = a.tilted ? a.tilted + L0.sum_off : nullptr;
+    sa.sum_frame_stride = a.sum_frame_stride;
+    sa.pitch = L0.sum_pitch; sa.W = det->cfg.width; sa.H = det->cfg.height;
+    sa.levels = cp.d_sc_levels.p; sa.nodes = cp.d_sc_nodes.p;
+    sa.n_levels = (int)cp.sc_levels.size(); sa.rows_per_frame = cp.sc_rows; sa.n_frames = a.n_frames;
+    sa.cascade_index = a.cascade_index; sa.frame_base = a.frame_base; sa.windows_per_frame = cp.windows_per_frame;
+    sa.codes = cp.d_codes.p + (size_t)a.frame_base * cp.windows_per_frame;
+    sa.rects = a.rects; sa.rect_cap = a.rect_cap; sa.counters = a.counters; sa.deep = a.deep; sa.queue_cap = det->queue_cap;
+    if (ev) CK(cudaEventRecord(ev[5], s));
+    CascadeArgs ta = a;   // the tile kernel, one launch per scale of window step 2
+    ta.codes = sa.codes; ta.rects = nullptr; ta.rect_cap = 0;
+    for (auto &t : cp.sc_tiles) { CK(launch_cascade_tiles(t->P, ta, t->tile_base, t->n_tiles, s)); (*launches)++; }
+    sa.first_window = cp.sc_tile_windows;
+    auto eval_pass = [&](int b, int e, SurvivorQueue in, SurvivorQueue out) -> int {
+        sa.stage_begin = b; sa.stage_end = e; sa.in = in.items; sa.in_count = in.count; sa.out = out.items; sa.out_count = out.count;
+        CK(launch_sc_eval(sa, n_sms, s));
+        return 0;
+    };
+    SurvivorQueue next;
+    if (int rc = run_pass_chain(det, cp, slot, false, s, launches, &next, eval_pass)) return rc;
+    if (cp.sc_deep_from < n_stages) {
+        sa.stage_begin = cp.sc_deep_from; sa.stage_end = n_stages; sa.in = next.items; sa.in_count = next.count;
+        CK(launch_sc_deep(sa, n_sms, s)); (*launches)++;
+    }
+    CK(launch_sc_rows(sa, s)); (*launches)++;
+    if (ev) { CK(cudaEventRecord(ev[6], s)); CK(cudaEventRecord(ev[7], s)); }
+    return 0;
+}
+
+// Image-pyramid mode: the level loop, all cascades in lock step over the shared factor sequence.  sizes: the union
+// pyramid; sizes_y2: whether a level's windows are 2 pixels apart (factor <= 2).
+static int plan_pyramid_levels(clfd_detector *det, std::vector<std::pair<int, int>> &sizes, std::vector<char> &sizes_y2) {
+    const clfd_detector_config &cfg = det->cfg;
+    const int W = cfg.width, H = cfg.height;
+    int max_w = cfg.max_w, max_h = cfg.max_h;
+    if (max_h == 0 || max_w == 0) { max_h = H; max_w = W; }   // tempcv.cpp:1230-1234
+    std::map<int, int> pyr_index;                    // factor index -> pyramid level
+    std::vector<bool> done(det->cas.size(), false);
+    double factor = 1;
+    for (int k = 0;; k++, factor *= cfg.scale_factor) {
         bool all_done = true;
         if (k >= 255) INVALID("more than 255 pyramid levels");
         const int sz_w = cv_round(W / factor), sz_h = cv_round(H / factor);
-        for (int ci = 0; ci < n_cascades; ci++) {
+        for (size_t ci = 0; ci < det->cas.size(); ci++) {
             if (done[ci]) continue;
-            const HostCascade &hc = cascades[ci]->host;
+            CascadePlan &cp = *det->cas[ci];
+            const HostCascade &hc = cp.cascade->host;
             const int win_w = cv_round(hc.win_w * factor), win_h = cv_round(hc.win_h * factor);
             const int sz1_w = sz_w - hc.win_w + 1, sz1_h = sz_h - hc.win_h + 1;
             if (sz1_w <= 0 || sz1_h <= 0) { done[ci] = true; continue; }                 // :1283
             if (win_w > max_w || win_h > max_h) { done[ci] = true; continue; }           // :1285
             all_done = false;
-            if (win_w < cfg->min_w || win_h < cfg->min_h) continue;                      // :1287
+            if (win_w < cfg.min_w || win_h < cfg.min_h) continue;                        // :1287
             const int ystep = factor > 2 ? 1 : 2;                                        // :1021
             const int xe = sz_w - hc.win_w, ye = sz_h - hc.win_h;                        // :1015-1020
             const int nx = xe > 0 ? (xe + ystep - 1) / ystep : 0, ny = ye > 0 ? (ye + ystep - 1) / ystep : 0;
             if (nx == 0 || ny == 0) continue;
             if (!pyr_index.count(k)) { pyr_index[k] = (int)sizes.size(); sizes.push_back({sz_w, sz_h}); sizes_y2.push_back(ystep == 2); }
-            CascadePlan &cp = *det->cas[ci];
             CasLevel CL;
             memset(&CL, 0, sizeof CL);
             CL.pyr_level = pyr_index[k];
@@ -898,9 +939,108 @@ int clfd_detector_create(clfd_context *ctx, const clfd_cascade *const *cascades,
         }
         if (all_done) break;
     }
+    return 0;
+}
+
+// Image-pyramid mode, mid kernel: the stages right after the tile prefix of a LINEAR cascade whose trees the tile
+// kernel cannot take, while they are too small for a warp per window (< 24 trees), at most 8.  Passes: the first ends
+// once it holds >= 10 trees, the later ones >= 30 (lanes are re-compacted between passes).
+static void plan_mid_passes(CascadePlan &cp) {
+    const HostCascade &hc = cp.cascade->host;
+    const DenseParams &P0 = cp.cascade->packed.dense[0];
+    if (hc.is_tree || P0.tail_stages >= P0.total_stages) return;
+    cp.mid_begin = cp.mid_end = P0.tail_stages;
+    while (cp.mid_end < hc.n_stages() && cp.mid_end - cp.mid_begin < 8 && hc.st_ntrees[cp.mid_end] < 24) cp.mid_end++;
+    cp.pass_cuts.assign(1, cp.mid_begin);
+    for (int st = cp.mid_begin, acc = 0; st < cp.mid_end; st++) {
+        acc += hc.st_ntrees[st];
+        if (acc >= (cp.pass_cuts.size() == 1 ? 10 : 30) || st + 1 == cp.mid_end) { cp.pass_cuts.push_back(st + 1); acc = 0; }
+    }
+}
+
+// Image-pyramid mode, one cascade: the tile kernel (or k_enqueue_all), the mid passes and the deep kernel.  ev (cascade
+// 0, profiling): ev[5] before the first kernel, ev[6] after the tile kernel, ev[7] after the last.
+static int enqueue_pyramid_cascade(clfd_detector *det, const CascadePlan &cp, CascadeArgs &a, int slot, cudaStream_t s,
+                                   cudaEvent_t *ev, int *launches) {
+    const DenseParams &P0 = cp.cascade->packed.dense[0];
+    const bool has_mid = cp.mid_end > cp.mid_begin;
+    if (ev) CK(cudaEventRecord(ev[5], s));
+    if (P0.tail_stages > 0) {
+        // ystep-2 levels (de-interleaved tile layout) and ystep-1 levels (natural layout)
+        if (cp.n_tiles_y2 > 0) { CK(launch_cascade_tiles(cp.dense[1], a, 0, cp.n_tiles_y2, s)); (*launches)++; }
+        if (cp.n_tiles > cp.n_tiles_y2) {
+            CK(launch_cascade_tiles(cp.dense[0], a, cp.n_tiles_y2, cp.n_tiles - cp.n_tiles_y2, s));
+            (*launches)++;
+        }
+    } else if (!has_mid) {   // (with mid passes, the first one walks the window grid itself)
+        CK(launch_enqueue_all(a, s)); (*launches)++;
+    }
+    if (ev) CK(cudaEventRecord(ev[6], s));
+    // cascades the tile kernel finishes itself (tail_stages == total_stages) never fill the queue
+    const bool tiles_finish = P0.tail_stages > 0 && P0.exec_stages == P0.total_stages;
+    if (!tiles_finish) {
+        if (has_mid) {
+            auto mid_pass = [&](int b, int e, SurvivorQueue in, SurvivorQueue out) -> int {
+                a.deep.mid_begin = b; a.deep.mid_end = e;
+                a.mid_in = in.items; a.mid_in_count = in.count; a.mid_out = out.items; a.mid_out_count = out.count;
+                CK(launch_cascade_mid(a, det->ctx->n_sms, s));
+                return 0;
+            };
+            SurvivorQueue next;
+            if (int rc = run_pass_chain(det, cp, slot, P0.tail_stages > 0, s, launches, &next, mid_pass)) return rc;
+            a.deep_in = next.items; a.deep_count = next.count;
+        }
+        if (cp.mid_end < P0.total_stages) { CK(launch_cascade_deep(a, det->ctx->n_sms, s)); (*launches)++; }
+    }
+    if (ev) CK(cudaEventRecord(ev[7], s));
+    return 0;
+}
+
+int clfd_detector_create(clfd_context *ctx, const clfd_cascade *const *cascades, int n_cascades,
+                         const clfd_detector_config *cfg, clfd_detector **out) {
+    if (!ctx || !cascades || !cfg || !out) INVALID("NULL argument");
+    *out = nullptr;
+    if (n_cascades <= 0 || n_cascades > 16) INVALID("n_cascades %d outside 1..16", n_cascades);
+    if (cfg->width <= 0 || cfg->height <= 0 || cfg->max_batch <= 0 || cfg->max_batch > 65535)
+        INVALID("bad frame geometry / batch");
+    if (!(cfg->scale_factor > 1)) INVALID("scale factor must be > 1");   // tempcv.cpp:1224-1225
+    if (cfg->width > 65535 || cfg->height > 65535) INVALID("frame too large");
+    CK(cudaSetDevice(ctx->device));
+    std::unique_ptr<clfd_detector> det(new clfd_detector());
+    det->ctx = ctx; det->cfg = *cfg;
+    memset(&det->stats, 0, sizeof det->stats);
+    const int W = cfg->width, H = cfg->height;
+
+    if (cfg->mode != CLFD_MODE_SCALE_IMAGE && cfg->mode != CLFD_MODE_SCALE_CASCADE) INVALID("unknown mode %d", cfg->mode);
+    const bool scale_cascade = cfg->mode == CLFD_MODE_SCALE_CASCADE;
+    bool any_tilted = false;
+    for (int ci = 0; ci < n_cascades; ci++) {
+        if (!cascades[ci]) INVALID("cascade %d is NULL", ci);
+        // the image-pyramid kernels keep a window's corner offsets in bytes (DeepNode) and its squared integral modulo
+        // 2^32, exact while (w - 2)(h - 2) * 255^2 < 2^32; the scale-cascade mode has neither limit
+        const HostCascade &hc = cascades[ci]->host;
+        if (!scale_cascade && (hc.win_w > kMaxPyramidWindow || hc.win_h > kMaxPyramidWindow))
+            INVALID("cascade %d: window %dx%d is larger than %d pixels, the limit of the image-pyramid mode (the "
+                    "scale-cascade mode takes it)", ci, hc.win_w, hc.win_h, kMaxPyramidWindow);
+        det->cas.emplace_back(new CascadePlan());
+        det->cas.back()->cascade = cascades[ci];
+        const_cast<clfd_cascade *>(cascades[ci])->refs.fetch_add(1);   // released by ~CascadePlan
+        any_tilted |= cascades[ci]->host.has_tilted;
     }
     cudaStream_t s = ctx->stream;
     int rc = 0;
+    std::vector<std::pair<int, int>> sizes;          // union pyramid
+    std::vector<char> sizes_y2;                      // ... and whether a level's windows are 2 pixels apart (factor <= 2)
+    if (scale_cascade) {
+        // one "pyramid level": the frame itself (a same-size INTER_LINEAR resize is the identity)
+        sizes.push_back({W, H});
+        for (auto &cpp : det->cas)
+            if ((rc = plan_sc_cascade(*cpp, *cfg, s))) return rc;
+    } else {
+        if ((rc = plan_pyramid_levels(det.get(), sizes, sizes_y2))) return rc;
+        for (auto &cpp : det->cas) plan_mid_passes(*cpp);
+    }
+    det->enqueue_cascade = scale_cascade ? enqueue_sc_cascade : enqueue_pyramid_cascade;
     // pyramid mode: every sum of squares the kernels form is a cascade window's (< 2^32), so the squared integral is
     // kept modulo 2^32 -- a third less integral traffic; the scale-cascade mode's windows grow with the scale: 64 bits
     det->pyr.sq32 = !scale_cascade && !getenv("CLFD_SQ64");
@@ -913,29 +1053,12 @@ int clfd_detector_create(clfd_context *ctx, const clfd_cascade *const *cascades,
     else if (sizes.empty()) { det->pyr.W = W; det->pyr.H = H; det->pyr.max_batch = cfg->max_batch; }
 
     long long max_wpf = 0;
-    bool need_queue_b = false;
+    bool need_queue_b = scale_cascade;
     for (auto &cpp : det->cas) {
         CascadePlan &cp = *cpp;
-        const PackedCascade &pk = cp.cascade->packed;
         if ((rc = cp.d_levels.upload(cp.levels, s)) || (rc = upload_cascade(cp, s))) return rc;
         if ((rc = cp.d_counters.alloc(kCnt * kSlots)) || (rc = cp.d_count_b.alloc(kSlots))) return rc;
-        // mid kernel: the stages right after the tile prefix of a LINEAR cascade whose trees the tile
-        // kernel cannot take, while they are too small for a warp per window (< 24 trees), at most 8
-        if (!scale_cascade && !cp.cascade->host.is_tree && pk.dense[0].tail_stages < pk.dense[0].total_stages) {
-            const HostCascade &hc = cp.cascade->host;
-            cp.mid_begin = cp.mid_end = pk.dense[0].tail_stages;
-            while (cp.mid_end < hc.n_stages() && cp.mid_end - cp.mid_begin < 8 && hc.st_ntrees[cp.mid_end] < 24) cp.mid_end++;
-            if (getenv("CLFD_NO_MID")) cp.mid_end = cp.mid_begin;
-            need_queue_b |= cp.mid_end > cp.mid_begin;
-            // passes: the first ends once it holds >= 10 trees, the later ones >= 30 (lanes are
-            // re-compacted between passes)
-            cp.mid_cuts.assign(1, cp.mid_begin);
-            int acc = 0;
-            for (int st = cp.mid_begin; st < cp.mid_end; st++) {
-                acc += hc.st_ntrees[st];
-                if (acc >= (cp.mid_cuts.size() == 1 ? 10 : 30) || st + 1 == cp.mid_end) { cp.mid_cuts.push_back(st + 1); acc = 0; }
-            }
-        }
+        need_queue_b |= cp.mid_end > cp.mid_begin;
         if ((cfg->want_codes || scale_cascade) && (rc = cp.d_codes.alloc((size_t)std::max<long long>(cp.windows_per_frame, 1) * cfg->max_batch)))
             return rc;
         max_wpf = std::max(max_wpf, cp.windows_per_frame);
@@ -943,10 +1066,10 @@ int clfd_detector_create(clfd_context *ctx, const clfd_cascade *const *cascades,
     }
     det->queue_cap = (unsigned long long)std::max<long long>(max_wpf, 1) * cfg->max_batch;
     det->rect_cap = cfg->max_rects > 0 ? (unsigned long long)cfg->max_rects : (1ull << 20);
-    if ((rc = det->queue.alloc(det->queue_cap)) || (rc = det->rects.alloc(det->rect_cap))) return rc;
-    if ((need_queue_b || scale_cascade) && (rc = det->queue_b.alloc(det->queue_cap))) return rc;
-    CK(cudaMallocHost((void **)&det->h_rects, det->rect_cap * sizeof(DevRect)));
-    CK(cudaMallocHost((void **)&det->h_counters, kSlots * kCnt * 16 * sizeof(unsigned long long)));
+    if ((rc = det->queue.alloc(det->queue_cap)) || (rc = det->slot[0].rects.alloc(det->rect_cap))) return rc;
+    if (need_queue_b && (rc = det->queue_b.alloc(det->queue_cap))) return rc;
+    CK(cudaMallocHost((void **)&det->slot[0].h_rects, det->rect_cap * sizeof(DevRect)));
+    for (auto &sl : det->slot) CK(cudaMallocHost((void **)&sl.h_counters, kCnt * 16 * sizeof(unsigned long long)));
     CK(cudaStreamSynchronize(s));
     det->stats.pyramid_pixels = det->pyr.pyramid_pixels;
     det->stats.bytes_resize = det->pyr.bytes_resize;
@@ -1042,144 +1165,27 @@ static int enqueue_range(clfd_detector *det, const uint8_t *frames_dev, int fram
             else CK(cudaMemsetAsync(cpp->d_counters.p + kCnt * slot + 1, 0, sizeof(unsigned long long), s));   // the queue is per range
             CK(cudaMemsetAsync(cpp->d_count_b.p + slot, 0, sizeof(unsigned long long), s));
         }
-    if (!(parts & kPartCascades)) {
-        ctx->launches += launches;
-        *n_launches += launches;
-        return 0;
-    }
-    int ci = 0;
-    for (auto &cpp : det->cas) {
-        CascadePlan &cp = *cpp;
-        if (cp.windows_per_frame > 0) {
-            const PackedCascade &pk = cp.cascade->packed;
-            CascadeArgs a = cascade_args(det, cp, ci, frame_base, n_frames);
-            a.codes = det->cfg.want_codes ? cp.d_codes.p + (size_t)frame_base * cp.windows_per_frame : nullptr;
-            a.count_exact = det->cfg.want_codes ? 1 : 0;
-            a.queue = det->queue.p; a.queue_cap = det->queue_cap;
-            a.rects = slot ? det->rects2.p : det->rects.p; a.rect_cap = det->rect_cap;
-            a.counters = cp.d_counters.p + kCnt * slot;
-            a.deep_in = a.queue; a.deep_count = a.counters + 1;
-            if (det->cfg.mode == CLFD_MODE_SCALE_CASCADE) {
-                ScArgs sa;
-                memset(&sa, 0, sizeof sa);
-                const PyrLevel &L0 = det->pyr.levels[0];
-                sa.sum = a.sum + L0.sum_off; sa.sq = a.sq + L0.sum_off; sa.tilted = a.tilted ? a.tilted + L0.sum_off : nullptr;
-                sa.sum_frame_stride = a.sum_frame_stride;
-                sa.pitch = L0.sum_pitch; sa.W = det->cfg.width; sa.H = det->cfg.height;
-                sa.levels = cp.d_sc_levels.p; sa.nodes = cp.d_sc_nodes.p;
-                sa.n_levels = (int)cp.sc_levels.size(); sa.rows_per_frame = cp.sc_rows; sa.n_frames = n_frames;
-                sa.cascade_index = ci; sa.frame_base = frame_base; sa.windows_per_frame = cp.windows_per_frame;
-                sa.codes = cp.d_codes.p + (size_t)frame_base * cp.windows_per_frame;
-                sa.rects = a.rects; sa.rect_cap = a.rect_cap; sa.counters = a.counters; sa.deep = a.deep;
-                if (ev && ci == 0) CK(cudaEventRecord(ev[5], s));
-                // scales with window step 2: the tile kernel, one launch per scale, exit codes only
-                if (!cp.sc_tiles.empty()) {
-                    CascadeArgs ta = a;
-                    ta.cas_levels = cp.d_sc_tile_levels.p; ta.n_cas_levels = (int)cp.sc_tiles.size();
-                    ta.codes = sa.codes; ta.rects = nullptr; ta.rect_cap = 0;
-                    for (auto &t : cp.sc_tiles) {
-                        CK(launch_cascade_tiles(t->P, ta, t->tile_base, t->n_tiles, s));
-                        launches++;
-                    }
-                    sa.first_window = cp.sc_tile_windows;
-                }
-                // passes over growing stage ranges (cumulative trees >= 10, 40, 90, 160, ... per pass), survivors
-                // re-compacted through the two queues in between; a stage tree runs as one pass
-                {
-                    const HostCascade &hc = cp.cascade->host;
-                    std::vector<int> cuts(1, 0);
-                    int deep_from = hc.n_stages();   // first stage of the final warp-per-survivor pass
-                    if (hc.is_tree || getenv("CLFD_SC_ONE_PASS")) cuts.push_back(hc.n_stages());
-                    else {
-                        static const int limit[7] = {10, 40, 90, 160, 300, 500, 800};
-                        int acc = 0;
-                        int deep_min = 50;
-                        if (const char *e = getenv("CLFD_SC_DEEP_MIN")) deep_min = atoi(e);
-                        for (int st = 0; st < hc.n_stages(); st++) {
-                            // stages of >= 32 trees fill a warp's lanes: from the first one on (after at
-                            // least one thread pass) the survivors are finished one warp per position
-                            if (st > 0 && hc.st_ntrees[st] >= deep_min) { deep_from = st; break; }
-                            acc += hc.st_ntrees[st];
-                            if (cuts.size() <= 7 && acc >= limit[cuts.size() - 1] && st + 1 < hc.n_stages()) { cuts.push_back(st + 1); acc = 0; }
-                        }
-                        if (cuts.back() != deep_from) cuts.push_back(deep_from);
-                    }
-                    QueueItem *qs[2] = {det->queue.p, det->queue_b.p};
-                    unsigned long long *cs[2] = {a.counters + 1, cp.d_count_b.p + slot};
-                    sa.queue_cap = det->queue_cap;
-                    int in = -1;
-                    for (size_t k = 0; k + 1 < cuts.size(); k++) {
-                        const int out = in == 0 ? 1 : 0;
-                        if (k >= 2) CK(cudaMemsetAsync(cs[out], 0, sizeof(unsigned long long), s));   // holds an older pass
-                        sa.stage_begin = cuts[k]; sa.stage_end = cuts[k + 1];
-                        sa.in = in < 0 ? nullptr : qs[in]; sa.in_count = in < 0 ? nullptr : cs[in];
-                        sa.out = qs[out]; sa.out_count = cs[out];
-                        CK(launch_sc_eval(sa, ctx->n_sms, s));
-                        launches++;
-                        in = out;
-                    }
-                    if (deep_from < hc.n_stages()) {
-                        sa.stage_begin = deep_from; sa.stage_end = hc.n_stages();
-                        sa.in = qs[in]; sa.in_count = cs[in];
-                        CK(launch_sc_deep(sa, ctx->n_sms, s));
-                        launches++;
-                    }
-                }
-                CK(launch_sc_rows(sa, s));
-                launches++;
-                if (ev && ci == 0) { CK(cudaEventRecord(ev[6], s)); CK(cudaEventRecord(ev[7], s)); }
-                if (ci + 1 < (int)det->cas.size())
-                    CK(cudaMemcpyAsync(det->cas[ci + 1]->d_counters.p + kCnt * slot, cp.d_counters.p + kCnt * slot, sizeof(unsigned long long),
-                                       cudaMemcpyDeviceToDevice, s));
-                ci++;
-                continue;
+    if (parts & kPartCascades) {
+        for (size_t ci = 0; ci < det->cas.size(); ci++) {
+            const CascadePlan &cp = *det->cas[ci];
+            if (cp.windows_per_frame > 0) {
+                CascadeArgs a = cascade_args(det, cp, (int)ci, frame_base, n_frames);
+                a.codes = det->cfg.want_codes ? cp.d_codes.p + (size_t)frame_base * cp.windows_per_frame : nullptr;
+                a.count_exact = det->cfg.want_codes ? 1 : 0;
+                a.queue = det->queue.p; a.queue_cap = det->queue_cap;
+                a.rects = det->slot[slot].rects.p; a.rect_cap = det->rect_cap;
+                a.counters = cp.d_counters.p + kCnt * slot;
+                a.deep_in = a.queue; a.deep_count = a.counters + 1;
+                int rc = det->enqueue_cascade(det, cp, a, slot, s, ci == 0 ? ev : nullptr, &launches);
+                if (rc) return rc;
             }
-            if (ev && ci == 0) CK(cudaEventRecord(ev[5], s));
-            if (pk.dense[0].tail_stages > 0) {
-                // ystep-2 levels (de-interleaved tile layout) and ystep-1 levels (natural layout)
-                if (cp.n_tiles_y2 > 0) { CK(launch_cascade_tiles(cp.dense[1], a, 0, cp.n_tiles_y2, s)); launches++; }
-                if (cp.n_tiles > cp.n_tiles_y2) {
-                    CK(launch_cascade_tiles(cp.dense[0], a, cp.n_tiles_y2, cp.n_tiles - cp.n_tiles_y2, s));
-                    launches++;
-                }
-            } else if (cp.mid_end > cp.mid_begin) {
-                // no tile prefix: the first mid pass walks the window grid itself
-            } else {
-                CK(launch_enqueue_all(a, s));
-                launches++;
-            }
-            if (ev && ci == 0) CK(cudaEventRecord(ev[6], s));
-            // cascades the tile kernel finishes itself (tail_stages == total_stages) never fill the queue
-            const bool tiles_finish = pk.dense[0].tail_stages > 0 && pk.dense[0].exec_stages == pk.dense[0].total_stages;
-            if (!tiles_finish) {
-                if (cp.mid_end > cp.mid_begin) {
-                    // ping-pong between the tile queue (counters[1]) and queue_b (count_b)
-                    QueueItem *qs[2] = {det->queue.p, det->queue_b.p};
-                    unsigned long long *cs[2] = {a.counters + 1, cp.d_count_b.p + slot};
-                    int in = pk.dense[0].tail_stages > 0 ? 0 : -1;   // -1: the grid
-                    for (size_t k = 0; k + 1 < cp.mid_cuts.size(); k++) {
-                        const int out = in == 0 ? 1 : 0;
-                        if (k > 0) CK(cudaMemsetAsync(cs[out], 0, sizeof(unsigned long long), s));   // holds an older pass
-                        a.mid_in = in < 0 ? nullptr : qs[in]; a.mid_in_count = in < 0 ? nullptr : cs[in];
-                        a.mid_out = qs[out]; a.mid_out_count = cs[out];
-                        a.deep.mid_begin = cp.mid_cuts[k]; a.deep.mid_end = cp.mid_cuts[k + 1];
-                        CK(launch_cascade_mid(a, ctx->n_sms, s));
-                        launches++;
-                        in = out;
-                    }
-                    a.deep_in = qs[in]; a.deep_count = cs[in];
-                }
-                if (cp.mid_end < pk.dense[0].total_stages) { CK(launch_cascade_deep(a, ctx->n_sms, s)); launches++; }
-            }
-            if (ev && ci == 0) CK(cudaEventRecord(ev[7], s));
+            // all cascades append to one rect buffer: carry the rect count over
+            if (ci + 1 < det->cas.size())
+                CK(cudaMemcpyAsync(det->cas[ci + 1]->d_counters.p + kCnt * slot, cp.d_counters.p + kCnt * slot, sizeof(unsigned long long),
+                                   cudaMemcpyDeviceToDevice, s));
         }
-        // all cascades append to one rect buffer: carry the rect count over
-        if (ci + 1 < (int)det->cas.size())
-            CK(cudaMemcpyAsync(det->cas[ci + 1]->d_counters.p + kCnt * slot, cp.d_counters.p + kCnt * slot, sizeof(unsigned long long),
-                               cudaMemcpyDeviceToDevice, s));
-        ci++;
+        det->have_events = ev != nullptr;
     }
-    det->have_events = ev != nullptr;
     ctx->launches += launches;
     *n_launches += launches;
     return 0;
@@ -1294,9 +1300,9 @@ int clfd_detector_enqueue_color(clfd_detector *det, const uint8_t *frames_dev, i
     CK(cudaSetDevice(ctx->device));
     cudaStream_t s = cuda_stream ? (cudaStream_t)cuda_stream : ctx->stream;
     const size_t dstride = round_up(det->cfg.width, 16), dframe = dstride * det->cfg.height;
-    if (!det->dev_frames[0].p && (rc = det->dev_frames[0].alloc(dframe * det->cfg.max_batch + 64))) return rc;
-    if ((rc = enqueue_color_to_gray(det, frames_dev, n_frames, channels, frame_stride, row_stride, det->dev_frames[0].p, s))) return rc;
-    if ((rc = clfd_detector_enqueue(det, det->dev_frames[0].p, n_frames, dframe, (int)dstride, cuda_stream))) return rc;
+    if (!det->slot[0].frames.p && (rc = det->slot[0].frames.alloc(dframe * det->cfg.max_batch + 64))) return rc;
+    if ((rc = enqueue_color_to_gray(det, frames_dev, n_frames, channels, frame_stride, row_stride, det->slot[0].frames.p, s))) return rc;
+    if ((rc = clfd_detector_enqueue(det, det->slot[0].frames.p, n_frames, dframe, (int)dstride, cuda_stream))) return rc;
     det->stats.kernel_launches += 1;
     det->color_events = det->profiling;
     return 0;
@@ -1309,7 +1315,6 @@ static int take_counters(clfd_detector *det, const unsigned long long *hc, int n
     const unsigned long long total = hc[kCnt * (nc - 1)];   // all cascades append to one rect buffer
     unsigned long long deep = 0, rect_over = 0, queue_over = 0;
     for (int ci = 0; ci < nc; ci++) {
-        memcpy(det->cas[ci]->h_counters, hc + kCnt * ci, kCnt * sizeof(unsigned long long));
         deep += hc[kCnt * ci + 1];
         rect_over += hc[kCnt * ci + 2];
         queue_over += hc[kCnt * ci + 3];
@@ -1356,21 +1361,21 @@ int clfd_detector_fetch(clfd_detector *det, clfd_rect *rects, int64_t cap, int64
     clfd_context *ctx = det->ctx;
     CK(cudaSetDevice(ctx->device));
     cudaStream_t s = cuda_stream ? (cudaStream_t)cuda_stream : ctx->stream;
-    const int nc = (int)det->cas.size();
-    for (int ci = 0; ci < nc; ci++)
-        CK(cudaMemcpyAsync(det->h_counters + kCnt * ci, det->cas[ci]->d_counters.p, kCnt * sizeof(unsigned long long),
+    BatchSlot &sl = det->slot[0];   // the slot of clfd_detector_enqueue
+    for (size_t ci = 0; ci < det->cas.size(); ci++)
+        CK(cudaMemcpyAsync(sl.h_counters + kCnt * ci, det->cas[ci]->d_counters.p, kCnt * sizeof(unsigned long long),
                            cudaMemcpyDeviceToHost, s));
     CK(cudaStreamSynchronize(s));
-    int rc = take_counters(det, det->h_counters, det->last_frames, n_rects);
+    int rc = take_counters(det, sl.h_counters, det->last_frames, n_rects);
     if (rc) return rc;
     const unsigned long long total = (unsigned long long)*n_rects;
     if (det->have_events) read_kernel_ms(det);
     if (total == 0 || !rects) return 0;
     if ((int64_t)total > cap) { set_error("rect buffer too small: need %llu, have %lld", total, (long long)cap); return CLFD_ERR_CAPACITY; }
-    CK(cudaMemcpyAsync(det->h_rects, det->rects.p, total * sizeof(DevRect), cudaMemcpyDeviceToHost, s));
+    CK(cudaMemcpyAsync(sl.h_rects, sl.rects.p, total * sizeof(DevRect), cudaMemcpyDeviceToHost, s));
     CK(cudaStreamSynchronize(s));
     static_assert(sizeof(DevRect) == sizeof(clfd_rect), "rect layout");
-    memcpy(rects, det->h_rects, total * sizeof(DevRect));
+    memcpy(rects, sl.h_rects, total * sizeof(DevRect));
     return 0;
 }
 
@@ -1393,19 +1398,17 @@ static int submit_batch(clfd_detector *det, const uint8_t *frames_host, int n_fr
     if (row_stride < W) INVALID("row stride %d smaller than the frame width %d", row_stride, W);
     if (det->n_submitted - det->n_collected >= kSlots) INVALID("%d batches already in flight: collect one first", kSlots);
     const int slot = (int)(det->n_submitted % kSlots);
+    BatchSlot &sl = det->slot[slot];
     const size_t dstride = round_up(W, 16), dframe = dstride * H;
     int rc;
-    if (!det->dev_frames[slot].p && (rc = det->dev_frames[slot].alloc(dframe * det->cfg.max_batch + 64))) return rc;
+    if (!sl.frames.p && (rc = sl.frames.alloc(dframe * det->cfg.max_batch + 64))) return rc;
     // colour staging: rows of W * channels bytes at a 16-byte pitch.  The slot's last batch has been collected, so the
     // buffer may grow here
     const size_t cstride = round_up((size_t)W * channels, 16), cframe = cstride * H;
-    if (channels != 1 && det->dev_color[slot].n < cframe * det->cfg.max_batch &&
-        (rc = det->dev_color[slot].alloc(cframe * det->cfg.max_batch)))
+    if (channels != 1 && sl.color.n < cframe * det->cfg.max_batch && (rc = sl.color.alloc(cframe * det->cfg.max_batch)))
         return rc;
-    if (slot == 1) {
-        if (!det->rects2.p && (rc = det->rects2.alloc(det->rect_cap))) return rc;
-        if (!det->h_rects1) CK(cudaMallocHost((void **)&det->h_rects1, (size_t)kEagerRects * sizeof(DevRect)));
-    }
+    if (!sl.rects.p && (rc = sl.rects.alloc(det->rect_cap))) return rc;   // slot 1 (slot 0's come with the detector)
+    if (!sl.h_rects) CK(cudaMallocHost((void **)&sl.h_rects, (size_t)kEagerRects * sizeof(DevRect)));
     int n_chunks = 1;
     if (n_frames >= 8) n_chunks = n_frames >= 32 ? 4 : 2;
     // with a batch already in flight the whole copy overlaps THAT batch's compute: no need to
@@ -1419,13 +1422,12 @@ static int submit_batch(clfd_detector *det, const uint8_t *frames_host, int n_fr
     if (!det->copy_stream) CK(cudaStreamCreateWithFlags(&det->copy_stream, cudaStreamNonBlocking));
     for (int k = 0; k < n_chunks; k++)
         if (!det->copied[k]) CK(cudaEventCreateWithFlags(&det->copied[k], cudaEventDisableTiming));
-    for (auto &e : det->done)
-        if (!e) CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+    for (auto &b : det->slot) if (!b.done) CK(cudaEventCreateWithFlags(&b.done, cudaEventDisableTiming));
     // The slot's staging buffer was last read by the batch submitted kSlots submits ago, which has
     // been collected (its done event was synchronised), so the copy may start right away -- while
     // the previous batch still computes.
     det->last_frames = n_frames;
-    det->slot_frames[slot] = n_frames;
+    sl.n_frames = n_frames;
     int launches = 0;
     cudaStream_t cs = det->copy_stream;
     // nf frames of `wbytes` bytes per row from the host to d (pitch dpitch, frames dfr apart); nothing behind the last
@@ -1446,12 +1448,12 @@ static int submit_batch(clfd_detector *det, const uint8_t *frames_host, int n_fr
         const int f0 = (int)((long long)n_frames * k / n_chunks), f1 = (int)((long long)n_frames * (k + 1) / n_chunks);
         const int nf = f1 - f0;
         if (nf <= 0) continue;
-        uint8_t *dst = det->dev_frames[slot].p + (size_t)f0 * dframe;
+        uint8_t *dst = sl.frames.p + (size_t)f0 * dframe;
         const uint8_t *src = frames_host + (size_t)f0 * frame_stride;
         if (channels == 1) {
             if ((rc = h2d(dst, dstride, dframe, src, W, nf))) return rc;
         } else {
-            uint8_t *stage = det->dev_color[slot].p + (size_t)f0 * cframe;
+            uint8_t *stage = sl.color.p + (size_t)f0 * cframe;
             if ((rc = h2d(stage, cstride, cframe, src, (size_t)W * channels, nf))) return rc;
             if ((rc = enqueue_color_to_gray(det, stage, nf, channels, cframe, (int)cstride, dst, cs))) return rc;
             launches++;
@@ -1463,21 +1465,19 @@ static int submit_batch(clfd_detector *det, const uint8_t *frames_host, int n_fr
         if (rc) return rc;
     }
     if (overlap) {   // pyramid of chunk k+1 beside the tile kernel of chunk k, each pyramid behind its chunk's copy
-        rc = enqueue_overlapped(det, det->dev_frames[slot].p, n_frames, dframe, (int)dstride, ctx->stream, n_chunks, det->copied,
+        rc = enqueue_overlapped(det, sl.frames.p, n_frames, dframe, (int)dstride, ctx->stream, n_chunks, det->copied,
                                 &launches, slot);
         if (rc) return rc;
     }
     det->stats.kernel_launches = launches;
     // results: counters of every cascade + the first rects, behind the kernels
     const int nc = (int)det->cas.size();
-    unsigned long long *hc = det->h_counters + (size_t)slot * kCnt * 16;
     for (int ci = 0; ci < nc; ci++)
-        CK(cudaMemcpyAsync(hc + kCnt * ci, det->cas[ci]->d_counters.p + kCnt * slot, kCnt * sizeof(unsigned long long),
+        CK(cudaMemcpyAsync(sl.h_counters + kCnt * ci, det->cas[ci]->d_counters.p + kCnt * slot, kCnt * sizeof(unsigned long long),
                            cudaMemcpyDeviceToHost, ctx->stream));
     const size_t eager = (size_t)std::min<unsigned long long>(det->rect_cap, kEagerRects);
-    CK(cudaMemcpyAsync(slot ? det->h_rects1 : det->h_rects, slot ? det->rects2.p : det->rects.p, eager * sizeof(DevRect),
-                       cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaEventRecord(det->done[slot], ctx->stream));
+    CK(cudaMemcpyAsync(sl.h_rects, sl.rects.p, eager * sizeof(DevRect), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaEventRecord(sl.done, ctx->stream));
     det->color_events = channels != 1 && det->profiling;
     det->n_submitted++;
     return 0;
@@ -1503,21 +1503,20 @@ int clfd_detect_collect(clfd_detector *det, clfd_rect *rects, int64_t cap, int64
     if (det->n_collected >= det->n_submitted) INVALID("no batch in flight");
     clfd_context *ctx = det->ctx;
     CK(cudaSetDevice(ctx->device));
-    const int slot = (int)(det->n_collected % kSlots);
+    BatchSlot &sl = det->slot[det->n_collected % kSlots];
     det->n_collected++;
-    CK(cudaEventSynchronize(det->done[slot]));
+    CK(cudaEventSynchronize(sl.done));
     if (det->have_events && det->n_collected == det->n_submitted) read_kernel_ms(det);   // the events are this batch's
-    int rc = take_counters(det, det->h_counters + (size_t)slot * kCnt * 16, det->slot_frames[slot], n_rects);
+    int rc = take_counters(det, sl.h_counters, sl.n_frames, n_rects);
     if (rc) return rc;
     const unsigned long long total = (unsigned long long)*n_rects;
     if (total == 0 || !rects) return 0;
     if ((int64_t)total > cap) { set_error("rect buffer too small: need %llu, have %lld", total, (long long)cap); return CLFD_ERR_CAPACITY; }
     static_assert(sizeof(DevRect) == sizeof(clfd_rect), "rect layout");
     const unsigned long long eager = std::min<unsigned long long>(total, kEagerRects);
-    memcpy(rects, slot ? det->h_rects1 : det->h_rects, eager * sizeof(DevRect));
+    memcpy(rects, sl.h_rects, eager * sizeof(DevRect));
     if (total > eager)   // rare: the slot's device buffer is untouched until the slot is submitted again
-        CK(cudaMemcpy(rects + eager, (slot ? det->rects2.p : det->rects.p) + eager, (total - eager) * sizeof(DevRect),
-                      cudaMemcpyDeviceToHost));
+        CK(cudaMemcpy(rects + eager, sl.rects.p + eager, (total - eager) * sizeof(DevRect), cudaMemcpyDeviceToHost));
     return 0;
 }
 
@@ -1606,7 +1605,7 @@ int clfd_detector_read_level(clfd_detector *det, int cascade, int level, int fra
                              uint64_t *sqsum, int32_t *tilted) {
     if (!det || cascade < 0 || cascade >= (int)det->cas.size()) INVALID("bad argument");
     CascadePlan &cp = *det->cas[cascade];
-    // pub_levels: the scale-cascade planner fills no CasLevel list; every one of its scales reads pyramid level 0
+    // pub_levels: the scale-cascade planner lists only its tile-kernel scales in `levels`; every scale reads pyramid level 0
     if (level < 0 || level >= (int)cp.pub_levels.size()) INVALID("level %d outside 0..%zu", level, cp.pub_levels.size());
     if (frame < 0 || frame >= det->last_frames) INVALID("frame %d outside the last batch", frame);
     if (tilted && !det->pyr.want_tilted) INVALID("detector has no tilted integral (no cascade with tilted features)");

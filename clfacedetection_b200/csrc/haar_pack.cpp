@@ -421,7 +421,6 @@ static void pack_dense_one(const HostCascade &c, int ystep, DenseParams &P, std:
     // six-offset form E0,E1,F0,F1,G0,G1 with rect0 = (E0-E1)+(F0-F1), rect1 = (E0-E1)+(G0-G1): six
     // corner loads instead of eight.  With p0,p3 entering a rect sum with + and p1,p2 with -, the
     // common pair can only be (p0,p2), (p3,p1), (p0,p1) or (p3,p2).
-    const bool share_corners = !getenv("CLFD_NO_SHARED_CORNERS");   // test hook
     int ns = 0, nstump = 0;
     while (ns < elig && nstump + c.st_ntrees[ns] * P.npt <= kMaxDenseStumps) {
         P.stage[ns].first = (uint16_t)nstump;
@@ -429,7 +428,7 @@ static void pack_dense_one(const HostCascade &c, int ystep, DenseParams &P, std:
         for (int t = c.st_first_tree[ns] * P.npt; t < c.st_first_tree[ns + 1] * P.npt; t++) {
             DenseStump st = tail[t];
             bool shared = false;
-            if (share_corners && P.npt == 1 && c.hid_nrects[c.tr_first_node[t]] == 2) {   // (multi-node trees keep their order)
+            if (P.npt == 1 && c.hid_nrects[c.tr_first_node[t]] == 2) {   // (multi-node trees keep their order)
                 const uint32_t *A = st.off, *B = st.off + 4;
                 static const int pairs[4][2] = {{0, 2}, {3, 1}, {0, 1}, {3, 2}};   // (plus, minus) corner
                 for (const auto &pr : pairs) {
@@ -478,7 +477,6 @@ static void pack_dense_one(const HostCascade &c, int ystep, DenseParams &P, std:
     P.track_abs = 0;
     for (float v : c.alpha)
         if (std::fabs(v) > 64.f) P.track_abs = 1;
-    if (getenv("CLFD_NO_TRACK_ABS")) P.track_abs = 0;   // A/B hook
     // stages run in fixed geometry before the first compaction (tunable for experiments)
     int nf = 3;
     if (const char *e = getenv("CLFD_N_FIXED")) nf = atoi(e);
