@@ -303,9 +303,9 @@ struct CascadePlan {
     DevBuf<int16_t> d_codes;
     DevBuf<unsigned long long> d_counters;
     DevBuf<unsigned long long> d_count_b;   // second-queue counter, one per slot
-    int mid_begin = 0, mid_end = 0;         // stages of the thread-per-window mid kernel (equal: none)
-    std::vector<int> pass_cuts;   // stage bounds of the survivor passes: mid kernel (mid_begin..mid_end) or k_sc_eval
-    int sc_deep_from = 0;                   // first stage of the k_sc_deep pass (n_stages: none)
+    int mid_begin = 0, mid_end = 0;         // image-pyramid mode: stages of the k_generic_pass passes (equal: none)
+    std::vector<int> pass_cuts;   // stage bounds of the k_generic_pass passes
+    int sc_deep_from = 0;                   // scale-cascade mode: first stage of the k_generic_deep pass (n_stages: none)
 };
 
 constexpr int kMaxChunks = 8;
@@ -369,26 +369,26 @@ struct clfd_detector {
     }
 };
 
-// A survivor queue and its item counter; items == nullptr stands for every window of the grid.
-struct SurvivorQueue { QueueItem *items = nullptr; unsigned long long *count = nullptr; };
-
-// launch(stage_begin, stage_end, in, out) for each pass of cp.pass_cuts, ping-ponging between det->queue (counter
-// counters[1], the first pass's input if from_queue, else the grid) and det->queue_b (counter d_count_b[slot]).  A counter
-// is cleared before a pass writes its queue unless this range has not written that queue yet.  *next: the last output.
-template <class Launch>
-static int run_pass_chain(const clfd_detector *det, const CascadePlan &cp, int slot, bool from_queue, cudaStream_t s,
-                          int *launches, SurvivorQueue *next, Launch launch) {
-    const SurvivorQueue q[2] = {{det->queue.p, cp.d_counters.p + kCnt * slot + 1}, {det->queue_b.p, cp.d_count_b.p + slot}};
+// k_generic_pass for each pass of cp.pass_cuts, ping-ponging between det->queue (counter counters[1], the first pass's
+// input if from_queue, else the grid) and det->queue_b (counter d_count_b[slot]).  A counter is cleared before a pass
+// writes its queue unless this range has not written that queue yet.  *p: the input of the pass after the chain.
+template <class Args>
+static int run_pass_chain(const clfd_detector *det, const CascadePlan &cp, const Args &a, int slot, bool from_queue,
+                          cudaStream_t s, int *launches, PassArgs *p) {
+    QueueItem *const items[2] = {det->queue.p, det->queue_b.p};
+    unsigned long long *const count[2] = {cp.d_counters.p + kCnt * slot + 1, cp.d_count_b.p + slot};
     bool written[2] = {from_queue, false};
-    SurvivorQueue in = from_queue ? q[0] : SurvivorQueue();
+    memset(p, 0, sizeof *p);
+    if (from_queue) { p->in = items[0]; p->in_count = count[0]; }
     for (size_t k = 0, out = from_queue; k + 1 < cp.pass_cuts.size(); k++, out ^= 1) {
-        if (written[out]) CK(cudaMemsetAsync(q[out].count, 0, sizeof(unsigned long long), s));   // holds an older pass
-        if (int rc = launch(cp.pass_cuts[k], cp.pass_cuts[k + 1], in, q[out])) return rc;
+        if (written[out]) CK(cudaMemsetAsync(count[out], 0, sizeof(unsigned long long), s));   // holds an older pass
+        p->stage_begin = cp.pass_cuts[k]; p->stage_end = cp.pass_cuts[k + 1];
+        p->out = items[out]; p->out_count = count[out];
+        CK(launch_generic_pass(a, *p, det->ctx->n_sms, s));
         (*launches)++;
         written[out] = true;
-        in = q[out];
+        p->in = items[out]; p->in_count = count[out];
     }
-    *next = in;
     return 0;
 }
 
@@ -781,7 +781,7 @@ static int plan_tiles(CasLevel &CL, int tile_h, int tile_base) {
     return CL.tiles_x * CL.tiles_y;
 }
 
-// Scale-cascade mode, one cascade: its scales over the frame itself (tempcv.cpp:1344-1380) with their k_sc_eval node
+// Scale-cascade mode, one cascade: its scales over the frame itself (tempcv.cpp:1344-1380) with their ScNode
 // tables, the tile-kernel route of the leading scales of window step 2, and the schedule of the survivor passes.
 static int plan_sc_cascade(CascadePlan &cp, const clfd_detector_config &cfg, cudaStream_t s) {
     const HostCascade &hc = cp.cascade->host;
@@ -839,9 +839,9 @@ static int plan_sc_cascade(CascadePlan &cp, const clfd_detector_config &cfg, cud
         cp.sc_tile_windows = L.win_base + (long long)L.nx * L.ny;
     }
     cp.bytes_cascade += (int64_t)(W + 1) * (H + 1) * (4 + 8 + (hc.has_tilted ? 4 : 0)) + nodes.size() * sizeof(ScNode);
-    // k_sc_eval passes over growing stage ranges (cumulative trees >= 10, 40, 90, 160, ... per pass), survivors
+    // k_generic_pass passes over growing stage ranges (cumulative trees >= 10, 40, 90, 160, ... per pass), survivors
     // re-compacted through the two queues in between; a stage tree runs as one pass.  From the first stage after stage 0
-    // that has >= 50 trees on, the survivors are finished one warp per position (k_sc_deep).
+    // that has >= 50 trees on, the survivors are finished one warp per position (k_generic_deep).
     static const int limit[7] = {10, 40, 90, 160, 300, 500, 800};
     cp.pass_cuts.assign(1, 0);
     cp.sc_deep_from = hc.n_stages();
@@ -854,37 +854,30 @@ static int plan_sc_cascade(CascadePlan &cp, const clfd_detector_config &cfg, cud
     return 0;
 }
 
-// Scale-cascade mode, one cascade: the tile kernel over the step-2 scales (exit codes only), the k_sc_eval passes,
-// k_sc_deep and k_sc_rows.  ev (cascade 0, profiling): ev[5] before the first kernel, ev[6] and ev[7] after the last.
+// Scale-cascade mode, one cascade: the tile kernel over the step-2 scales (exit codes only), the k_generic_pass
+// passes, k_generic_deep and k_sc_rows.  ev (cascade 0, profiling): ev[5] before the first kernel, ev[6] and ev[7] after the last.
 static int enqueue_sc_cascade(clfd_detector *det, const CascadePlan &cp, CascadeArgs &a, int slot, cudaStream_t s,
                               cudaEvent_t *ev, int *launches) {
-    const int n_sms = det->ctx->n_sms, n_stages = cp.cascade->host.n_stages();
+    const int n_stages = cp.cascade->host.n_stages();
     ScArgs sa;
     memset(&sa, 0, sizeof sa);
+    static_cast<CascadeArgs &>(sa) = a;
     const PyrLevel &L0 = det->pyr.levels[0];
     sa.sum = a.sum + L0.sum_off; sa.sq = a.sq + L0.sum_off; sa.tilted = a.tilted ? a.tilted + L0.sum_off : nullptr;
-    sa.sum_frame_stride = a.sum_frame_stride;
-    sa.pitch = L0.sum_pitch; sa.W = det->cfg.width; sa.H = det->cfg.height;
-    sa.levels = cp.d_sc_levels.p; sa.nodes = cp.d_sc_nodes.p;
-    sa.n_levels = (int)cp.sc_levels.size(); sa.rows_per_frame = cp.sc_rows; sa.n_frames = a.n_frames;
-    sa.cascade_index = a.cascade_index; sa.frame_base = a.frame_base; sa.windows_per_frame = cp.windows_per_frame;
     sa.codes = cp.d_codes.p + (size_t)a.frame_base * cp.windows_per_frame;
-    sa.rects = a.rects; sa.rect_cap = a.rect_cap; sa.counters = a.counters; sa.deep = a.deep; sa.queue_cap = det->queue_cap;
+    sa.pitch = L0.sum_pitch; sa.W = det->cfg.width; sa.H = det->cfg.height;
+    sa.scales = cp.d_sc_levels.p; sa.nodes = cp.d_sc_nodes.p;
+    sa.n_scales = (int)cp.sc_levels.size(); sa.rows_per_frame = cp.sc_rows;
+    sa.first_window = cp.sc_tile_windows;
     if (ev) CK(cudaEventRecord(ev[5], s));
     CascadeArgs ta = a;   // the tile kernel, one launch per scale of window step 2
     ta.codes = sa.codes; ta.rects = nullptr; ta.rect_cap = 0;
     for (auto &t : cp.sc_tiles) { CK(launch_cascade_tiles(t->P, ta, t->tile_base, t->n_tiles, s)); (*launches)++; }
-    sa.first_window = cp.sc_tile_windows;
-    auto eval_pass = [&](int b, int e, SurvivorQueue in, SurvivorQueue out) -> int {
-        sa.stage_begin = b; sa.stage_end = e; sa.in = in.items; sa.in_count = in.count; sa.out = out.items; sa.out_count = out.count;
-        CK(launch_sc_eval(sa, n_sms, s));
-        return 0;
-    };
-    SurvivorQueue next;
-    if (int rc = run_pass_chain(det, cp, slot, false, s, launches, &next, eval_pass)) return rc;
+    PassArgs p;
+    if (int rc = run_pass_chain(det, cp, sa, slot, false, s, launches, &p)) return rc;
     if (cp.sc_deep_from < n_stages) {
-        sa.stage_begin = cp.sc_deep_from; sa.stage_end = n_stages; sa.in = next.items; sa.in_count = next.count;
-        CK(launch_sc_deep(sa, n_sms, s)); (*launches)++;
+        p.stage_begin = cp.sc_deep_from; p.stage_end = n_stages;
+        CK(launch_generic_deep(sa, p, det->ctx->n_sms, s)); (*launches)++;
     }
     CK(launch_sc_rows(sa, s)); (*launches)++;
     if (ev) { CK(cudaEventRecord(ev[6], s)); CK(cudaEventRecord(ev[7], s)); }
@@ -942,7 +935,7 @@ static int plan_pyramid_levels(clfd_detector *det, std::vector<std::pair<int, in
     return 0;
 }
 
-// Image-pyramid mode, mid kernel: the stages right after the tile prefix of a LINEAR cascade whose trees the tile
+// Image-pyramid mode, k_generic_pass: the stages right after the tile prefix of a LINEAR cascade whose trees the tile
 // kernel cannot take, while they are too small for a warp per window (< 24 trees), at most 8.  Passes: the first ends
 // once it holds >= 10 trees, the later ones >= 30 (lanes are re-compacted between passes).
 static void plan_mid_passes(CascadePlan &cp) {
@@ -958,12 +951,11 @@ static void plan_mid_passes(CascadePlan &cp) {
     }
 }
 
-// Image-pyramid mode, one cascade: the tile kernel (or k_enqueue_all), the mid passes and the deep kernel.  ev (cascade
+// Image-pyramid mode, one cascade: the tile kernel, the k_generic_pass passes and k_generic_deep.  ev (cascade
 // 0, profiling): ev[5] before the first kernel, ev[6] after the tile kernel, ev[7] after the last.
 static int enqueue_pyramid_cascade(clfd_detector *det, const CascadePlan &cp, CascadeArgs &a, int slot, cudaStream_t s,
                                    cudaEvent_t *ev, int *launches) {
     const DenseParams &P0 = cp.cascade->packed.dense[0];
-    const bool has_mid = cp.mid_end > cp.mid_begin;
     if (ev) CK(cudaEventRecord(ev[5], s));
     if (P0.tail_stages > 0) {
         // ystep-2 levels (de-interleaved tile layout) and ystep-1 levels (natural layout)
@@ -972,25 +964,18 @@ static int enqueue_pyramid_cascade(clfd_detector *det, const CascadePlan &cp, Ca
             CK(launch_cascade_tiles(cp.dense[0], a, cp.n_tiles_y2, cp.n_tiles - cp.n_tiles_y2, s));
             (*launches)++;
         }
-    } else if (!has_mid) {   // (with mid passes, the first one walks the window grid itself)
-        CK(launch_enqueue_all(a, s)); (*launches)++;
     }
     if (ev) CK(cudaEventRecord(ev[6], s));
     // cascades the tile kernel finishes itself (tail_stages == total_stages) never fill the queue
     const bool tiles_finish = P0.tail_stages > 0 && P0.exec_stages == P0.total_stages;
     if (!tiles_finish) {
-        if (has_mid) {
-            auto mid_pass = [&](int b, int e, SurvivorQueue in, SurvivorQueue out) -> int {
-                a.deep.mid_begin = b; a.deep.mid_end = e;
-                a.mid_in = in.items; a.mid_in_count = in.count; a.mid_out = out.items; a.mid_out_count = out.count;
-                CK(launch_cascade_mid(a, det->ctx->n_sms, s));
-                return 0;
-            };
-            SurvivorQueue next;
-            if (int rc = run_pass_chain(det, cp, slot, P0.tail_stages > 0, s, launches, &next, mid_pass)) return rc;
-            a.deep_in = next.items; a.deep_count = next.count;
+        // without a tile prefix, the first pass (or the deep kernel) walks the window grid itself
+        PassArgs p;
+        if (int rc = run_pass_chain(det, cp, a, slot, P0.tail_stages > 0, s, launches, &p)) return rc;
+        if (cp.mid_end < P0.total_stages) {
+            p.stage_begin = cp.mid_end; p.stage_end = P0.total_stages;   // (queue items carry their first stage)
+            CK(launch_generic_deep(a, p, det->ctx->n_sms, s)); (*launches)++;
         }
-        if (cp.mid_end < P0.total_stages) { CK(launch_cascade_deep(a, det->ctx->n_sms, s)); (*launches)++; }
     }
     if (ev) CK(cudaEventRecord(ev[7], s));
     return 0;
@@ -1140,7 +1125,6 @@ static CascadeArgs cascade_args(const clfd_detector *det, const CascadePlan &cp,
     a.deep.n_stages = hc.n_stages(); a.deep.is_tree = hc.is_tree; a.deep.has_tilted = hc.has_tilted;
     a.deep.win_w = hc.win_w; a.deep.win_h = hc.win_h;
     a.deep.inv_area = cp.cascade->packed.dense[0].inv_area;
-    a.deep.mid_begin = cp.mid_begin; a.deep.mid_end = cp.mid_end;
     return a;
 }
 
@@ -1175,7 +1159,6 @@ static int enqueue_range(clfd_detector *det, const uint8_t *frames_dev, int fram
                 a.queue = det->queue.p; a.queue_cap = det->queue_cap;
                 a.rects = det->slot[slot].rects.p; a.rect_cap = det->rect_cap;
                 a.counters = cp.d_counters.p + kCnt * slot;
-                a.deep_in = a.queue; a.deep_count = a.counters + 1;
                 int rc = det->enqueue_cascade(det, cp, a, slot, s, ci == 0 ? ev : nullptr, &launches);
                 if (rc) return rc;
             }

@@ -158,7 +158,6 @@ struct DeepCascadeDev {
     const DeepNode *nodes;
     const float *alpha;
     int n_stages, is_tree, has_tilted, win_w, win_h;
-    int mid_begin, mid_end;      // stages the thread-per-window mid kernel evaluates (equal: none)
     double inv_area;
 };
 
@@ -215,9 +214,9 @@ struct ScLevel {          // one scale
 constexpr int kScCodeSkipped = -32768;   // grid position the skip rule never evaluates (tempcv.cpp:1161)
 constexpr int kScCodeOutside = -32767;   // window rejected by the bounds check (tempcv.cpp:817-820, result -1)
 
-struct QueueItem {        // survivor handed to the deep kernel
-    uint32_t key;           // frame << 16 | cas_level << 8 | next_stage
-    uint32_t xy;            // y << 16 | x   (window origin, pixels of the level)
+struct QueueItem {        // survivor handed to the generic kernels
+    uint32_t key;           // frame << 16 | cas_level << 8 | next_stage   (scale-cascade mode: frame)
+    uint32_t xy;            // y << 16 | x   (window origin, pixels of the level; scale-cascade mode: window index)
 };
 
 struct DevRect {

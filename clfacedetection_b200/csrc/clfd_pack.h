@@ -20,7 +20,7 @@ void pack_cascade(const HostCascade &c, PackedCascade &out);
 // mode: fills L.inv_area / L.eq_off and n_nodes() ScNodes at `out` (pitch = elements per integral row)
 void pack_sc_level(const HostCascade &c, double factor, int pitch, ScLevel &L, ScNode *out);
 // scale-cascade mode, scales with window step 2: this scale as a ystep-2 blob of the tile kernel; false if
-// the tile kernel cannot finish the cascade at this scale (the detector then keeps k_sc_eval for it)
+// the tile kernel cannot finish the cascade at this scale (the detector then keeps the generic kernels for it)
 bool pack_sc_dense(const HostCascade &c, double scale, DenseParams &P, std::vector<TailStump> &tail,
                    std::vector<DenseStage> &stage_tab);
 const char *get_error();

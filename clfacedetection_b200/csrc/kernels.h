@@ -91,11 +91,8 @@ struct CascadeArgs {
     int count_exact;                // tile kernel: the instantiation that counts FP64 fallbacks / near-threshold sums (counters[4], [5])
     long long windows_per_frame;
     int16_t *codes;                 // device, [n_frames][windows_per_frame] or NULL
-    QueueItem *queue; unsigned long long queue_cap;   // written by the tile kernel / k_enqueue_all, counted in counters[1]
-    // mid kernel pass: input queue (NULL = every grid window) -> output queue
-    const QueueItem *mid_in; const unsigned long long *mid_in_count;
-    QueueItem *mid_out; unsigned long long *mid_out_count;
-    const QueueItem *deep_in; const unsigned long long *deep_count;   // what the deep kernel reads
+    QueueItem *queue; unsigned long long queue_cap;   // written by the tile kernel, counted in counters[1]; capacity of
+                                                      // every survivor queue
     DevRect *rects; unsigned long long rect_cap;
     unsigned long long *counters;   // [0] rects  [1] queue items  [2] rect overflow [3] queue overflow
     DeepCascadeDev deep;
@@ -103,42 +100,36 @@ struct CascadeArgs {
 // dense tile kernel (+ hand-off of survivors to the queue)
 // tiles [tile0, tile0 + n_tiles) must all belong to levels with ystep == P.ystep
 cudaError_t launch_cascade_tiles(const DenseParams &P, const CascadeArgs &a, int tile0, int n_tiles, cudaStream_t stream);
-// fill the queue with every window (cascades without a dense prefix)
-cudaError_t launch_enqueue_all(const CascadeArgs &a, cudaStream_t stream);
-// thread-per-window evaluation of stages [deep.mid_begin, deep.mid_end) (generic trees), survivors -> queue_b
-cudaError_t launch_cascade_mid(const CascadeArgs &a, int n_sms, cudaStream_t stream);
-// warp-per-window evaluation of the queue
-cudaError_t launch_cascade_deep(const CascadeArgs &a, int n_sms, cudaStream_t stream);
 // reject-level output: scans the exit codes of n_frames frames, appends the candidates of
 // tempcv.cpp:1084-1094 (count at counter[0]) with the exact stage sum of their last stage
 cudaError_t launch_roc_collect(const CascadeArgs &a, RocItem *out, unsigned long long cap, unsigned long long *counter, cudaStream_t stream);
 
-// ---- scale-cascade mode (kernels_sc.cu) -----------------------------------------------
-struct ScArgs {
-    const int32_t *sum; const unsigned long long *sq; const int32_t *tilted;   // full-frame integrals (level 0)
-    size_t sum_frame_stride;
+// ---- scale-cascade mode -------------------------------------------------------------
+// The CascadeArgs part holds the full-frame integrals (level 0, pre-offset to it), the exit codes (always present in
+// this mode), rects, counters and the cascade; `levels`, `cas_levels` and `queue` are not read.
+struct ScArgs : CascadeArgs {
     int pitch, W, H;                // elements per integral row, frame size
-    const ScLevel *levels;          // device
-    const ScNode *nodes;            // device, n_levels x n_nodes
-    int n_levels, rows_per_frame, n_frames, cascade_index, frame_base;
-    long long windows_per_frame;
+    const ScLevel *scales;          // device
+    const ScNode *nodes;            // device, n_scales x n_nodes
+    int n_scales, rows_per_frame;
     long long first_window;         // grid positions below this one are evaluated by the tile kernel (step-2 scales)
-    int16_t *codes;                 // device, [n_frames][windows_per_frame] (always present in this mode)
-    DevRect *rects; unsigned long long rect_cap;
-    unsigned long long *counters;   // [0] rects [2] rect overflow [3] queue overflow
-    DeepCascadeDev deep;            // stages / tree_first_node / alpha (scale independent)
-    // one evaluation pass: stages [stage_begin, stage_end) of the positions in `in` (NULL = every grid
-    // position); survivors of a non-final pass go to `out`
+};
+// the invoker's skip rule + rect emission over the finished exit codes (k_sc_rows, kernels_sc.cu)
+cudaError_t launch_sc_rows(const ScArgs &a, cudaStream_t stream);
+
+// ---- generic kernels of both modes (kernels_clod.cu) --------------------------------
+// One survivor pass: stages [stage_begin, stage_end) of the windows in `in` (NULL: every window of the grid); the
+// survivors of a pass that does not end the cascade go to `out`.
+struct PassArgs {
     int stage_begin, stage_end;
     const QueueItem *in; const unsigned long long *in_count;
     QueueItem *out; unsigned long long *out_count;
-    unsigned long long queue_cap;
 };
-// one evaluation pass over the grid / a survivor queue (k_sc_eval)
-cudaError_t launch_sc_eval(const ScArgs &a, int n_sms, cudaStream_t stream);
-// final pass, warp per survivor: stages [stage_begin, n_stages) of a linear cascade (k_sc_deep)
-cudaError_t launch_sc_deep(const ScArgs &a, int n_sms, cudaStream_t stream);
-// the invoker's skip rule + rect emission over the finished exit codes (k_sc_rows)
-cudaError_t launch_sc_rows(const ScArgs &a, cudaStream_t stream);
+// Args: CascadeArgs (image-pyramid mode) or ScArgs (scale-cascade mode).
+// thread per window over one stage range, or the whole walk of a stage tree (k_generic_pass)
+template <class Args> cudaError_t launch_generic_pass(const Args &a, const PassArgs &p, int n_sms, cudaStream_t stream);
+// warp per window from p.stage_begin to the end of the cascade (k_generic_deep); with p.in == NULL it sets counters[1]
+// to the number of grid windows
+template <class Args> cudaError_t launch_generic_deep(const Args &a, const PassArgs &p, int n_sms, cudaStream_t stream);
 
 }  // namespace clfd

@@ -18,11 +18,12 @@
 //       up to four nodes (NODES: per-window "node I am at" state over padded node records),
 //       the alt_tree stage tree (TREE: stages in depth-first order, per-window target position).
 //       The scale-cascade mode runs its step-2 scales through it as well (clfd_api.cu).
-//   k_cascade_mid / k_cascade_deep : generic fallback for cascades the tile kernel cannot finish
-//       (larger trees, a tile that does not fit shared memory): the survivors of the tile prefix
-//       (or every window) are pooled in one global queue and evaluated one thread / one WARP per
-//       window, lanes striding over the trees of a stage.  The stage sum is reduced with shuffles
-//       when the packer proved the alpha sum exact in any order, otherwise accumulated in tree order.
+//   k_generic_pass / k_generic_deep : generic fallback for cascades the tile kernel cannot finish
+//       (larger trees, a tile that does not fit shared memory), shared with the scale-cascade mode:
+//       the survivors of the tile prefix (or every window) are pooled in one global queue and
+//       evaluated one thread / one WARP per window, lanes striding over the trees of a stage.  The
+//       stage sum is reduced with shuffles when the packer proved the alpha sum exact in any order,
+//       otherwise accumulated in tree order.
 //   k_roc_collect : reject-level output (tempcv.cpp:1084-1094) as a pass over the exit codes.
 //
 // Arithmetic is bit-identical to the reference's C expressions: integer rect sums; FP64
@@ -134,7 +135,7 @@ __device__ __forceinline__ void emit_rect(const CascadeArgs &a, const CasLevel &
 // Hand-over: the survivors are counting-sorted by bank class and dealt to the eight warps.
 // Phase 2, warp-autonomous (all remaining stages the tile kernel knows; see the kernel body):
 //   stump-based upright cascades are finished here; the others hand the survivors of their
-//   eligible prefix to the queue of k_cascade_mid / k_cascade_deep.
+//   eligible prefix to the queue of k_generic_pass / k_generic_deep.
 // ------------------------------------------------------------------------------------
 // Tile accesses use 32-bit shared-window addresses and explicit ld.shared (a generic pointer
 // would make the compiler rebuild the shared window base inside every loop).
@@ -991,37 +992,27 @@ cudaError_t launch_cascade_tiles(const DenseParams &P, const CascadeArgs &a, int
 
 #ifndef CLFD_TILES_COUNT_TU
 // ------------------------------------------------------------------------------------
-// enqueue-all: cascades without a dense prefix start every window in the deep kernel
+// generic kernels: what the tile kernel does not finish (larger trees, tilted features, stage trees, a tile that does
+// not fit shared memory), in global memory, in both detection modes:
+//   k_generic_pass : one THREAD per window for a stage range of a linear cascade, or the whole walk of a stage tree.
+//       Early stages have few trees (3, 9, 14, ... in frontalface_alt2), so a warp per window would idle most lanes,
+//       and they still see most windows.  Input: every grid window or a survivor queue; the survivors go to the other
+//       queue.  Run in a few passes, ping-ponging between the two queues, so the lanes are re-compacted while the
+//       survivor count still drops fast.  Lanes hold consecutive windows, so the corner loads of a warp fall into a
+//       few cache lines.
+//   k_generic_deep : one WARP per window from a first stage to the end, lanes striding over the trees of a stage.  The
+//       stage sum is reduced with shuffles when the packer proved it exact in any order (DeepStage flags bit 1),
+//       otherwise the lanes' leaf values are added in tree order.
+// Both are templates over the window type of a mode (PyramidWindow, ScaleWindow), which
+//   kTreePass              : whether its planner runs a stage tree through k_generic_pass (its whole walk),
+//   from_grid / from_queue : turns a grid index or a queue item into a window (and its first stage),
+//   setup                  : computes the window's sigma (false: outside the frame, exit code written),
+//   node / rect            : reads the fields of a node record and the integer sum of its rect k,
+//   item                   : turns a survivor into a queue item,
+//   finish                 : writes what a finished window leaves behind (exit code, rect).
+// The arithmetic is the reference's, written once: FP64 sigma with separately rounded operations, float products
+// accumulated in double, or exact double products on the stump fast path (tempcv.cpp:872-898).
 // ------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(256) k_enqueue_all(const CascadeArgs a) {
-    const long long w = (long long)blockIdx.x * 256 + threadIdx.x;
-    const int frame = blockIdx.y;
-    if (w == 0 && frame == 0) a.counters[1] = (ull)a.windows_per_frame * a.n_frames;
-    if (w >= a.windows_per_frame) return;
-    int lo = 0, hi = a.n_cas_levels - 1;
-    while (lo < hi) {
-        const int mid = (lo + hi + 1) >> 1;
-        if (__ldg(&a.cas_levels[mid].win_base) <= w) lo = mid; else hi = mid - 1;
-    }
-    const int nx = __ldg(&a.cas_levels[lo].nx), ystep = __ldg(&a.cas_levels[lo].ystep);
-    const int local = (int)(w - __ldg(&a.cas_levels[lo].win_base));
-    const int iy = local / nx, ix = local - iy * nx;
-    QueueItem it;
-    it.key = ((uint32_t)frame << 16) | ((uint32_t)lo << 8);
-    it.xy = ((uint32_t)(iy * ystep) << 16) | (uint32_t)(ix * ystep);
-    a.queue[(size_t)frame * a.windows_per_frame + w] = it;
-}
-
-cudaError_t launch_enqueue_all(const CascadeArgs &a, cudaStream_t stream) {
-    if (a.windows_per_frame == 0 || a.n_frames == 0) return cudaSuccess;
-    k_enqueue_all<<<dim3((unsigned)((a.windows_per_frame + 255) / 256), a.n_frames), 256, 0, stream>>>(a);
-    return cudaGetLastError();
-}
-
-// ------------------------------------------------------------------------------------
-// deep kernel: one warp per queued window
-// ------------------------------------------------------------------------------------
-constexpr int kDeepThreads = 256;
 
 // A window's view of an int32 integral in global memory: element (dy, dx) relative to the window origin.  Natural
 // layout: sh = 0.  Column-de-interleaved level (PyrLevel::di; window origins have even x there): sh = 1, half =
@@ -1043,212 +1034,325 @@ __device__ __forceinline__ int rect_sum_g(const SumView &v, uint32_t dxw, uint32
            v.at((int)((dyw >> 16) & 255u), (int)((dxw >> 16) & 255u)) + v.at((int)(dyw >> 24), (int)(dxw >> 24));
 }
 
-// One tree of the generic cascade for one window: icvEvalHidHaarClassifier (tempcv.cpp:771-792) and
-// the stump fast paths (tempcv.cpp:872-930).  Returns the leaf value.
-__device__ __forceinline__ float deep_eval_tree(const DeepCascadeDev &D, int tree, const SumView &sum, const SumView &til,
-                                                double sigma, bool dbl) {
+// Image-pyramid mode: the windows of the cascade's levels (CasLevel) on the pyramid's integral images, DeepNode
+// records with byte corners (valid on any level pitch and on de-interleaved levels).  Queue items:
+// key = frame << 16 | cas_level << 8 | next stage (the tile kernel writes them too), xy = y << 16 | x.
+struct PyramidWindow {
+    typedef CascadeArgs Args;
+    static constexpr bool kTreePass = false;   // stage trees go to k_generic_deep (plan_mid_passes plans no pass for them)
+    int frame, cl, x, y;
+    CasLevel CL;
+    SumView sum, til;
+
+    static __device__ __forceinline__ ull grid_size(const Args &a) { return (ull)a.windows_per_frame * a.n_frames; }
+    __device__ __forceinline__ void locate(const Args &a, int f, long long w) {
+        int lo = 0, hi = a.n_cas_levels - 1;
+        while (lo < hi) {
+            const int mid = (lo + hi + 1) >> 1;
+            if (__ldg(&a.cas_levels[mid].win_base) <= w) lo = mid; else hi = mid - 1;
+        }
+        const int nx = __ldg(&a.cas_levels[lo].nx), ystep = __ldg(&a.cas_levels[lo].ystep);
+        const int local = (int)(w - __ldg(&a.cas_levels[lo].win_base));
+        const int iy = local / nx;
+        frame = f; cl = lo; x = (local - iy * nx) * ystep; y = iy * ystep;
+    }
+    __device__ __forceinline__ void from_grid(const Args &a, ull item, int &) {
+        const int f = (int)(item / (ull)a.windows_per_frame);
+        locate(a, f, (long long)(item - (ull)f * a.windows_per_frame));
+    }
+    __device__ __forceinline__ void from_queue(const Args &, const QueueItem &q, int &stage) {
+        frame = q.key >> 16; cl = (q.key >> 8) & 255; stage = q.key & 255;
+        x = q.xy & 0xffff; y = q.xy >> 16;
+    }
+    __device__ __forceinline__ QueueItem item(int next_stage) const {
+        QueueItem it;
+        it.key = ((uint32_t)frame << 16) | ((uint32_t)cl << 8) | (uint32_t)next_stage;
+        it.xy = ((uint32_t)y << 16) | (uint32_t)x;
+        return it;
+    }
+    __device__ __forceinline__ bool setup(const Args &a, double &sigma) {
+        const DeepCascadeDev &D = a.deep;
+        CL = a.cas_levels[cl];
+        const PyrLevel L = a.levels[CL.pyr_level];
+        const int pitch = L.sum_pitch;
+        const size_t lvl = (size_t)frame * a.sum_frame_stride + L.sum_off;
+        sum = sum_view(a.sum, L, lvl, y, x, L.di != 0);
+        til = a.tilted ? sum_view(a.tilted, L, lvl, y, x, false) : sum;
+        const int eq_w = D.win_w - 2, eq_h = D.win_h - 2;
+        const int g0 = pitch + 1, g1 = g0 + eq_w, g2 = (1 + eq_h) * pitch + 1, g3 = g2 + eq_w;
+        const int s4 = sum.at(1, 1) - sum.at(1, 1 + eq_w) - sum.at(1 + eq_h, 1) + sum.at(1 + eq_h, 1 + eq_w);
+        const ull q4 = sq_rect(a.sq, a.sq32 != 0, lvl + (size_t)y * pitch + x, g0, g1, g2, g3);
+        sigma = window_sigma(s4, q4, D.inv_area);
+        return true;
+    }
+    struct Node { uint4 c0, c1; float w0, w1, w2, thr; int left, right, flags; };   // c0 = dx[0..11], dy[0..3]; c1 = dy[4..11]
+    __device__ __forceinline__ Node node(const DeepCascadeDev &D, int n) const {
+        const uint4 *nd = reinterpret_cast<const uint4 *>(D.nodes + n);
+        Node r;
+        r.c0 = __ldg(nd); r.c1 = __ldg(nd + 1);
+        const uint4 c2 = __ldg(nd + 2);
+        r.flags = __ldg(reinterpret_cast<const int *>(nd + 3));
+        r.w0 = __uint_as_float(r.c1.z); r.w1 = __uint_as_float(r.c1.w); r.w2 = __uint_as_float(c2.x); r.thr = __uint_as_float(c2.y);
+        r.left = (int)c2.z; r.right = (int)c2.w;
+        return r;
+    }
+    __device__ __forceinline__ int rect(const Node &nd, int k) const {
+        const SumView &base = (nd.flags & 1) ? til : sum;
+        return k == 0 ? rect_sum_g(base, nd.c0.x, nd.c0.w) : k == 1 ? rect_sum_g(base, nd.c0.y, nd.c1.x) : rect_sum_g(base, nd.c0.z, nd.c1.y);
+    }
+    __device__ __forceinline__ void finish(const Args &a, int code, bool accepted) const {
+        if (accepted) emit_rect(a, CL, frame, x, y);
+        if (a.codes) a.codes[(size_t)frame * a.windows_per_frame + CL.win_base + (size_t)(y / CL.ystep) * CL.nx + x / CL.ystep] = (int16_t)code;
+    }
+};
+
+// Scale-cascade mode: the windows of the scales (ScLevel) on the frame's own integral image, ScNode records with the
+// corners of each scale as element offsets.  Rects are left to k_sc_rows.  Queue items: key = frame, xy = window.
+struct ScaleWindow {
+    typedef ScArgs Args;
+    static constexpr bool kTreePass = true;    // a stage tree runs as one k_generic_pass (plan_sc_cascade)
+    int frame;
+    long long w;
+    const int32_t *__restrict__ sum;
+    const int32_t *__restrict__ til;
+    const ScNode *__restrict__ nodes;
+
+    // the tile kernel took the windows below first_window
+    static __device__ __forceinline__ ull grid_size(const Args &a) { return (ull)(a.windows_per_frame - a.first_window) * a.n_frames; }
+    __device__ __forceinline__ void from_grid(const Args &a, ull item, int &) {
+        const ull per_frame = (ull)(a.windows_per_frame - a.first_window);
+        frame = (int)(item / per_frame); w = a.first_window + (long long)(item - (ull)frame * per_frame);
+    }
+    __device__ __forceinline__ void from_queue(const Args &, const QueueItem &q, int &) { frame = (int)q.key; w = (long long)q.xy; }
+    __device__ __forceinline__ QueueItem item(int) const {
+        QueueItem it;
+        it.key = (uint32_t)frame; it.xy = (uint32_t)w;
+        return it;
+    }
+    __device__ __forceinline__ bool setup(const Args &a, double &sigma) {
+        int lo = 0, hi = a.n_scales - 1;
+        while (lo < hi) {
+            const int mid = (lo + hi + 1) >> 1;
+            if (__ldg(&a.scales[mid].win_base) <= w) lo = mid; else hi = mid - 1;
+        }
+        const ScLevel L = a.scales[lo];
+        const int local = (int)(w - L.win_base);
+        const int iy = local / L.nx, ix = local - iy * L.nx;
+        const int x = __double2int_rn(__dmul_rn((double)ix, L.ystep));   // cvRound(ix*ystep), tempcv.cpp:1144
+        const int y = __double2int_rn(__dmul_rn((double)iy, L.ystep));   // cvRound(iy*ystep), tempcv.cpp:1141
+        if (x < 0 || y < 0 || x + L.win_w >= a.W + 1 || y + L.win_h >= a.H + 1) {   // tempcv.cpp:817-820
+            a.codes[(size_t)frame * a.windows_per_frame + w] = (int16_t)kScCodeOutside;
+            return false;
+        }
+        const size_t off = (size_t)frame * a.sum_frame_stride + (size_t)y * a.pitch + x;
+        sum = a.sum + off;
+        til = a.tilted ? a.tilted + off : sum;
+        const ull *__restrict__ sq = a.sq + off;
+        const int s4 = __ldg(sum + L.eq_off[0]) - __ldg(sum + L.eq_off[1]) - __ldg(sum + L.eq_off[2]) + __ldg(sum + L.eq_off[3]);
+        const ull q4 = __ldg(sq + L.eq_off[0]) - __ldg(sq + L.eq_off[1]) - __ldg(sq + L.eq_off[2]) + __ldg(sq + L.eq_off[3]);
+        sigma = window_sigma(s4, q4, L.inv_area);
+        nodes = a.nodes + L.node_base;
+        return true;
+    }
+    struct Node { int4 o0, o1; const int4 *o2; float w0, w1, w2, thr; int left, right, flags; };
+    __device__ __forceinline__ Node node(const DeepCascadeDev &, int n) const {
+        const ScNode *nd = nodes + n;
+        Node r;
+        r.o0 = __ldg(reinterpret_cast<const int4 *>(nd->off));
+        r.o1 = __ldg(reinterpret_cast<const int4 *>(nd->off) + 1);
+        r.o2 = reinterpret_cast<const int4 *>(nd->off) + 2;   // loaded by three-rect nodes only
+        const float4 wt = __ldg(reinterpret_cast<const float4 *>(nd->w));   // w0, w1, w2, thr
+        const int4 lr = __ldg(reinterpret_cast<const int4 *>(&nd->left));   // left, right, flags, pad
+        r.w0 = wt.x; r.w1 = wt.y; r.w2 = wt.z; r.thr = wt.w;
+        r.left = lr.x; r.right = lr.y; r.flags = lr.z;
+        return r;
+    }
+    __device__ __forceinline__ int rect(const Node &nd, int k) const {
+        const int32_t *__restrict__ base = (nd.flags & 1) ? til : sum;
+        const int4 o = k == 0 ? nd.o0 : k == 1 ? nd.o1 : __ldg(nd.o2);
+        return __ldg(base + o.x) - __ldg(base + o.y) - __ldg(base + o.z) + __ldg(base + o.w);
+    }
+    __device__ __forceinline__ void finish(const Args &a, int code, bool) const {
+        a.codes[(size_t)frame * a.windows_per_frame + w] = (int16_t)code;
+    }
+};
+
+// One tree for one window: icvEvalHidHaarClassifier (tempcv.cpp:771-792) and the stump fast paths
+// (tempcv.cpp:872-930).  Returns the leaf value.
+template <class Win>
+__device__ __forceinline__ float eval_tree(const DeepCascadeDev &D, const Win &win, int tree, double sigma, bool dbl) {
     const int n0 = __ldg(D.tree_first_node + tree);
     int idx = 0;
     do {
-        const uint4 *nd = reinterpret_cast<const uint4 *>(D.nodes + n0 + idx);
-        const uint4 c0 = __ldg(nd), c1 = __ldg(nd + 1), c2 = __ldg(nd + 2);
-        const int flags = __ldg(reinterpret_cast<const int *>(nd + 3));
-        // c0 = dx[0..11], dy[0..3]; c1 = dy[4..11], w0, w1; c2 = w2, thr, left, right
-        const SumView &base = (flags & 1) ? til : sum;
-        const int r0 = rect_sum_g(base, c0.x, c0.w);
-        const int r1 = rect_sum_g(base, c0.y, c1.x);
-        const float w0 = __uint_as_float(c1.z), w1 = __uint_as_float(c1.w);
-        const float thr = __uint_as_float(c2.y);
-        const double t = __dmul_rn((double)thr, sigma);
+        const typename Win::Node nd = win.node(D, n0 + idx);
+        const int r0 = win.rect(nd, 0), r1 = win.rect(nd, 1);
+        const double t = __dmul_rn((double)nd.thr, sigma);
         double sv;
-        if (dbl) {
-            sv = __fma_rn((double)r1, (double)w1, __dmul_rn((double)r0, (double)w0));
+        if (dbl) {   // both products are exact in double, so one fma equals mul, mul, add
+            sv = __fma_rn((double)r1, (double)nd.w1, __dmul_rn((double)r0, (double)nd.w0));
         } else {
-            sv = __dadd_rn((double)__fmul_rn(__int2float_rn(r0), w0), (double)__fmul_rn(__int2float_rn(r1), w1));
-            if ((flags >> 8) == 3) {
-                const int r2 = rect_sum_g(base, c0.z, c1.y);
-                sv = __dadd_rn(sv, (double)__fmul_rn(__int2float_rn(r2), __uint_as_float(c2.x)));
-            }
+            sv = __dadd_rn((double)__fmul_rn(__int2float_rn(r0), nd.w0), (double)__fmul_rn(__int2float_rn(r1), nd.w1));
+            if ((nd.flags >> 8) == 3) sv = __dadd_rn(sv, (double)__fmul_rn(__int2float_rn(win.rect(nd, 2)), nd.w2));
         }
-        idx = sv < t ? (int)c2.z : (int)c2.w;
+        idx = sv < t ? nd.left : nd.right;
     } while (idx > 0);
     return __ldg(D.alpha + n0 + tree - idx);
 }
 
-// ------------------------------------------------------------------------------------
-// mid kernel: one THREAD per window for the stages [mid_begin, mid_end) of a linear cascade
-// whose trees the tile kernel cannot evaluate (multi-node trees, tilted features).  Those
-// stages have few trees (3, 9, 14, ... in frontalface_alt2), so a warp per window would idle
-// most lanes, and they still see most windows.  Input: every grid window (cascades without a
-// tile prefix) or the tile kernel's queue; survivors go to the second queue for the deep kernel.
-// Lanes hold consecutive windows, so the corner loads of a warp fall into a few cache lines.
-// Run in a few passes of two or three stages each, ping-ponging between the two queues, so
-// the lanes are re-compacted while the survivor count still drops fast.
-// ------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(128) k_cascade_mid(const __grid_constant__ CascadeArgs a) {
+// A stage sum for one window, one thread: the trees in order.
+template <class Win>
+__device__ __forceinline__ double thread_stage_sum(const DeepCascadeDev &D, const Win &win, const DeepStage &st, double sigma, bool dbl) {
+    double S = 0.0;
+    for (int j = 0; j < st.ntrees; j++) S = __dadd_rn(S, (double)eval_tree(D, win, st.first_tree + j, sigma, dbl));
+    return S;
+}
+
+// A stage sum for one window, one warp: lanes stride over the trees; shuffle-reduced when the order does not matter
+// (flags bit 1), otherwise the lanes' leaf values are added in tree order.
+template <class Win>
+__device__ __forceinline__ double warp_stage_sum(const DeepCascadeDev &D, const Win &win, const DeepStage &st, double sigma, int lane) {
+    const bool dbl = st.flags & 1, order_free = st.flags & 2;
+    double S = 0.0, part = 0.0;
+    for (int j0 = 0; j0 < st.ntrees; j0 += 32) {
+        const int j = j0 + lane;
+        float av = 0.f;
+        if (j < st.ntrees) av = eval_tree(D, win, st.first_tree + j, sigma, dbl);
+        if (order_free) {
+            part = __dadd_rn(part, (double)av);
+        } else {
+            const int cnt = min(32, st.ntrees - j0);
+            for (int k = 0; k < cnt; k++) S = __dadd_rn(S, (double)__shfl_sync(0xffffffffu, av, k));
+        }
+    }
+    if (order_free) {
+#pragma unroll
+        for (int d = 16; d > 0; d >>= 1) part = __dadd_rn(part, __shfl_xor_sync(0xffffffffu, part, d));
+        S = part;
+    }
+    return S;
+}
+
+// Stages [i, end) of a linear cascade (tempcv.cpp:862-966): the first stage that rejects, or end.
+template <class StageSum>
+__device__ __forceinline__ int run_stages(const DeepCascadeDev &D, int i, int end, StageSum stage_sum) {
+    for (; i < end; i++) {
+        const DeepStage st = D.stages[i];
+        if (stage_sum(st) < (double)st.thr) break;
+    }
+    return i;
+}
+
+// The stage-tree walk from stage ptr (tempcv.cpp:834-861): 2 * last stage evaluated + accepted.
+template <class StageSum>
+__device__ __forceinline__ int walk_stage_tree(const DeepCascadeDev &D, int ptr, StageSum stage_sum) {
+    for (;;) {
+        const DeepStage st = D.stages[ptr];
+        if (stage_sum(st) >= (double)st.thr) {
+            if (st.child < 0) return 2 * ptr + 1;
+            ptr = st.child;
+        } else {
+            int p = ptr;
+            while (p >= 0 && __ldg(&D.stages[p].next) < 0) p = __ldg(&D.stages[p].parent);
+            if (p < 0) return 2 * ptr;
+            ptr = __ldg(&D.stages[p].next);
+        }
+    }
+}
+
+// Appends the windows whose lane has pass_on set to p.out: one atomic per warp; overflow is counted in counters[3].
+template <class Win>
+__device__ __forceinline__ void append_survivors(bool pass_on, const Win &win, const PassArgs &p, ull cap, ull *counters, int lane) {
+    const unsigned m = __ballot_sync(0xffffffffu, pass_on);
+    if (!m) return;
+    ull qb = 0;
+    if (lane == 0) qb = atomicAdd(p.out_count, (ull)__popc(m));
+    qb = __shfl_sync(0xffffffffu, qb, 0);
+    if (!pass_on) return;
+    const ull slot = qb + __popc(m & ((1u << lane) - 1u));
+    if (slot < cap) p.out[slot] = win.item(p.stage_end);
+    else atomicAdd(counters + 3, 1ull);
+}
+
+template <class Win>
+__global__ void __launch_bounds__(128) k_generic_pass(const __grid_constant__ typename Win::Args a, const __grid_constant__ PassArgs p) {
     const DeepCascadeDev &D = a.deep;
     const int lane = threadIdx.x & 31;
-    const bool from_grid = a.mid_in == nullptr;
-    ull n = from_grid ? (ull)a.windows_per_frame * a.n_frames : *a.mid_in_count;
+    const bool from_grid = p.in == nullptr;
+    ull n = from_grid ? Win::grid_size(a) : *p.in_count;
     if (!from_grid && n > a.queue_cap) n = a.queue_cap;
+    const bool last_pass = p.stage_end >= D.n_stages;
     const ull stride = (ull)gridDim.x * 128;
-    // whole warps iterate together (ballots below)
+    // whole warps iterate together (ballot in append_survivors)
     for (ull base_item = ((ull)blockIdx.x * 128 + threadIdx.x) - lane; base_item < n; base_item += stride) {
         const ull item = base_item + lane;
-        const bool valid = item < n;
-        int frame = 0, cl = 0, x = 0, y = 0;
-        if (valid) {
-            if (from_grid) {
-                frame = (int)(item / (ull)a.windows_per_frame);
-                const long long w = (long long)(item - (ull)frame * a.windows_per_frame);
-                int lo = 0, hi = a.n_cas_levels - 1;
-                while (lo < hi) {
-                    const int mid = (lo + hi + 1) >> 1;
-                    if (__ldg(&a.cas_levels[mid].win_base) <= w) lo = mid; else hi = mid - 1;
-                }
-                cl = lo;
-                const int nx = __ldg(&a.cas_levels[lo].nx), ystep = __ldg(&a.cas_levels[lo].ystep);
-                const int local = (int)(w - __ldg(&a.cas_levels[lo].win_base));
-                const int iy = local / nx;
-                x = (local - iy * nx) * ystep; y = iy * ystep;
+        Win win;
+        bool pass_on = false;
+        double sigma;
+        int stage = p.stage_begin;
+        if (item < n) {
+            if (from_grid) win.from_grid(a, item, stage);
+            else win.from_queue(a, p.in[item], stage);
+        }
+        if (item < n && win.setup(a, sigma)) {
+            // (a stage tree never sets flags bit 0: its walk is compiled without the stump fast path)
+            auto tree_sum = [&](const DeepStage &st) { return thread_stage_sum(D, win, st, sigma, false); };
+            auto stage_sum = [&](const DeepStage &st) { return thread_stage_sum(D, win, st, sigma, st.flags & 1); };
+            if (Win::kTreePass && D.is_tree) {
+                const int code = walk_stage_tree(D, stage, tree_sum);
+                win.finish(a, code, code & 1);
             } else {
-                const QueueItem q = a.mid_in[item];
-                frame = q.key >> 16; cl = (q.key >> 8) & 255;
-                x = q.xy & 0xffff; y = q.xy >> 16;
+                stage = run_stages(D, stage, p.stage_end, stage_sum);
+                if (stage < p.stage_end || last_pass) win.finish(a, stage, stage >= D.n_stages);   // rejected at stage, or accepted
+                else pass_on = true;
             }
         }
-        bool alive = valid;
-        int stage = D.mid_begin;
-        const CasLevel CL = a.cas_levels[cl];
-        if (valid) {
-            const PyrLevel L = a.levels[CL.pyr_level];
-            const int pitch = L.sum_pitch;
-            const size_t off = (size_t)frame * a.sum_frame_stride + L.sum_off + (size_t)y * pitch + x;
-            const size_t lvl = (size_t)frame * a.sum_frame_stride + L.sum_off;
-            const SumView sum = sum_view(a.sum, L, lvl, y, x, L.di != 0);
-            const SumView til = a.tilted ? sum_view(a.tilted, L, lvl, y, x, false) : sum;
-            const int eq_w = D.win_w - 2, eq_h = D.win_h - 2;
-            const int g0 = pitch + 1, g1 = g0 + eq_w, g2 = (1 + eq_h) * pitch + 1, g3 = g2 + eq_w;
-            const int s4 = sum.at(1, 1) - sum.at(1, 1 + eq_w) - sum.at(1 + eq_h, 1) + sum.at(1 + eq_h, 1 + eq_w);
-            const ull q4 = sq_rect(a.sq, a.sq32 != 0, off, g0, g1, g2, g3);
-            const double sigma = window_sigma(s4, q4, D.inv_area);
-            for (; stage < D.mid_end; stage++) {
-                const DeepStage st = D.stages[stage];
-                const bool dbl = st.flags & 1;
-                double S = 0.0;
-                for (int j = 0; j < st.ntrees; j++)
-                    S = __dadd_rn(S, (double)deep_eval_tree(D, st.first_tree + j, sum, til, sigma, dbl));
-                if (S < (double)st.thr) { alive = false; break; }
-            }
-        }
-        if (valid && !alive && a.codes)
-            a.codes[(size_t)frame * a.windows_per_frame + CL.win_base + (size_t)(y / CL.ystep) * CL.nx + x / CL.ystep] = (int16_t)stage;
-        const bool accepted = alive && D.mid_end >= D.n_stages;
-        if (accepted) {
-            emit_rect(a, CL, frame, x, y);
-            if (a.codes)
-                a.codes[(size_t)frame * a.windows_per_frame + CL.win_base + (size_t)(y / CL.ystep) * CL.nx + x / CL.ystep] = (int16_t)D.n_stages;
-        }
-        const bool pass_on = alive && !accepted;
-        const unsigned m = __ballot_sync(0xffffffffu, pass_on);
-        if (m) {
-            ull qb = 0;
-            if (lane == 0) qb = atomicAdd(a.mid_out_count, (ull)__popc(m));
-            qb = __shfl_sync(0xffffffffu, qb, 0);
-            if (pass_on) {
-                const ull slot = qb + __popc(m & ((1u << lane) - 1u));
-                if (slot < a.queue_cap) {
-                    QueueItem it;
-                    it.key = ((uint32_t)frame << 16) | ((uint32_t)cl << 8) | (uint32_t)D.mid_end;
-                    it.xy = ((uint32_t)y << 16) | (uint32_t)x;
-                    a.mid_out[slot] = it;
-                } else {
-                    atomicAdd(a.counters + 3, 1ull);
-                }
-            }
-        }
+        append_survivors(pass_on, win, p, a.queue_cap, a.counters, lane);
     }
 }
 
-cudaError_t launch_cascade_mid(const CascadeArgs &a, int n_sms, cudaStream_t stream) {
-    if (a.n_frames == 0) return cudaSuccess;
-    k_cascade_mid<<<n_sms * 16, 128, 0, stream>>>(a);
+template <class Win>
+__global__ void __launch_bounds__(256) k_generic_deep(const __grid_constant__ typename Win::Args a, const __grid_constant__ PassArgs p) {
+    const DeepCascadeDev &D = a.deep;
+    const int lane = threadIdx.x & 31;
+    const ull warp0 = ((ull)blockIdx.x * 256 + threadIdx.x) >> 5;
+    const ull nwarps = ((ull)gridDim.x * 256) >> 5;
+    const bool from_grid = p.in == nullptr;
+    ull n = from_grid ? Win::grid_size(a) : *p.in_count;
+    if (!from_grid && n > a.queue_cap) n = a.queue_cap;
+    if (from_grid && blockIdx.x == 0 && threadIdx.x == 0) a.counters[1] = n;   // every window was handed to this kernel
+    for (ull item = warp0; item < n; item += nwarps) {
+        Win win;
+        double sigma;
+        int stage = p.stage_begin;
+        if (from_grid) win.from_grid(a, item, stage);
+        else win.from_queue(a, p.in[item], stage);
+        if (!win.setup(a, sigma)) continue;
+        auto stage_sum = [&](const DeepStage &st) { return warp_stage_sum(D, win, st, sigma, lane); };
+        const int code = D.is_tree ? walk_stage_tree(D, stage, stage_sum) : run_stages(D, stage, D.n_stages, stage_sum);
+        if (lane == 0) win.finish(a, code, D.is_tree ? (code & 1) : code >= D.n_stages);
+    }
+}
+
+template <class Args> struct WindowOf;
+template <> struct WindowOf<CascadeArgs> { typedef PyramidWindow type; };
+template <> struct WindowOf<ScArgs> { typedef ScaleWindow type; };
+
+template <class Args>
+cudaError_t launch_generic_pass(const Args &a, const PassArgs &p, int n_sms, cudaStream_t stream) {
+    if (a.windows_per_frame == 0 || a.n_frames == 0) return cudaSuccess;
+    k_generic_pass<typename WindowOf<Args>::type><<<n_sms * 16, 128, 0, stream>>>(a, p);
     return cudaGetLastError();
 }
-
-__global__ void __launch_bounds__(kDeepThreads) k_cascade_deep(const __grid_constant__ CascadeArgs a) {
-    const int lane = threadIdx.x & 31;
-    const ull warp0 = ((ull)blockIdx.x * kDeepThreads + threadIdx.x) >> 5;
-    const ull nwarps = ((ull)gridDim.x * kDeepThreads) >> 5;
-    ull n = *a.deep_count;
-    if (n > a.queue_cap) n = a.queue_cap;
-    const DeepCascadeDev &D = a.deep;
-
-    for (ull item = warp0; item < n; item += nwarps) {
-        const QueueItem q = a.deep_in[item];
-        const int frame = q.key >> 16, cl = (q.key >> 8) & 255, stage0 = q.key & 255;
-        const int x = q.xy & 0xffff, y = q.xy >> 16;
-        const CasLevel CL = a.cas_levels[cl];
-        const PyrLevel L = a.levels[CL.pyr_level];
-        const int pitch = L.sum_pitch;
-        const size_t off = (size_t)frame * a.sum_frame_stride + L.sum_off + (size_t)y * pitch + x;
-        const size_t lvl = (size_t)frame * a.sum_frame_stride + L.sum_off;
-        const SumView sum = sum_view(a.sum, L, lvl, y, x, L.di != 0);
-        const SumView til = a.tilted ? sum_view(a.tilted, L, lvl, y, x, false) : sum;
-
-        const int eq_w = D.win_w - 2, eq_h = D.win_h - 2;
-        const int g0 = pitch + 1, g1 = g0 + eq_w, g2 = (1 + eq_h) * pitch + 1, g3 = g2 + eq_w;
-        const int s4 = sum.at(1, 1) - sum.at(1, 1 + eq_w) - sum.at(1 + eq_h, 1) + sum.at(1 + eq_h, 1 + eq_w);
-        const ull q4 = sq_rect(a.sq, a.sq32 != 0, off, g0, g1, g2, g3);
-        const double sigma = window_sigma(s4, q4, D.inv_area);
-
-        int ptr = stage0, last = stage0, accepted = 0;
-        for (;;) {
-            const DeepStage st = D.stages[ptr];
-            last = ptr;
-            const bool dbl = st.flags & 1, order_free = st.flags & 2;
-            double S = 0.0, part = 0.0;
-            for (int j0 = 0; j0 < st.ntrees; j0 += 32) {
-                const int j = j0 + lane;
-                float av = 0.f;
-                if (j < st.ntrees) av = deep_eval_tree(D, st.first_tree + j, sum, til, sigma, dbl);
-                if (order_free) {
-                    part = __dadd_rn(part, (double)av);
-                } else {
-                    const int cnt = min(32, st.ntrees - j0);
-                    for (int k = 0; k < cnt; k++) S = __dadd_rn(S, (double)__shfl_sync(0xffffffffu, av, k));
-                }
-            }
-            if (order_free) {
-#pragma unroll
-                for (int d = 16; d > 0; d >>= 1) part = __dadd_rn(part, __shfl_xor_sync(0xffffffffu, part, d));
-                S = part;
-            }
-            const bool pass = S >= (double)st.thr;
-            if (D.is_tree) {  // tempcv.cpp:849-859
-                if (pass) {
-                    ptr = st.child;
-                    if (ptr < 0) { accepted = 1; break; }
-                } else {
-                    int p = ptr;
-                    while (p >= 0 && __ldg(&D.stages[p].next) < 0) p = __ldg(&D.stages[p].parent);
-                    if (p < 0) break;
-                    ptr = __ldg(&D.stages[p].next);
-                }
-            } else {
-                if (!pass) break;
-                if (++ptr >= D.n_stages) { accepted = 1; break; }
-            }
-        }
-        if (lane == 0) {
-            if (accepted) emit_rect(a, CL, frame, x, y);
-            if (a.codes) {
-                const int code = D.is_tree ? 2 * last + accepted : (accepted ? D.n_stages : last);
-                a.codes[(size_t)frame * a.windows_per_frame + CL.win_base + (size_t)(y / CL.ystep) * CL.nx + x / CL.ystep] = (int16_t)code;
-            }
-        }
-    }
+template <class Args>
+cudaError_t launch_generic_deep(const Args &a, const PassArgs &p, int n_sms, cudaStream_t stream) {
+    if (a.windows_per_frame == 0 || a.n_frames == 0) return cudaSuccess;
+    k_generic_deep<typename WindowOf<Args>::type><<<n_sms * 8, 256, 0, stream>>>(a, p);
+    return cudaGetLastError();
 }
+template cudaError_t launch_generic_pass(const CascadeArgs &, const PassArgs &, int, cudaStream_t);
+template cudaError_t launch_generic_pass(const ScArgs &, const PassArgs &, int, cudaStream_t);
+template cudaError_t launch_generic_deep(const CascadeArgs &, const PassArgs &, int, cudaStream_t);
+template cudaError_t launch_generic_deep(const ScArgs &, const PassArgs &, int, cudaStream_t);
 
 // ------------------------------------------------------------------------------------
 // reject levels (cvHaarDetectObjectsForROC with outputRejectLevels, tempcv.cpp:1084-1094):
@@ -1269,36 +1373,18 @@ __global__ void __launch_bounds__(256) k_roc_collect(const CascadeArgs a, RocIte
         if (D.n_stages - code >= 4) return;
         level = code; last = code == D.n_stages ? D.n_stages - 1 : code;
     }
-    int lo = 0, hi = a.n_cas_levels - 1;
-    while (lo < hi) {
-        const int mid = (lo + hi + 1) >> 1;
-        if (__ldg(&a.cas_levels[mid].win_base) <= w) lo = mid; else hi = mid - 1;
-    }
-    const CasLevel CL = a.cas_levels[lo];
-    const PyrLevel L = a.levels[CL.pyr_level];
-    const int local = (int)(w - CL.win_base);
-    const int iy = local / CL.nx, ix = local - iy * CL.nx;
-    const int x = ix * CL.ystep, y = iy * CL.ystep;
-    const int pitch = L.sum_pitch;
-    const size_t off = (size_t)frame * a.sum_frame_stride + L.sum_off + (size_t)y * pitch + x;
-    const size_t lvl = (size_t)frame * a.sum_frame_stride + L.sum_off;
-    const SumView sum = sum_view(a.sum, L, lvl, y, x, L.di != 0);
-    const SumView til = a.tilted ? sum_view(a.tilted, L, lvl, y, x, false) : sum;
-    const int eq_w = D.win_w - 2, eq_h = D.win_h - 2;
-    const int g0 = pitch + 1, g1 = g0 + eq_w, g2 = (1 + eq_h) * pitch + 1, g3 = g2 + eq_w;
-    const int s4 = sum.at(1, 1) - sum.at(1, 1 + eq_w) - sum.at(1 + eq_h, 1) + sum.at(1 + eq_h, 1 + eq_w);
-    const ull q4 = sq_rect(a.sq, a.sq32 != 0, off, g0, g1, g2, g3);
-    const double sigma = window_sigma(s4, q4, D.inv_area);
+    PyramidWindow win;
+    win.locate(a, frame, w);
+    double sigma;
+    win.setup(a, sigma);
     const DeepStage st = D.stages[last];
-    double S = 0.0;
-    for (int j = 0; j < st.ntrees; j++)
-        S = __dadd_rn(S, (double)deep_eval_tree(D, st.first_tree + j, sum, til, sigma, st.flags & 1));
+    const double S = thread_stage_sum(D, win, st, sigma, st.flags & 1);
     const ull slot = atomicAdd(counter, 1ull);
     if (slot >= cap) return;
     RocItem it;
-    it.r.x = __double2int_rn(__dmul_rn((double)x, CL.factor));
-    it.r.y = __double2int_rn(__dmul_rn((double)y, CL.factor));
-    it.r.w = CL.win_w; it.r.h = CL.win_h; it.r.frame = a.frame_base + frame; it.r.cascade = a.cascade_index;
+    it.r.x = __double2int_rn(__dmul_rn((double)win.x, win.CL.factor));
+    it.r.y = __double2int_rn(__dmul_rn((double)win.y, win.CL.factor));
+    it.r.w = win.CL.win_w; it.r.h = win.CL.win_h; it.r.frame = a.frame_base + frame; it.r.cascade = a.cascade_index;
     it.level = level; it.pad = 0; it.win = w; it.weight = S;
     out[slot] = it;
 }
@@ -1306,12 +1392,6 @@ __global__ void __launch_bounds__(256) k_roc_collect(const CascadeArgs a, RocIte
 cudaError_t launch_roc_collect(const CascadeArgs &a, RocItem *out, unsigned long long cap, unsigned long long *counter, cudaStream_t stream) {
     if (a.windows_per_frame == 0 || a.n_frames == 0) return cudaSuccess;
     k_roc_collect<<<dim3((unsigned)((a.windows_per_frame + 255) / 256), a.n_frames), 256, 0, stream>>>(a, out, cap, counter);
-    return cudaGetLastError();
-}
-
-cudaError_t launch_cascade_deep(const CascadeArgs &a, int n_sms, cudaStream_t stream) {
-    if (a.n_frames == 0) return cudaSuccess;
-    k_cascade_deep<<<n_sms * 8, kDeepThreads, 0, stream>>>(a);
     return cudaGetLastError();
 }
 

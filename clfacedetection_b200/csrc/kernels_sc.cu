@@ -6,21 +6,17 @@
 // features, one integral), so this is what replaces runStage when the caller asks for the
 // demo's other column.
 //
-//   k_sc_eval : one thread per grid position (scale, iy, ix), lanes = consecutive ix, so the
-//       32 corner loads of a warp are 32 * ystep * 4 bytes apart at most (a few cache lines);
-//       the integral image of a frame (8-25 MB) lives in L2.  Linear cascades run in a few
-//       passes over growing stage ranges with the survivors re-compacted through a queue in
-//       between (thread per survivor), so lanes stay busy; the large late stages (>= 32 trees) run
-//       one warp per survivor, lanes over trees (k_sc_deep).  Every position is evaluated --
-//       the reference's skip rule makes the set of evaluated windows depend on the RESULTS of
-//       their left neighbours, so it is applied afterwards:
+// The windows are evaluated by the tile kernel (scales of window step 2) and by the generic kernels
+// (kernels_clod.cu, ScaleWindow): one thread per grid position (scale, iy, ix), lanes = consecutive ix,
+// so the 32 corner loads of a warp are 32 * ystep * 4 bytes apart at most (a few cache lines); the
+// integral image of a frame (8-25 MB) lives in L2.  Linear cascades run in a few passes over growing
+// stage ranges with the survivors re-compacted through a queue in between, and the large late stages
+// (>= 50 trees) one warp per survivor, lanes over trees.  Every position is evaluated -- the
+// reference's skip rule makes the set of evaluated windows depend on the RESULTS of their left
+// neighbours, so it is applied afterwards:
 //   k_sc_rows : one thread per grid row walks its exit codes left to right with the invoker's
 //       rule "ixstep = result != 0 ? 1 : 2" (tempcv.cpp:1161), marks the positions the
 //       reference never evaluates and appends a rect for every evaluated, accepted window.
-//
-// Arithmetic: exactly the reference's (no FP32 filter here): FP64 sigma with separately rounded
-// operations, float products accumulated in double, or exact double products on the stump
-// fast path (tempcv.cpp:872-898), stage sums in tree order.
 #include <cstdint>
 
 #include "kernels.h"
@@ -29,220 +25,16 @@ namespace clfd {
 
 typedef unsigned long long ull;
 
-__device__ __forceinline__ double sc_sigma(int s4, ull q4, double inv_area) {
-    // tempcv.cpp:822-832, every operation rounded separately
-    const double mean = __dmul_rn((double)s4, inv_area);
-    const double v = __dsub_rn(__dmul_rn((double)q4, inv_area), __dmul_rn(mean, mean));
-    return v >= 0. ? sqrt(v) : 1.;
-}
-
-// icvEvalHidHaarClassifier (tempcv.cpp:771-792) / the stump fast paths (tempcv.cpp:872-930)
-__device__ __forceinline__ float sc_eval_tree(const ScNode *__restrict__ nodes, int n0, const float *__restrict__ alpha_tree,
-                                              const int32_t *__restrict__ sum, const int32_t *__restrict__ til, double sigma,
-                                              bool dbl) {
-    int idx = 0;
-    do {
-        const ScNode *nd = nodes + n0 + idx;
-        const int4 o0 = __ldg(reinterpret_cast<const int4 *>(nd->off));
-        const int4 o1 = __ldg(reinterpret_cast<const int4 *>(nd->off) + 1);
-        const float4 wt = __ldg(reinterpret_cast<const float4 *>(nd->w));      // w0, w1, w2, thr
-        const int4 lr = __ldg(reinterpret_cast<const int4 *>(&nd->left));      // left, right, flags, pad
-        const int32_t *__restrict__ base = (lr.z & 1) ? til : sum;
-        const int r0 = __ldg(base + o0.x) - __ldg(base + o0.y) - __ldg(base + o0.z) + __ldg(base + o0.w);
-        const int r1 = __ldg(base + o1.x) - __ldg(base + o1.y) - __ldg(base + o1.z) + __ldg(base + o1.w);
-        const double t = __dmul_rn((double)wt.w, sigma);
-        double sv;
-        if (dbl) {   // both products are exact in double, so one fma equals mul, mul, add
-            sv = __fma_rn((double)r1, (double)wt.y, __dmul_rn((double)r0, (double)wt.x));
-        } else {
-            sv = __dadd_rn((double)__fmul_rn(__int2float_rn(r0), wt.x), (double)__fmul_rn(__int2float_rn(r1), wt.y));
-            if ((lr.z >> 8) == 3) {
-                const int4 o2 = __ldg(reinterpret_cast<const int4 *>(nd->off) + 2);
-                const int r2 = __ldg(base + o2.x) - __ldg(base + o2.y) - __ldg(base + o2.z) + __ldg(base + o2.w);
-                sv = __dadd_rn(sv, (double)__fmul_rn(__int2float_rn(r2), wt.z));
-            }
-        }
-        idx = sv < t ? lr.x : lr.y;
-    } while (idx > 0);
-    return __ldg(alpha_tree - idx);
-}
-
-// One pass: stages [a.stage_begin, a.stage_end) for every grid position (a.in == NULL) or for the
-// survivors of the previous pass (queue items: key = frame, xy = position index).  A window
-// rejected here gets its exit code; survivors of a pass that is not the last go to a.out.
-// Stage-tree cascades run as ONE pass (their walk is not a linear stage sequence).
-__global__ void __launch_bounds__(128) k_sc_eval(const __grid_constant__ ScArgs a) {
-    const DeepCascadeDev &D = a.deep;
-    const int lane = threadIdx.x & 31;
-    const bool from_grid = a.in == nullptr;
-    const ull grid_per_frame = (ull)(a.windows_per_frame - a.first_window);   // the tile kernel took the rest
-    ull n = from_grid ? grid_per_frame * a.n_frames : *a.in_count;
-    if (!from_grid && n > a.queue_cap) n = a.queue_cap;
-    const bool last_pass = a.stage_end >= D.n_stages;
-    const ull stride = (ull)gridDim.x * 128;
-    for (ull base_item = ((ull)blockIdx.x * 128 + threadIdx.x) - lane; base_item < n; base_item += stride) {
-        const ull item = base_item + lane;
-        const bool valid = item < n;
-        int frame = 0;
-        long long w = 0;
-        if (valid) {
-            if (from_grid) { frame = (int)(item / grid_per_frame); w = a.first_window + (long long)(item - (ull)frame * grid_per_frame); }
-            else { const QueueItem q = a.in[item]; frame = (int)q.key; w = (long long)q.xy; }
-        }
-        bool pass_on = false;
-        if (valid) {
-            int lo = 0, hi = a.n_levels - 1;
-            while (lo < hi) {
-                const int mid = (lo + hi + 1) >> 1;
-                if (__ldg(&a.levels[mid].win_base) <= w) lo = mid; else hi = mid - 1;
-            }
-            const ScLevel L = a.levels[lo];
-            const int local = (int)(w - L.win_base);
-            const int iy = local / L.nx, ix = local - iy * L.nx;
-            const int x = __double2int_rn(__dmul_rn((double)ix, L.ystep));   // cvRound(ix*ystep), tempcv.cpp:1144
-            const int y = __double2int_rn(__dmul_rn((double)iy, L.ystep));   // cvRound(iy*ystep), tempcv.cpp:1141
-            int16_t *code_out = a.codes + (size_t)frame * a.windows_per_frame + w;
-            if (x < 0 || y < 0 || x + L.win_w >= a.W + 1 || y + L.win_h >= a.H + 1) {   // tempcv.cpp:817-820
-                *code_out = (int16_t)kScCodeOutside;
-            } else {
-                const size_t off = (size_t)frame * a.sum_frame_stride + (size_t)y * a.pitch + x;
-                const int32_t *__restrict__ sum = a.sum + off;
-                const int32_t *__restrict__ til = a.tilted ? a.tilted + off : sum;
-                const ull *__restrict__ sq = a.sq + off;
-                const int s4 = __ldg(sum + L.eq_off[0]) - __ldg(sum + L.eq_off[1]) - __ldg(sum + L.eq_off[2]) + __ldg(sum + L.eq_off[3]);
-                const ull q4 = __ldg(sq + L.eq_off[0]) - __ldg(sq + L.eq_off[1]) - __ldg(sq + L.eq_off[2]) + __ldg(sq + L.eq_off[3]);
-                const double sigma = sc_sigma(s4, q4, L.inv_area);
-                const ScNode *__restrict__ nodes = a.nodes + L.node_base;
-                if (D.is_tree) {   // tempcv.cpp:834-861
-                    int ptr = 0, last = 0, accepted = 0;
-                    for (;;) {
-                        const DeepStage st = D.stages[ptr];
-                        last = ptr;
-                        double S = 0.0;
-                        for (int j = 0; j < st.ntrees; j++) {
-                            const int tree = st.first_tree + j, n0 = __ldg(D.tree_first_node + tree);
-                            S = __dadd_rn(S, (double)sc_eval_tree(nodes, n0, D.alpha + n0 + tree, sum, til, sigma, false));
-                        }
-                        if (S >= (double)st.thr) {
-                            ptr = st.child;
-                            if (ptr < 0) { accepted = 1; break; }
-                        } else {
-                            int p = ptr;
-                            while (p >= 0 && __ldg(&D.stages[p].next) < 0) p = __ldg(&D.stages[p].parent);
-                            if (p < 0) break;
-                            ptr = __ldg(&D.stages[p].next);
-                        }
-                    }
-                    *code_out = (int16_t)(2 * last + accepted);
-                } else {           // tempcv.cpp:862-966
-                    int i = a.stage_begin;
-                    for (; i < a.stage_end; i++) {
-                        const DeepStage st = D.stages[i];
-                        const bool dbl = st.flags & 1;
-                        double S = 0.0;
-                        for (int j = 0; j < st.ntrees; j++) {
-                            const int tree = st.first_tree + j, n0 = __ldg(D.tree_first_node + tree);
-                            S = __dadd_rn(S, (double)sc_eval_tree(nodes, n0, D.alpha + n0 + tree, sum, til, sigma, dbl));
-                        }
-                        if (S < (double)st.thr) break;
-                    }
-                    if (i < a.stage_end || last_pass) *code_out = (int16_t)i;   // rejected at i, or accepted (i == n_stages)
-                    else pass_on = true;
-                }
-            }
-        }
-        const unsigned m = __ballot_sync(0xffffffffu, pass_on);
-        if (m) {
-            ull qb = 0;
-            if (lane == 0) qb = atomicAdd(a.out_count, (ull)__popc(m));
-            qb = __shfl_sync(0xffffffffu, qb, 0);
-            if (pass_on) {
-                const ull slot = qb + __popc(m & ((1u << lane) - 1u));
-                if (slot < a.queue_cap) {
-                    QueueItem it;
-                    it.key = (uint32_t)frame; it.xy = (uint32_t)w;
-                    a.out[slot] = it;
-                } else {
-                    atomicAdd(a.counters + 3, 1ull);
-                }
-            }
-        }
-    }
-}
-
-// Final pass for the large stages (>= 32 trees): one WARP per surviving position, lanes stride over
-// the trees of a stage, from a.stage_begin to the end of a LINEAR cascade.  The stage sum is reduced
-// with shuffles when the packer proved it exact in any order (DeepStage flags bit1), otherwise the
-// lanes' leaf values are added in tree order.
-__global__ void __launch_bounds__(256) k_sc_deep(const __grid_constant__ ScArgs a) {
-    const DeepCascadeDev &D = a.deep;
-    const int lane = threadIdx.x & 31;
-    const ull warp0 = ((ull)blockIdx.x * 256 + threadIdx.x) >> 5;
-    const ull nwarps = ((ull)gridDim.x * 256) >> 5;
-    ull n = *a.in_count;
-    if (n > a.queue_cap) n = a.queue_cap;
-    for (ull item = warp0; item < n; item += nwarps) {
-        const QueueItem q = a.in[item];
-        const int frame = (int)q.key;
-        const long long w = (long long)q.xy;
-        int lo = 0, hi = a.n_levels - 1;
-        while (lo < hi) {
-            const int mid = (lo + hi + 1) >> 1;
-            if (__ldg(&a.levels[mid].win_base) <= w) lo = mid; else hi = mid - 1;
-        }
-        const ScLevel L = a.levels[lo];
-        const int local = (int)(w - L.win_base);
-        const int iy = local / L.nx, ix = local - iy * L.nx;
-        const int x = __double2int_rn(__dmul_rn((double)ix, L.ystep));
-        const int y = __double2int_rn(__dmul_rn((double)iy, L.ystep));
-        const size_t off = (size_t)frame * a.sum_frame_stride + (size_t)y * a.pitch + x;   // in bounds: checked by the first pass
-        const int32_t *__restrict__ sum = a.sum + off;
-        const int32_t *__restrict__ til = a.tilted ? a.tilted + off : sum;
-        const ull *__restrict__ sq = a.sq + off;
-        const int s4 = __ldg(sum + L.eq_off[0]) - __ldg(sum + L.eq_off[1]) - __ldg(sum + L.eq_off[2]) + __ldg(sum + L.eq_off[3]);
-        const ull q4 = __ldg(sq + L.eq_off[0]) - __ldg(sq + L.eq_off[1]) - __ldg(sq + L.eq_off[2]) + __ldg(sq + L.eq_off[3]);
-        const double sigma = sc_sigma(s4, q4, L.inv_area);
-        const ScNode *__restrict__ nodes = a.nodes + L.node_base;
-        int i = a.stage_begin;
-        for (; i < D.n_stages; i++) {
-            const DeepStage st = D.stages[i];
-            const bool dbl = st.flags & 1, order_free = st.flags & 2;
-            double S = 0.0, part = 0.0;
-            for (int j0 = 0; j0 < st.ntrees; j0 += 32) {
-                const int j = j0 + lane;
-                float av = 0.f;
-                if (j < st.ntrees) {
-                    const int tree = st.first_tree + j, n0 = __ldg(D.tree_first_node + tree);
-                    av = sc_eval_tree(nodes, n0, D.alpha + n0 + tree, sum, til, sigma, dbl);
-                }
-                if (order_free) {
-                    part = __dadd_rn(part, (double)av);
-                } else {
-                    const int cnt = min(32, st.ntrees - j0);
-                    for (int k = 0; k < cnt; k++) S = __dadd_rn(S, (double)__shfl_sync(0xffffffffu, av, k));
-                }
-            }
-            if (order_free) {
-#pragma unroll
-                for (int d = 16; d > 0; d >>= 1) part = __dadd_rn(part, __shfl_xor_sync(0xffffffffu, part, d));
-                S = part;
-            }
-            if (S < (double)st.thr) break;
-        }
-        if (lane == 0) a.codes[(size_t)frame * a.windows_per_frame + w] = (int16_t)i;   // rejected at i, or n_stages = accepted
-    }
-}
-
 __global__ void __launch_bounds__(128) k_sc_rows(const __grid_constant__ ScArgs a) {
     const int row = blockIdx.x * 128 + threadIdx.x;
     const int frame = blockIdx.y;
     if (row >= a.rows_per_frame) return;
-    int lo = 0, hi = a.n_levels - 1;
+    int lo = 0, hi = a.n_scales - 1;
     while (lo < hi) {
         const int mid = (lo + hi + 1) >> 1;
-        if (__ldg(&a.levels[mid].row_base) <= row) lo = mid; else hi = mid - 1;
+        if (__ldg(&a.scales[mid].row_base) <= row) lo = mid; else hi = mid - 1;
     }
-    const ScLevel L = a.levels[lo];
+    const ScLevel L = a.scales[lo];
     const int iy = row - L.row_base;
     int16_t *codes = a.codes + (size_t)frame * a.windows_per_frame + L.win_base + (size_t)iy * L.nx;
     const DeepCascadeDev &D = a.deep;
@@ -272,18 +64,6 @@ __global__ void __launch_bounds__(128) k_sc_rows(const __grid_constant__ ScArgs 
         }
         evaluate = result != 0;
     }
-}
-
-cudaError_t launch_sc_eval(const ScArgs &a, int n_sms, cudaStream_t stream) {
-    if (a.windows_per_frame == 0 || a.n_frames == 0) return cudaSuccess;
-    k_sc_eval<<<n_sms * 16, 128, 0, stream>>>(a);
-    return cudaGetLastError();
-}
-
-cudaError_t launch_sc_deep(const ScArgs &a, int n_sms, cudaStream_t stream) {
-    if (a.windows_per_frame == 0 || a.n_frames == 0) return cudaSuccess;
-    k_sc_deep<<<n_sms * 8, 256, 0, stream>>>(a);
-    return cudaGetLastError();
 }
 
 cudaError_t launch_sc_rows(const ScArgs &a, cudaStream_t stream) {

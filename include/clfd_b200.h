@@ -184,7 +184,7 @@ typedef struct clfd_level {
 typedef struct clfd_run_stats {
     int64_t windows;          /* windows evaluated (all frames, all cascades) */
     int64_t rects;            /* accepted windows */
-    int64_t deep_windows;     /* windows handed from the tile kernel to the mid / deep kernels */
+    int64_t deep_windows;     /* windows handed from the tile kernel to the generic kernels */
     int64_t kernel_launches;  /* kernels launched by the last enqueue */
     int64_t pyramid_pixels;   /* per frame */
     int64_t bytes_resize, bytes_integral, bytes_cascade; /* algorithmic bytes per frame (SURVEY 8-d); bytes_integral:

@@ -444,19 +444,27 @@ def test_submit_collect_pipeline_keeps_batches_apart(gpu_ctx):
     det.close()
 
 
-@pytest.mark.parametrize("tiles", [True, False])
+@pytest.mark.parametrize("per_frame_ranges", [True, False])
 @pytest.mark.parametrize("name,sf,shape", [("frontalface_alt", 1.2, (640, 480)), ("frontalface_alt2", 1.3, (500, 380)),
                                            ("frontalface_alt_tree", 1.25, (480, 360)), ("fullbody", 1.2, (400, 420)),
                                            ("eye_tree_eyeglasses", 1.1, (330, 250)), ("frontalface_default", 1.15, (700, 300))])
-def test_scale_cascade_mode_equals_ref_sc_oracle(gpu_ctx, monkeypatch, name, sf, shape, tiles):
+def test_scale_cascade_mode_equals_ref_sc_oracle(gpu_ctx, monkeypatch, name, sf, shape, per_frame_ranges):
     """CLFD_MODE_SCALE_CASCADE (SURVEY 8-f row 3): one integral image, features scaled per factor,
     step max(2, factor) and the skip rule of HaarDetectObjects_ScaleCascade_Invoker -- exit codes
-    (including skipped / out-of-bounds markers) and the rect set identical to the REF-SC oracle."""
+    (including skipped / out-of-bounds markers) and the rect set identical to the REF-SC oracle.
+    The batch runs as one range, or as one range per frame (the kernels see pre-offset codes, the
+    survivor queues restart and the rect count carries over between ranges)."""
     W, H = shape
     frames = np.stack([octave_frame(W, H, 21), uniform_frame(W, H, 22), np.full((H, W), 255, np.uint8)])
     cas = clfd.Cascade(cascade_path(name))
     det = clfd.Detector(gpu_ctx, cas, W, H, max_batch=3, scale_factor=sf, scale_cascade=True)
+    monkeypatch.setenv("CLFD_DETECT_CHUNKS", "1")
+    if per_frame_ranges:
+        launches_one_range = det.detect(frames).stats["kernel_launches"]
+        monkeypatch.setenv("CLFD_DETECT_CHUNKS", "3")
     res = det.detect(frames)
+    if per_frame_ranges:
+        assert res.stats["kernel_launches"] > launches_one_range   # the batch really was cut
     codes = det.codes(0, 3)
     oc = oracle_cascade(name)
     for f in range(3):
